@@ -4,6 +4,11 @@ iterations/s at 1/2/4/8 B200 vs the numpy CPU path).
 
     python bench.py --gpus N --steps K --warmup W            (torchrun for N > 1)
     python bench.py --impl reference --gpus N --steps K --warmup W
+    python bench.py --gpus 1 --steps K --warmup W --dump-outputs DIR
+
+--dump-outputs DIR writes what the last timed step returned (At, Bt, ct and the per-point fit status, all
+float64) as DIR/<name>.npy.  The inputs depend only on the arguments, so two builds run with the same
+arguments can be compared output for output.
 
 Workload (config.workload): BASELINE.json configs[2] — quadrotor 12-state, IrsLqrZeroOrder,
 T=100, N=1e5 samples/step per GPU.  A "step" is one full smoothing linearization
@@ -107,6 +112,14 @@ def _reference_timing_note():
         return "; ".join("%s T=%d N=%d: %.3g samples/s" % (k, v["T"], v["N"], v["samples_per_s"]) for k, v in t.items())
     except Exception:
         return "unavailable"
+
+
+def dump_outputs(out_dir, arrays):
+    """arrays: name -> numpy array, written as out_dir/<name>.npy in float64 (the fit status as 0.0 / 1.0 / 2.0)."""
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), np.asarray(a, dtype=np.float64))
+    log("outputs of the last timed step written to", out_dir)
 
 
 def quadrotor_problem(for_cpu=False):
@@ -234,7 +247,9 @@ def run_gpu(args, rank, local_rank, world):
 
     tick = torch.zeros((1,), dtype=torch.float32, device="cuda")
 
-    def timed(fn, steps, warmup):
+    def timed(fn, steps, warmup, outputs=None):
+        """Device time of `steps` calls after `warmup` untimed ones.  `outputs` (a list) receives host copies
+        of the tensors the last timed call returned, taken after the end event."""
         for k in range(warmup):
             fn(k)
         barrier()
@@ -246,9 +261,11 @@ def run_gpu(args, rank, local_rank, world):
             dist.all_reduce(tick)
         e0.record()
         for k in range(steps):
-            fn(warmup + k)
+            last = fn(warmup + k)
         e1.record()
         barrier()
+        if outputs is not None:
+            outputs.extend(_device.to_numpy(t) for t in last)
         ms = torch.tensor([e0.elapsed_time(e1)], dtype=torch.float64, device="cuda")
         if world > 1:
             dist.all_reduce(ms, op=dist.ReduceOp.MAX)
@@ -256,7 +273,10 @@ def run_gpu(args, rank, local_rank, world):
 
     # 1. headline: device-resident throughput of the whole smoothing pass
     t_w0 = time.time()
-    ms = timed(step_device, args.steps, args.warmup)
+    last_step = [] if args.dump_outputs and rank == 0 else None
+    ms = timed(step_device, args.steps, args.warmup, outputs=last_step)
+    if last_step is not None:
+        dump_outputs(args.dump_outputs, dict(zip(("At", "Bt", "ct", "status"), last_step)))
     samples_per_step = world * T_STEPS * N_SAMPLES
     value = samples_per_step * args.steps / (ms * 1e-3)
 
@@ -604,7 +624,13 @@ def main():
     ap.add_argument("--no-batched", action="store_true", help="skip the 4096-instance leg (configs[4])")
     ap.add_argument("--no-other-configs", action="store_true", help="skip the pendulum/bicycle/three_cart legs")
     ap.add_argument("--no-strong", action="store_true", help="skip the strong-scaling legs")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the outputs of the last timed step as DIR/<name>.npy (GPU arm only)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs needs the GPU arm (--impl ours)")
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))

@@ -1,9 +1,8 @@
 """Worker wire protocol (SURVEY.md section 8(f)-4; reference: zmq_parallel_cmp/array_io.py:6-26,
 examples/planar_hand/planar_hand_worker.py:19-80, irs_lqr/irs_lqr_quasistatic.py:118-126, 228-263).
-CPU: the framing round-trips and is byte compatible with the reference's own array_io (when /root/reference is
-present).  GPU: a GpuLinearizationWorker thread answers the solver-side task loop; the blocks equal the direct
-linearization bit for bit, whatever the stride."""
-import os
+CPU: the framing round-trips and is byte compatible with the reference's array_io.  GPU: a GpuLinearizationWorker
+thread answers the solver-side task loop; the blocks equal the direct linearization bit for bit, whatever the
+stride."""
 import threading
 
 import numpy as np
@@ -38,23 +37,19 @@ def test_framing_round_trip():
 
 
 def test_framing_is_byte_compatible_with_the_reference():
-    from oracle import ref_import
-    if not ref_import.reference_available():
-        pytest.skip("reference tree not present")
-    import importlib.util
-    spec = importlib.util.spec_from_file_location(
-        "ref_array_io", os.path.join(ref_import.REFERENCE_ROOT, "zmq_parallel_cmp", "array_io.py"))
-    ref = importlib.util.module_from_spec(spec)
-    spec.loader.exec_module(ref)
+    """The reference's message (zmq_parallel_cmp/array_io.py:6-26) is two frames: pyzmq's send_json of
+    dict(dtype=str(A.dtype), shape=A.shape, t=t, n_samples=n_samples, std=std), then the raw C-order array.
+    The frames below are those bytes, so the check needs nothing outside this repository."""
     from irs_mpc_b200 import worker
     ctx = zmq.Context.instance()
     tx, rx = _pair(ctx, "compat")
     A = np.random.default_rng(0).standard_normal((5, 7))
     worker.send_array(tx, A, t=[0, 1, 2, 3, 4], n_samples=50, std=[0.3])
-    B, t, n_samples, std = ref.recv_array(rx)                  # the reference reads what we send
-    np.testing.assert_array_equal(A, B)
-    assert (t, n_samples, std) == ([0, 1, 2, 3, 4], 50, [0.3])
-    ref.send_array(tx, A * 2, t=[9], n_samples=-1, std=[-1])   # and we read what the reference sends
+    header, payload = rx.recv_multipart()                      # the frames the reference's recv_array parses
+    assert header == b'{"dtype": "float64", "shape": [5, 7], "t": [0, 1, 2, 3, 4], "n_samples": 50, "std": [0.3]}'
+    assert payload == A.tobytes()
+    tx.send_multipart([b'{"dtype": "float64", "shape": [5, 7], "t": [9], "n_samples": -1, "std": [-1]}',
+                       (A * 2).tobytes()])                     # and we read what the reference's send_array sends
     B, t, n_samples, std = worker.recv_array(rx)
     np.testing.assert_array_equal(A * 2, B)
     assert (t, n_samples, std) == ([9], -1, [-1])
