@@ -229,8 +229,10 @@ int irs_project_batch_f64(int system, const double* params_host, int nparams, do
 /* solve_tvlqr backward pass (irs_lqr/tv_lqr.py:30-145, inactive bounds): affine Riccati recursion
  * for I independent instances.  At [I,T,n,n], Bt [I,T,n,m], ct [I,T,n], Q/Qd [n,n], R [m,m]
  * (full R; the QP's 1/2 u'Ru of tv_lqr.py:110 is applied inside), xd [I,T+1,n] (xd_stride =
- * (T+1)*n) or one shared trajectory (xd_stride = 0).  Outputs K [I,T,m,n], k [I,T,m],
- * status [I] (1 = H not SPD / NaN -> the caller raises the reference's ValueError, tv_lqr.py:139). */
+ * (T+1)*n) or one shared trajectory (xd_stride = 0).  The weights need not be symmetric: the cost
+ * only sees their symmetric parts, and those are what the recursion uses.  Outputs K [I,T,m,n], k [I,T,m],
+ * status [I] (1 = an H not SPD, or a K_t / k_t not finite -> the caller raises the reference's ValueError,
+ * tv_lqr.py:139). */
 int irs_tvlqr_riccati(int n, int m, const double* At, const double* Bt, const double* ct,
                       const double* Q, const double* Qd, const double* R,
                       const double* xd, long long xd_stride, int I, int T,

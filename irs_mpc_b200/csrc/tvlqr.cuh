@@ -107,7 +107,7 @@ __device__ __forceinline__ double dot4(const double* a, int sa, const double* b,
 
 template <int n, int m>
 struct TvlqrSmem {
-    double P[n * n], A[n * n], PA[n * n];
+    double P[n * n], A[n * n], PA[n * n], Qs[n * n];
     double B[n * m], PB[n * m], G[m * n], Kt[m * n];
     double H[m * m];
     double p[n], w[n], c[n], xd[n], g[m], kt[m];
@@ -150,14 +150,19 @@ __global__ void __launch_bounds__(G == 32 ? 32 * kTvlqrWarps : G) tvlqr_riccati_
         }
     };
     prefetch(a.T - 1);
-    // terminal condition: P_T = Qd, p_T = -Qd xd_T
+    // terminal condition: P_T = sym(Qd), p_T = -sym(Qd) xd_T; sym(Q) for the gradient term.  The cost
+    // x'Qx only sees the symmetric part of a weight, so that is what the recursion uses (for symmetric
+    // input 0.5 (a + a) = a exactly: nothing changes).
     for (int e = gt; e < n * n; e += G) {
-        s.P[e] = a.Qd[e];
-        if (a.Pout != nullptr) a.Pout[((long long)inst * (a.T + 1) + a.T) * n * n + e] = a.Qd[e];
+        const int i = e / n, j = e % n;
+        const double qd = 0.5 * (a.Qd[e] + a.Qd[j * n + i]);
+        s.P[e] = qd;
+        s.Qs[e] = 0.5 * (a.Q[e] + a.Q[j * n + i]);
+        if (a.Pout != nullptr) a.Pout[((long long)inst * (a.T + 1) + a.T) * n * n + e] = qd;
     }
     for (int i = gt; i < n; i += G) {
         double acc = 0.0;
-        for (int q = 0; q < n; ++q) acc -= a.Qd[i * n + q] * xd_i[(long long)a.T * n + q];
+        for (int q = 0; q < n; ++q) acc -= 0.5 * (a.Qd[i * n + q] + a.Qd[q * n + i]) * xd_i[(long long)a.T * n + q];
         s.p[i] = acc;
     }
     for (int t = a.T - 1; t >= 0; --t) {
@@ -239,10 +244,12 @@ __global__ void __launch_bounds__(G == 32 ? 32 * kTvlqrWarps : G) tvlqr_riccati_
                         a.k[it * m + i] = y[i];
                     }
                 }
+#pragma unroll
+                for (int i = 0; i < m; ++i) ok = ok && isfinite(y[i]);      // NaN / Inf in c or xd reach k only
             }
         }
         group_sync();
-        // P <- sym(Q + A'PA + G'K),  p <- -Q xd_t + A'w + G'k.  Each thread forms entry (i,j) and its
+        // P <- sym(Q + A'PA + G'K),  p <- -sym(Q) xd_t + A'w + G'k.  Each thread forms entry (i,j) and its
         // mirror (j,i) and writes their mean: P stays exactly symmetric without a second pass.
         double Pnew[(n * n + n + G - 1) / G];
 #pragma unroll
@@ -255,7 +262,7 @@ __global__ void __launch_bounds__(G == 32 ? 32 * kTvlqrWarps : G) tvlqr_riccati_
                 Pnew[k] = 0.5 * (aij + aji);
             } else if (e < n * n + n) {
                 const int i = e - n * n;
-                Pnew[k] = (dot4<n>(&s.A[i], n, s.w, 1) - dot4<n>(&a.Q[i * n], 1, s.xd, 1)) +
+                Pnew[k] = (dot4<n>(&s.A[i], n, s.w, 1) - dot4<n>(&s.Qs[i * n], 1, s.xd, 1)) +
                           dot4<m>(&s.G[i], n, s.kt, 1);
             }
         }
@@ -273,7 +280,7 @@ __global__ void __launch_bounds__(G == 32 ? 32 * kTvlqrWarps : G) tvlqr_riccati_
         // (the group_sync after the next step's operand stores orders these writes before its reads)
     }
     group_sync();
-    // NaN guard on the final value function
+    // NaN guard on the final value function (every K_t, k_t has been checked where it was written)
     for (int e = gt; e < n * n; e += G)
         if (!(s.P[e] == s.P[e])) ok = false;
     if constexpr (G == 32) {
@@ -380,15 +387,19 @@ __global__ void __launch_bounds__(kTvlqrTiledThreads) tvlqr_riccati_tiled_kernel
         if (gt < n) { s.c[gt] = rc;  s.xd[gt] = rxd; }
     };
     prefetch();
-    // terminal condition: P_T = Qd, p_T = -Qd xd_T (or the carried (P, p) of a later segment);
-    // constants into shared memory
+    // terminal condition: P_T = sym(Qd), p_T = -sym(Qd) xd_T (or the carried (P, p) of a later segment);
+    // constants into shared memory, Q as sym(Q) (the weights' symmetric parts: see the generic kernel)
     double* carry_i = a.carry != nullptr ? a.carry + (long long)inst * (n * n + n) : nullptr;
-    for (int e = gt; e < n * n; e += G) { s.P[e] = t_hi == a.T ? a.Qd[e] : carry_i[e];  s.Q[e] = a.Q[e]; }
+    for (int e = gt; e < n * n; e += G) {
+        const int i = e / n, j = e % n;
+        s.P[e] = t_hi == a.T ? 0.5 * (a.Qd[e] + a.Qd[j * n + i]) : carry_i[e];
+        s.Q[e] = 0.5 * (a.Q[e] + a.Q[j * n + i]);
+    }
     for (int e = gt; e < m * m; e += G) s.Rh[e] = 0.5 * a.R[e];
     for (int i = gt; i < n; i += G) {
         if (t_hi == a.T) {
             double acc = 0.0;
-            for (int q = 0; q < n; ++q) acc -= a.Qd[i * n + q] * xd_i[(long long)a.T * n + q];
+            for (int q = 0; q < n; ++q) acc -= 0.5 * (a.Qd[i * n + q] + a.Qd[q * n + i]) * xd_i[(long long)a.T * n + q];
             s.p[i] = acc;
         } else {
             s.p[i] = carry_i[n * n + i];
@@ -467,12 +478,14 @@ __global__ void __launch_bounds__(kTvlqrTiledThreads) tvlqr_riccati_tiled_kernel
                     pk[i] = y[i];
                 }
             }
+#pragma unroll
+            for (int i = 0; i < m; ++i) ok = ok && isfinite(y[i]);
         }
         pK -= m * n;
         pk -= m;
         __syncthreads();
         // ---- phase 4: Pn = Q + A' PA + G' K (warps 0-1; raw, symmetrised when stored),
-        //               p <- -Q xd_t + A' w + G' k (warp 2) ----
+        //               p <- -sym(Q) xd_t + A' w + G' k (warp 2) ----
         double pnew = 0.0;
         if (gt < hn * hn) {
             double acc[2][2] = {{s.Q[pa_r0 * n + pa_c0], s.Q[pa_r0 * n + pa_c0 + 1]},
@@ -496,7 +509,7 @@ __global__ void __launch_bounds__(kTvlqrTiledThreads) tvlqr_riccati_tiled_kernel
         if (t > t_lo) publish();
         __syncthreads();
     }
-    // NaN guard on the final value function
+    // NaN guard on the final value function (K_t, k_t: checked where written)
     for (int e = gt; e < n * n; e += G)
         if (!(s.P[e] == s.P[e])) ok = false;
     ok = __syncthreads_and(ok);
@@ -525,7 +538,7 @@ __global__ void __launch_bounds__(kTvlqrTiledThreads) tvlqr_riccati_tiled_kernel
 // quarter warp exits, the second instance of a warp sits 16 bytes (mod 32) beside the first so that their
 // quarter-warp-sharing lanes hit different banks, the rows of P [A | B], of P and of sym(Q) are shifted by 16 bytes
 // per row group so that tile accesses of different row groups do too, and vector operands are read along contiguous rows (P is
-// symmetric, Q is kept transposed).  Eight instances per block of 128 threads, four blocks per SM: all 4096
+// symmetric, and so is sym(Q)).  Eight instances per block of 128 threads, four blocks per SM: all 4096
 // instances of configs[4] are resident at once.  Next step's operands are prefetched into registers (18
 // doubles per lane) during the last product of the current step.
 // ---------------------------------------------------------------------------------------------
@@ -554,7 +567,7 @@ struct RicPackInst {
 template <int n, int m>
 struct RicPackSmem {
     double Qs[RicPackInst<n, m>::kP + (RicPackInst<n, m>::kP & 1)];      // sym(Q), rows shifted like P (tile loads)
-    double Qt[n * n], Rh[m * m];                                         // Q^T (gradient term), R / 2
+    double Rh[m * m];                                                    // R / 2
     RicPackInst<n, m> inst[kRicPackPerBlock];
 };
 
@@ -612,7 +625,6 @@ __global__ void __launch_bounds__(kRicPackThreads, 4) tvlqr_riccati_packed_kerne
     for (int e = tid; e < n * n; e += kRicPackThreads) {
         const int r = e / n, c = e % n;
         sm.Qs[Inst::p_row(r) + c] = 0.5 * (a.Q[e] + a.Q[c * n + r]);       // x' Q x only sees the symmetric part
-        sm.Qt[e] = a.Q[c * n + r];
     }
     for (int e = tid; e < m * m; e += kRicPackThreads) sm.Rh[e] = 0.5 * a.R[e];
     __syncthreads();
@@ -652,14 +664,14 @@ __global__ void __launch_bounds__(kRicPackThreads, 4) tvlqr_riccati_packed_kerne
         }
     };
     prefetch(a.T - 1);
-    // terminal condition P_T = sym(Qd) (x' Qd x only sees the symmetric part), p_T = -Qd xd_T
+    // terminal condition P_T = sym(Qd) (x' Qd x only sees the symmetric part), p_T = -sym(Qd) xd_T
     for (int e = j; e < n * n; e += kRicPackLanes) {
         const int r = e / n, c = e % n;
         s.P[Inst::p_row(r) + c] = 0.5 * (a.Qd[r * n + c] + a.Qd[c * n + r]);
     }
     {
         double acc = 0.0;
-        for (int q = 0; q < n; ++q) acc -= a.Qd[j * n + q] * xd_i[(long long)a.T * n + q];
+        for (int q = 0; q < n; ++q) acc -= 0.5 * (a.Qd[j * n + q] + a.Qd[q * n + j]) * xd_i[(long long)a.T * n + q];
         s.p[j] = acc;
     }
     publish();
@@ -721,6 +733,7 @@ __global__ void __launch_bounds__(kRicPackThreads, 4) tvlqr_riccati_packed_kerne
                 for (int q = 0; q < m; ++q) acc = fma(-Hi[i][q], s.GH[q * W + j], acc);
                 s.Kt[i * n + j] = acc;
                 if (live) Kg[i * n + j] = acc;
+                ok = ok && isfinite(acc);      // NaN / Inf in c or xd reach k only: checked below
             }
             if (j == 0) {
                 double* kg = a.k + (inst * a.T + t) * m;
@@ -731,6 +744,7 @@ __global__ void __launch_bounds__(kRicPackThreads, 4) tvlqr_riccati_packed_kerne
                     for (int q = 0; q < m; ++q) acc = fma(-Hi[i][q], s.g[q], acc);
                     s.kt[i] = acc;
                     if (live) kg[i] = acc;
+                    ok = ok && isfinite(acc);
                 }
             }
         }
@@ -739,7 +753,7 @@ __global__ void __launch_bounds__(kRicPackThreads, 4) tvlqr_riccati_packed_kerne
         // phase 4 and the other warps' work; prefetching a whole step ahead spilled at 128 registers)
         if (t > 0) prefetch(t - 1);
         // ---- phase 4: Pn += G^T K (lanes 0-5) -> P and its mirror (no phase reads P any more),
-        //               p <- -Q xd_t + A^T w + G^T k (every lane one row) ----
+        //               p <- -sym(Q) xd_t + A^T w + G^T k (every lane one row; sym(Q) read along row j = column j) ----
         if (pn_tile) {
             tile4_atb<m, false>(s.GH, W, pn_r0, s.Kt, n, pn_c0, pn);
             if (pn_r0 == pn_c0) {
@@ -758,7 +772,7 @@ __global__ void __launch_bounds__(kRicPackThreads, 4) tvlqr_riccati_packed_kerne
 #pragma unroll
             for (int q = 0; q < n; ++q) {
                 av = fma(s.AB[q * W + j], s.w[q], av);
-                qv = fma(sm.Qt[q * n + j], s.xd[q], qv);
+                qv = fma(sm.Qs[Inst::p_row(q) + j], s.xd[q], qv);
             }
 #pragma unroll
             for (int q = 0; q < m; ++q) gv = fma(s.GH[q * W + j], s.kt[q], gv);
@@ -769,7 +783,7 @@ __global__ void __launch_bounds__(kRicPackThreads, 4) tvlqr_riccati_packed_kerne
         if (t > 0) publish();
         __syncwarp(kRicPackMask);
     }
-    // NaN guard on the final value function; one status per instance
+    // NaN guard on the final value function (K_t, k_t: checked where written); one status per instance
     for (int e = j; e < n * n; e += kRicPackLanes) {
         const double v = s.P[Inst::p_row(e / n) + e % n];
         if (!(v == v)) ok = false;

@@ -162,7 +162,7 @@ __global__ void __launch_bounds__(32) box_mpc_kernel(const BoxMpcArgs a) {
     double* u = wu + T * m;
     double* kk = u + T * m;
     double* Pc = kk + T * m;
-    double* qxd = Pc + T * n;     // Q xd_t (t < T), Qd xd_T
+    double* qxd = Pc + T * n;     // sym(Q) xd_t (t < T), sym(Qd) xd_T
     double* pv = qxd + (T + 1) * n;   // [2][n] rolling p_{t+1}, p_t
     double* ww = pv + 2 * n;      // [n]
     double* gv = ww + n;          // [m]
@@ -201,21 +201,22 @@ __global__ void __launch_bounds__(32) box_mpc_kernel(const BoxMpcArgs a) {
         }
         Ap = sA;  Bp = sB;  Kp = sK;  Hp = sH;  cp = sc;
     }
-    // Pc_t = P_{t+1} c_t, Q xd_t; cold start of the split variables: z = clip(target), w = 0
+    // Pc_t = P_{t+1} c_t, sym(Q) xd_t, sym(Qd) xd_T (the cost only sees the weights' symmetric parts, as
+    // in tvlqr_riccati_kernel); cold start of the split variables: z = clip(target), w = 0
     for (int e = lane; e < T * n; e += 32) {
         const int t = e / n, i = e % n;
         const double* Pr = a.P + ((long long)inst * (T + 1) + t + 1) * n * n + i * n;
         double acc = 0.0, accq = 0.0;
         for (int q = 0; q < n; ++q) {
             acc += Pr[q] * a.ct[(base + t) * n + q];
-            accq += a.Q[i * n + q] * xd_i[(long long)t * n + q];
+            accq += 0.5 * (a.Q[i * n + q] + a.Q[q * n + i]) * xd_i[(long long)t * n + q];
         }
         Pc[e] = acc;
         qxd[e] = accq;
     }
     if (lane < n) {
         double accq = 0.0;
-        for (int q = 0; q < n; ++q) accq += a.Qd[lane * n + q] * xd_i[(long long)T * n + q];
+        for (int q = 0; q < n; ++q) accq += 0.5 * (a.Qd[lane * n + q] + a.Qd[q * n + lane]) * xd_i[(long long)T * n + q];
         qxd[T * n + lane] = accq;
     }
     for (int e = lane; e < (T + 1) * n; e += 32) {

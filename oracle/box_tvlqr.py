@@ -22,6 +22,12 @@ DEFAULT_EPS = 1e-8
 DEFAULT_MAX_ITER = 100000
 
 
+def _sym(W):
+    """The symmetric part of a weight: x'Wx sees nothing else (for symmetric W exactly W)."""
+    W = np.asarray(W, dtype=np.float64)
+    return 0.5 * (W + W.T)
+
+
 def penalties(Q, R, rho0=DEFAULT_RHO0):
     """Per-coordinate ADMM penalties: rho0 times the cost curvature of the coordinate, floored at
     the mean curvature (coordinates with zero weight still get a usable penalty)."""
@@ -35,6 +41,7 @@ def augmented_gains(At, Bt, ct, Q, Qd, R, dx, du):
     """Matrix part of the Riccati recursion for the augmented cost (independent of z, w and of the
     start time): K_t, Hinv_t, P_t (t = 0..T)."""
     T, n, m = At.shape[0], Q.shape[0], R.shape[0]
+    Q, Qd, R = _sym(Q), _sym(Qd), _sym(R)
     Qe, Qde, Re = Q + 0.5 * np.diag(dx), Qd + 0.5 * np.diag(dx), 0.5 * R + 0.5 * np.diag(du)
     K = np.zeros((T, m, n))
     Hinv = np.zeros((T, m, m))
@@ -61,6 +68,7 @@ def admm_box_qp(At, Bt, ct, Q, Qd, R, x0, xd, xlo, xhi, ulo, uhi, gains=None, dx
     zeros.  Bounds are per coordinate (constant in time), as IrsLqr passes them (irs_lqr.py:160-167);
     the bound on the fixed x_{t0} is not part of the problem."""
     T, n, m = At.shape[0], Q.shape[0], R.shape[0]
+    Q, Qd = _sym(Q), _sym(Qd)
     if dx is None:
         dx, du = penalties(Q, R)
     if gains is None:
@@ -166,6 +174,7 @@ def dense_qp_reference(At, Bt, ct, Q, Qd, R, x0, xd, xlo, xhi, ulo, uhi):
     (x = Sx x0 + Su u + s0) and solve the inequality-constrained QP in u with scipy (SLSQP)."""
     from scipy.optimize import minimize
     T, n, m = At.shape[0], Q.shape[0], R.shape[0]
+    Q, Qd, R = _sym(Q), _sym(Qd), _sym(R)      # the gradient below assumes symmetric weights
     Su = np.zeros(((T + 1) * n, T * m))
     s0 = np.zeros((T + 1) * n)
     s0[:n] = x0

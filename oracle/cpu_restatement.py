@@ -442,22 +442,29 @@ def exact_tv_matrices(system, x_trj, u_trj):
     return At, Bt, ct
 
 
-def tvlqr_riccati(At, Bt, ct, Q, Qd, R, xd_trj):
+def tvlqr_riccati(At, Bt, ct, Q, Qd, R, xd_trj, return_hessians=False):
     """Backward pass equivalent to the QP of irs_lqr/tv_lqr.py:69-137 when no bound is active.
 
     Cost restated from the QP: sum_{s<T} (x_s-xd_s)'Q(x_s-xd_s) + (1/2) u_s'R u_s  (:110, :127;
     Drake's AddQuadraticCost(Q,b,x) is 0.5 x'Qx + b'x) + (x_T-xd_T)'Qd(x_T-xd_T) (:130), subject to
     x_{s+1} = A_s x_s + B_s u_s + c_s (:92-95).  Value function V_s(x) = x'P_s x + 2 p_s'x + const.
-    Returns feedback gains K[T,m,n], k[T,m] with u_s = K_s x_s + k_s.
+    The cost only sees the symmetric parts of Q, Qd and R, so the recursion runs on those (for symmetric
+    weights 0.5 (W + W') = W exactly).
+    Returns feedback gains K[T,m,n], k[T,m] with u_s = K_s x_s + k_s; with return_hessians also the
+    value-function Hessians P[T+1,n,n] and the step Hessians H[T,m,m] = R/2 + B'P_{s+1}B.
     """
     T = At.shape[0]
     n = Q.shape[0]
     m = R.shape[0]
+    Q, Qd, R = 0.5 * (Q + Q.T), 0.5 * (Qd + Qd.T), 0.5 * (R + R.T)
     Rh = 0.5 * R
     K = np.zeros((T, m, n))
     k = np.zeros((T, m))
+    Ps = np.zeros((T + 1, n, n))
+    Hs = np.zeros((T, m, m))
     P = Qd.copy()
     p = -Qd.dot(xd_trj[T])
+    Ps[T] = P
     for t in range(T - 1, -1, -1):
         A, B, c = At[t], Bt[t], ct[t]
         PA = P.dot(A)
@@ -466,6 +473,7 @@ def tvlqr_riccati(At, Bt, ct, Q, Qd, R, xd_trj):
         H = Rh + B.T.dot(PB)
         G = B.T.dot(PA)
         g = B.T.dot(w)
+        Hs[t] = H
         L = np.linalg.cholesky(H)          # raises LinAlgError if H is not SPD
         Kt = -np.linalg.solve(L.T, np.linalg.solve(L, G))
         kt = -np.linalg.solve(L.T, np.linalg.solve(L, g))
@@ -473,6 +481,9 @@ def tvlqr_riccati(At, Bt, ct, Q, Qd, R, xd_trj):
         p = -Q.dot(xd_trj[t]) + A.T.dot(w) + G.T.dot(kt)
         P = Q + A.T.dot(PA) + G.T.dot(Kt)
         P = 0.5 * (P + P.T)
+        Ps[t] = P
+    if return_hessians:
+        return K, k, Ps, Hs
     return K, k
 
 
