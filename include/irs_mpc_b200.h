@@ -271,8 +271,9 @@ int irs_tvlqr_riccati_segment(int n, int m, const double* At, const double* Bt, 
  *    are the ADMM penalties;
  *    K0 [I,T,m,n], k0 [I,T,m] (optional, mpc = 1): the UNCONSTRAINED gains; a start time whose
  *    unconstrained plan stays inside [lo - tol, hi + tol] skips its QP (its bounds are inactive, the
- *    minimiser is K0 x + k0).  status[i] = 1 if a solve did not reach eps within max_iter (-> the
- *    reference's ValueError).
+ *    minimiser is K0 x + k0).  A solve stops when max |y - z| and the change of z are both
+ *    <= eps max(1, |z|) (units of z: invariant under a scaling of the weights).  status[i] = 1 if a
+ *    solve did not reach eps within max_iter (-> the reference's ValueError).
  *    Algorithm and its check against a dense QP solve: oracle/box_tvlqr.py. */
 int irs_tvlqr_riccati_ex(int n, int m, const double* At, const double* Bt, const double* ct,
                          const double* Q, const double* Qd, const double* R,

@@ -325,6 +325,9 @@ __global__ void __launch_bounds__(32) box_mpc_kernel(const BoxMpcArgs a) {
                 __syncwarp();
             }
             // ---- relaxed projection, dual update, residuals (element-wise over the horizon) ----
+            // Both residuals are measured in the units of z (primal: |y - z|, dual: the change of z), so the
+            // stopping test does not change under a common scaling of (Q, Qd, R), which leaves the QP's
+            // minimiser unchanged.  (A dual residual weighted by the penalties would be in cost units.)
             double r_prim = 0.0, r_dual = 0.0, scale = 1.0;
             for (int e = (t0 + 1) * n + lane; e < (T + 1) * n; e += 32) {
                 const int i = e % n;
@@ -332,7 +335,7 @@ __global__ void __launch_bounds__(32) box_mpc_kernel(const BoxMpcArgs a) {
                 const double zn = fmin(fmax(xh + wx[e], a.xlo[(e / n) * a.xbox_stride + i]), a.xhi[(e / n) * a.xbox_stride + i]);
                 wx[e] += xh - zn;
                 r_prim = fmax(r_prim, fabs(x[e] - zn));
-                r_dual = fmax(r_dual, fabs(a.dx[i] * (zn - zx[e])));
+                r_dual = fmax(r_dual, fabs(zn - zx[e]));
                 scale = fmax(scale, fabs(zn));
                 zx[e] = zn;
             }
@@ -342,7 +345,7 @@ __global__ void __launch_bounds__(32) box_mpc_kernel(const BoxMpcArgs a) {
                 const double zn = fmin(fmax(uh + wu[e], a.ulo[(e / m) * a.ubox_stride + j]), a.uhi[(e / m) * a.ubox_stride + j]);
                 wu[e] += uh - zn;
                 r_prim = fmax(r_prim, fabs(u[e] - zn));
-                r_dual = fmax(r_dual, fabs(a.du[j] * (zn - zu[e])));
+                r_dual = fmax(r_dual, fabs(zn - zu[e]));
                 scale = fmax(scale, fabs(zn));
                 zu[e] = zn;
             }

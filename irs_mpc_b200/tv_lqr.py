@@ -60,7 +60,7 @@ def riccati_device(At, Bt, ct, Q, Qd, R, xd, xd_stride):
 # ADMM parameters of the bounded solve (csrc/tvlqr_box.cuh)
 BOX_RHO0 = 1.0
 BOX_ALPHA = 1.6
-BOX_EPS = 1e-8
+BOX_EPS = 1e-10
 BOX_MAX_ITER = 100000
 BOUND_TOL = 1e-9
 

@@ -988,7 +988,7 @@ def _bicycle_lin(T, u_const):
 
 
 def test_solve_tvlqr_active_bounds_matches_admm_oracle_and_dense_qp(api):
-    """One QP with an active steer / steer-rate box: the CUDA ADMM against the numpy ADMM (1e-6) and
+    """One QP with an active steer / steer-rate box: the CUDA ADMM against the numpy ADMM (1e-7) and
     against an independent dense QP solve (scipy SLSQP, 1e-5); the plan obeys the bounds."""
     from oracle import box_tvlqr as bq
     T = 12
@@ -1000,8 +1000,8 @@ def test_solve_tvlqr_active_bounds_matches_admm_oracle_and_dense_qp(api):
     xs, us = api.solve_tvlqr(At, Bt, ct, cfg["Q"], cfg["Qd"], cfg["R"], cfg["x0"], cfg["xd_trj"], None,
                              x_bound_abs=xb, u_bound_abs=ub)
     xo, uo, _ = bq.admm_box_qp(At, Bt, ct, cfg["Q"], cfg["Qd"], cfg["R"], cfg["x0"], cfg["xd_trj"], xlo, xhi, ulo, uhi)
-    np.testing.assert_allclose(xs, xo, rtol=0, atol=1e-6)
-    np.testing.assert_allclose(us, uo, rtol=0, atol=1e-6)
+    np.testing.assert_allclose(xs, xo, rtol=0, atol=1e-7)
+    np.testing.assert_allclose(us, uo, rtol=0, atol=1e-7)
     xr, ur, res = bq.dense_qp_reference(At, Bt, ct, cfg["Q"], cfg["Qd"], cfg["R"], cfg["x0"], cfg["xd_trj"], xlo, xhi,
                                         ulo, uhi)
     assert res.success
@@ -1036,8 +1036,8 @@ def test_solve_tvlqr_time_varying_and_relative_bounds(api):
     args = (At, Bt, ct, cfg["Q"], cfg["Qd"], cfg["R"], cfg["x0"], cfg["xd_trj"])
     xs, us = api.solve_tvlqr(*args, None, x_bound_abs=np.stack((xlo, xhi)), u_bound_abs=np.stack((ulo, uhi)))
     xo, uo, _ = bq.admm_box_qp(*args, xlo, xhi, ulo, uhi)
-    np.testing.assert_allclose(xs, xo, rtol=0, atol=1e-6)
-    np.testing.assert_allclose(us, uo, rtol=0, atol=1e-6)
+    np.testing.assert_allclose(xs, xo, rtol=0, atol=1e-7)
+    np.testing.assert_allclose(us, uo, rtol=0, atol=1e-7)
     xr, ur, res = bq.dense_qp_reference(*args, xlo, xhi, ulo, uhi)
     assert res.success
     np.testing.assert_allclose(us, ur, rtol=0, atol=2e-5)
@@ -1079,8 +1079,8 @@ def test_bicycle_descent_with_active_steer_bound_matches_oracle(api):
     xo, uo, _ = bq.mpc_box_descent(orc, At, Bt, ct, cfg["Q"], cfg["Qd"], cfg["R"], cfg["x0"], cfg["xd_trj"],
                                    cfg["xbound"][0], cfg["xbound"][1], cfg["ubound"][0], cfg["ubound"][1],
                                    gains0=gains0)
-    np.testing.assert_allclose(u_new, uo, rtol=0, atol=2e-6)
-    np.testing.assert_allclose(x_new, xo, rtol=0, atol=2e-6)
+    np.testing.assert_allclose(u_new, uo, rtol=0, atol=1e-6)
+    np.testing.assert_allclose(x_new, xo, rtol=0, atol=1e-6)
     assert np.max(np.abs(x_new[:, 4])) <= np.pi / 4 + 1e-6
     assert np.max(np.abs(x_new[:, 4])) > np.pi / 4 - 1e-3
     assert cost < solver.cost
