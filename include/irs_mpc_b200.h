@@ -20,7 +20,7 @@
 extern "C" {
 #endif
 
-#define IRS_ABI_VERSION 3
+#define IRS_ABI_VERSION 4
 
 /* system ids — the reference's four analytic DynamicalSystem subclasses
  * (examples/pendulum/pendulum_dynamics.py:8, examples/bicycle/bicycle_dynamics.py:8,
@@ -146,34 +146,14 @@ int irs_smooth_finalize(int system, const double* params_host, int nparams, int 
  * is CUDA-graph replayable); done_counter: zero-initialised local device word.  A peer that does
  * not deliver within timeout_s sets status[p] = 2 instead of hanging the GPU.  Every rank must
  * issue the same sequence of calls on the same exchange; P may change from call to call.  All P
- * blocks must be co-resident: P <= irs_smooth_finalize_peer_capacity (error otherwise).
- * prepushed != 0: this rank's blocks and flags were sent by irs_smooth_zero_order_accumulate_push (below); the
- * kernel then skips its own reduction and stores and only waits, sums and fits. */
+ * blocks must be co-resident: P <= irs_smooth_finalize_peer_capacity (error otherwise). */
 int irs_smooth_finalize_peer(int system, const double* params_host, int nparams, int order,
                              const double* x_nom, const double* u_nom, int P, int C, const float* partials,
                              const void* peer_bufs_dev, const void* peer_flags_dev, int* epoch_dev,
                              unsigned int* done_counter, long long slot_stride, int flag_stride,
-                             int rank, int world, double timeout_s, double n_total, int centered, int prepushed,
+                             int rank, int world, double timeout_s, double n_total, int centered,
                              double* At, double* Bt, double* ct, int* status, void* stream);
 int irs_smooth_finalize_peer_capacity(int system, int order, int* max_points);
-
-/* The exchange of irs_smooth_finalize_peer STARTED by the accumulate kernel: irs_smooth_zero_order_accumulate with
- * the exchange of the sample-sharded step (same peer_bufs_dev / peer_flags_dev / epoch_dev / strides as the
- * irs_smooth_finalize_peer call that follows it, which must then pass prepushed = 1).  The block that completes the
- * last chunk of a nominal point reduces the point's chunks (same fixed order, bit-identical sums) and stores the
- * fp64 block into every rank's exchange buffer while the rest of the launch is still sampling, so the fit kernel
- * only waits for arrival flags.  point_counters: P zero-initialised local device words (left zero by the kernel).
- * Only for systems whose zero-order Gram runs on the tensor cores (irs_smooth_push_supported != 0). */
-int irs_smooth_push_supported(int system, int order);
-int irs_smooth_zero_order_accumulate_push(int system, const double* params_host, int nparams, int flags,
-                                          const double* x_nom, const double* u_nom, int P, long long N,
-                                          const float* sigma_host, const float* noise,
-                                          unsigned long long seed, unsigned iter, unsigned stream_id,
-                                          unsigned p0, unsigned long long i0,
-                                          int C, long long S, float* partials,
-                                          const void* peer_bufs_dev, const void* peer_flags_dev, const int* epoch_dev,
-                                          unsigned int* point_counters, long long slot_stride, int flag_stride,
-                                          int rank, int world, void* stream);
 
 /* irs_smooth_finalize for a TIMESTEP-SHARDED run (one process per GPU; BASELINE north star: "the T x N
  * sample rollouts shard along the time axis, with an all-gather of the small per-step (A_t, B_t, c_t)

@@ -12,7 +12,7 @@ LIB_PATH = os.environ.get("IRS_MPC_B200_LIB") or os.path.join(_HERE, "libirs_mpc
 CSRC = os.path.join(_HERE, "csrc")
 INCLUDE = os.path.join(os.path.dirname(_HERE), "include")
 
-ABI_VERSION = 3      # IRS_ABI_VERSION of include/irs_mpc_b200.h this binding was written against
+ABI_VERSION = 4      # IRS_ABI_VERSION of include/irs_mpc_b200.h this binding was written against
 
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17",
               "-shared", "-Xcompiler", "-fPIC"]
@@ -63,11 +63,7 @@ SIGNATURES = {
                                           _ull, _u, _u, _u, _ull, _i, _ll, _vp, _vp],
     "irs_smooth_reduce_chunks": [_i, _i, _vp, _i, _i, _vp, _vp],
     "irs_smooth_finalize_peer": [_i, _c_double_p, _i, _i, _vp, _vp, _i, _i, _vp, _vp, _vp, _vp, _vp, _ll, _i,
-                                 _i, _i, ctypes.c_double, ctypes.c_double, _i, _i, _vp, _vp, _vp, _vp, _vp],
-    "irs_smooth_push_supported": [_i, _i],
-    "irs_smooth_zero_order_accumulate_push": [_i, _c_double_p, _i, _i, _vp, _vp, _i, _ll, _vp, _vp,
-                                              _ull, _u, _u, _u, _ull, _i, _ll, _vp,
-                                              _vp, _vp, _vp, _vp, _ll, _i, _i, _i, _vp],
+                                 _i, _i, ctypes.c_double, ctypes.c_double, _i, _vp, _vp, _vp, _vp, _vp],
     "irs_smooth_finalize_peer_capacity": [_i, _i, ctypes.POINTER(_i)],
     "irs_smooth_finalize_gather": [_i, _c_double_p, _i, _i, _vp, _vp, _i, _i, _vp, _vp, _vp, _vp, _vp, _ll, _i, _i,
                                    _i, _i, ctypes.c_double, ctypes.c_double, _i, _vp, _vp],

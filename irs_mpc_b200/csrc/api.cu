@@ -151,15 +151,11 @@ static int launch_zero_order_mlp(const SmoothArgs& a, cudaStream_t st) {
     // Tile groups per block and blocks per SM (1 KB of shared memory reserved per block, 512 TMEM columns per SM).
     // Two one-group blocks per SM were measured faster than one block of two or three groups (the reference's
     // 100 / 100 network: 0.272 against 0.305 / 0.289 ms); wider networks, whose operand tiles leave room for one
-    // block only, take as many groups as fit.  IRS_MLP_GROUPS forces a count (tuning).
+    // block only, take as many groups as fit.
     const int max_groups = MlpTcSmem<Sys>::groups_for(L, max_smem);
     IRS_REQUIRE(max_groups >= 1, "hidden widths %d / %d need %d bytes of shared memory (limit %d)", L.H1, L.H2,
                 MlpTcSmem<Sys>(L, 1).total, max_smem);
-    int groups = per_sm_smem / (MlpTcSmem<Sys>(L, 1).total + 1024) >= 2 ? 1 : max_groups;
-    if (const char* e = getenv("IRS_MLP_GROUPS")) {
-        const int want = atoi(e);
-        if (want >= 1 && want <= max_groups) groups = want;
-    }
+    const int groups = per_sm_smem / (MlpTcSmem<Sys>(L, 1).total + 1024) >= 2 ? 1 : max_groups;
     const MlpTcSmem<Sys> sm(L, groups);
     int per_sm = per_sm_smem / (sm.total + 1024);
     const int tmem_cols = MlpTcLayout::tmem_alloc_cols(groups * L.tmem_cols_per_group());
@@ -198,8 +194,6 @@ static int launch_zero_order_tc_mode(const SmoothArgs& a, cudaStream_t st) {
         int occ = by_regs < by_smem ? by_regs : by_smem;
         if (by_tmem < occ) occ = by_tmem;
         if (occ > 32) occ = 32;
-        if (const char* e = getenv("IRS_TC_BLOCKS_PER_SM"))      // tuning: cap the resident blocks
-            if (atoi(e) >= 1 && atoi(e) < occ) occ = atoi(e);
         blocks_per_sm = occ < 1 ? 1 : occ;
     }
     // persistent grid: every resident block walks the (point, chunk) item list with stride gridDim.x
@@ -234,7 +228,6 @@ static int fill_smooth_args(SmoothArgs* a, int system, const double* params_host
                             unsigned iter, unsigned stream_id, unsigned p0, unsigned long long i0,
                             int C, long long S, float* partials) {
     if (load_params(system, params_host, nparams, &a->prm)) return 1;
-    memset(&a->push, 0, sizeof(a->push));
     IRS_REQUIRE(x_nom && u_nom && partials, "null pointer argument");
     IRS_REQUIRE(P >= 1 && N >= 1, "need at least one nominal point and one sample (P=%d, N=%lld)", P, N);
     IRS_REQUIRE(C >= 1 && S >= 1 && (long long)C * S >= N, "chunk plan (C=%d, S=%lld) does not cover N=%lld", C, S, N);
@@ -398,14 +391,11 @@ static void launch_rollout(const RolloutArgs& a, cudaStream_t st) {
         }
     }
     if constexpr (is_mlp<Sys>::value) {
-        // learned dynamics: one block per instance with the network in registers (IRS_ROLLOUT_MLP=0: the warp kernel)
-        const char* e = getenv("IRS_ROLLOUT_MLP");
-        if (e == nullptr || atoi(e) != 0) {
-            rollout_mlp_kernel<Sys, CLOSED><<<(unsigned)a.I, kMlpMaxHidden, 0, st>>>(a);
-            return;
-        }
+        // learned dynamics: one block per instance with the network in registers
+        rollout_mlp_kernel<Sys, CLOSED><<<(unsigned)a.I, kMlpMaxHidden, 0, st>>>(a);
+    } else {
+        rollout_kernel<Sys, CLOSED><<<(a.I + kRolloutWarps - 1) / kRolloutWarps, 32 * kRolloutWarps, 0, st>>>(a);
     }
-    rollout_kernel<Sys, CLOSED><<<(a.I + kRolloutWarps - 1) / kRolloutWarps, 32 * kRolloutWarps, 0, st>>>(a);
 }
 
 template <class Sys>
@@ -464,14 +454,11 @@ int irs_smooth_plan(int system, int order, int P, long long N, long long chunk_s
     // P*C blocks give several waves over 148 SMs.  The plan depends on N (and on the caller's
     // chunk_samples) ONLY, never on P, so that a timestep-sharded run (P split over ranks) sums in
     // exactly the same order as the single-GPU run and reproduces it bit for bit.
-    // chunk_samples = 0: the default target of 4096 (IRS_CHUNK_SAMPLES overrides it); callers whose
-    // launches are smaller than a resident grid (timestep-pipelined descents, strong scaling) ask for
-    // smaller chunks so that every SM still holds several work items.
+    // chunk_samples = 0: the default target of 4096; callers whose launches are smaller than a resident
+    // grid (strong scaling) ask for smaller chunks so that every SM still holds several work items.
     const long long tile = 256;        // a block round: 128 lanes x (one sample | one antithetic pair)
     long long target = 4096;
-    const char* e = getenv("IRS_CHUNK_SAMPLES");
-    if (e && atoll(e) > 0) target = atoll(e);
-    if (system == kMlp21 && order == 0 && !(e && atoll(e) > 0)) target = 1536;   // 12 tiles of 128 for up to 3 tile groups; several waves of items
+    if (system == kMlp21 && order == 0) target = 1536;   // 12 tiles of 128 for up to 3 tile groups; several waves of items
     if (chunk_samples > 0) target = chunk_samples;
     long long c = (N + target - 1) / target;
     long long s = (N + c - 1) / c;
@@ -482,20 +469,16 @@ int irs_smooth_plan(int system, int order, int P, long long N, long long chunk_s
     return 0;
 }
 
-static int zero_order_accumulate_impl(int system, const double* params_host, int nparams, int flags,
-                                      const double* x_nom, const double* u_nom, int P, long long N,
-                                      const float* sigma_host, const float* noise,
-                                      unsigned long long seed, unsigned iter, unsigned stream_id,
-                                      unsigned p0, unsigned long long i0,
-                                      int C, long long S, float* partials, const PeerPushArgs* push, void* stream) {
+int irs_smooth_zero_order_accumulate(int system, const double* params_host, int nparams, int flags,
+                                     const double* x_nom, const double* u_nom, int P, long long N,
+                                     const float* sigma_host, const float* noise,
+                                     unsigned long long seed, unsigned iter, unsigned stream_id,
+                                     unsigned p0, unsigned long long i0,
+                                     int C, long long S, float* partials, void* stream) {
     SmoothArgs a;
     if (fill_smooth_args(&a, system, params_host, nparams, flags, x_nom, u_nom, P, N, sigma_host, noise,
                          seed, iter, stream_id, p0, i0, C, S, partials))
         return 1;
-    if (push != nullptr) {
-        IRS_REQUIRE(use_tensor_cores(system), "system %d accumulates on the CUDA cores: no in-kernel push", system);
-        a.push = *push;
-    }
     cudaStream_t st = (cudaStream_t)stream;
     if (use_tensor_cores(system)) {
         switch (system) {
@@ -519,40 +502,6 @@ static int zero_order_accumulate_impl(int system, const double* params_host, int
     }
     set_error("unknown system id %d", system);
     return 1;
-}
-
-int irs_smooth_zero_order_accumulate(int system, const double* params_host, int nparams, int flags,
-                                     const double* x_nom, const double* u_nom, int P, long long N,
-                                     const float* sigma_host, const float* noise,
-                                     unsigned long long seed, unsigned iter, unsigned stream_id,
-                                     unsigned p0, unsigned long long i0,
-                                     int C, long long S, float* partials, void* stream) {
-    return zero_order_accumulate_impl(system, params_host, nparams, flags, x_nom, u_nom, P, N, sigma_host, noise, seed,
-                                      iter, stream_id, p0, i0, C, S, partials, nullptr, stream);
-}
-
-int irs_smooth_push_supported(int system, int order) {
-    return (system >= 0 && system < kNumSystems && order == 0 && system != kMlp21 && use_tensor_cores(system)) ? 1 : 0;
-}
-
-int irs_smooth_zero_order_accumulate_push(int system, const double* params_host, int nparams, int flags,
-                                          const double* x_nom, const double* u_nom, int P, long long N,
-                                          const float* sigma_host, const float* noise,
-                                          unsigned long long seed, unsigned iter, unsigned stream_id,
-                                          unsigned p0, unsigned long long i0,
-                                          int C, long long S, float* partials,
-                                          const void* peer_bufs_dev, const void* peer_flags_dev, const int* epoch_dev,
-                                          unsigned int* point_counters, long long slot_stride, int flag_stride,
-                                          int rank, int world, void* stream) {
-    IRS_REQUIRE(peer_bufs_dev && peer_flags_dev && epoch_dev && point_counters, "null pointer argument");
-    IRS_REQUIRE(world >= 1 && world <= kFinalizeThreads && rank >= 0 && rank < world, "bad rank / world");
-    IRS_REQUIRE(irs_smooth_push_supported(system, 0), "system %d has no in-kernel push (irs_smooth_push_supported)", system);
-    const int width = irs_partial_width(system, 0);
-    IRS_REQUIRE(slot_stride >= (long long)P * width && flag_stride >= P, "exchange buffers too small for P=%d", P);
-    const PeerPushArgs push{(double* const*)peer_bufs_dev, (int* const*)peer_flags_dev, epoch_dev, point_counters,
-                            slot_stride, flag_stride, rank, world};
-    return zero_order_accumulate_impl(system, params_host, nparams, flags, x_nom, u_nom, P, N, sigma_host, noise, seed,
-                                      iter, stream_id, p0, i0, C, S, partials, &push, stream);
 }
 
 int irs_smooth_first_order_accumulate(int system, const double* params_host, int nparams, int flags,
@@ -714,7 +663,7 @@ int irs_smooth_finalize_peer(int system, const double* params_host, int nparams,
                              const double* x_nom, const double* u_nom, int P, int C, const float* partials,
                              const void* peer_bufs_dev, const void* peer_flags_dev, int* epoch_dev,
                              unsigned int* done_counter, long long slot_stride, int flag_stride,
-                             int rank, int world, double timeout_s, double n_total, int centered, int prepushed,
+                             int rank, int world, double timeout_s, double n_total, int centered,
                              double* At, double* Bt, double* ct, int* status, void* stream) {
     IRS_REQUIRE(system >= 0 && system < kNumSystems, "unknown system id %d", system);
     IRS_REQUIRE(partials && peer_bufs_dev && peer_flags_dev && epoch_dev && done_counter, "null pointer argument");
@@ -727,7 +676,7 @@ int irs_smooth_finalize_peer(int system, const double* params_host, int nparams,
     IRS_REQUIRE(P <= resident, "the fused exchange needs its %d blocks co-resident (%d fit): use the all-gather path", P, resident);
     PeerFusedArgs px{(double* const*)peer_bufs_dev, (int* const*)peer_flags_dev, epoch_dev, done_counter,
                      slot_stride, flag_stride, rank, world, (unsigned long long)(timeout_s * 1e9),
-                     kPeerExchange, 0, 0, 0, prepushed ? 1 : 0};
+                     kPeerExchange, 0, 0, 0};
     return smooth_finalize_impl(system, params_host, nparams, order, x_nom, u_nom, P, C, partials, nullptr, 1, 0,
                                 n_total, centered, At, Bt, ct, status, &px, stream);
 }
@@ -745,7 +694,7 @@ int irs_smooth_finalize_gather(int system, const double* params_host, int nparam
     const SystemDims dm = system_dims(system);
     IRS_REQUIRE(out_stride >= (long long)P_total * (dm.n * (dm.n + dm.m + 1) + 1), "output buffers too small");
     PeerFusedArgs px{(double* const*)peer_out_bufs_dev, (int* const*)peer_flags_dev, epoch_dev, done_counter,
-                     0, 0, rank, world, (unsigned long long)(timeout_s * 1e9), kPeerGather, p0, P_total, out_stride, 0};
+                     0, 0, rank, world, (unsigned long long)(timeout_s * 1e9), kPeerGather, p0, P_total, out_stride};
     if (P == 0) {      // this rank owns no timestep: it still takes part in the step
         peer_gather_wait_kernel<<<1, 128, 0, (cudaStream_t)stream>>>(px);
         return check_launch("peer_gather_wait_kernel");
@@ -937,21 +886,17 @@ static int tvlqr_riccati_impl(int n, int m, const double* At, const double* Bt, 
     }
     if (t_hi > 0) per_block = true;                                 // segments exist in the tiled kernel only
     const bool extra = Hinv_out != nullptr || P_out != nullptr;     // only the generic kernel writes them
-    static const bool no_tiles = getenv("IRS_TVLQR_NO_TILES") != nullptr;
     // many instances of a 4-divisible problem (quadrotor): two instances per warp, 4 x 4 register tiles
     // (tvlqr.cuh: tvlqr_riccati_packed_kernel).  That kernel's time is flat up to one block of eight instances per
     // SM (0.37 ms at T = 100 up to 1,184 instances, then 0.49 / 0.64 / 0.83 ms at 2048 / 3072 / 4096); the block
     // kernel takes 0.19 / 0.23 / 0.30 / 0.47 / 0.71 / 1.28 ms at 300 / 512 / 768 / 1024 / 2048 / 4096 and crosses it
-    // between 768 and 1024 instances (IRS_PACKED_MIN_INSTANCES; measured with tools/batched_bench.py).  Results of
-    // the two kernels agree to 1e-10 (summation order), so a shard of 512 instances and the unsharded 4096 differ at
-    // that level.  IRS_TVLQR_VARIANT=block|warp|packed overrides.
-    static const long long packed_min = [] {
-        const char* e = getenv("IRS_PACKED_MIN_INSTANCES");
-        return e && atoll(e) > 0 ? atoll(e) : 1000ll;
-    }();
+    // between 768 and 1024 instances (measured with tools/batched_bench.py).  Results of the two kernels agree to
+    // 1e-10 (summation order), so a shard of 512 instances and the unsharded 4096 differ at that level.
+    // IRS_TVLQR_VARIANT=block|warp|packed overrides.
+    constexpr long long kPackedMinInstances = 1000;
     const char* variant = getenv("IRS_TVLQR_VARIANT");
     const bool force_packed = variant != nullptr && !strcmp(variant, "packed");
-    if (n == 12 && m == 4 && !extra && t_hi == 0 && (force_packed || (variant == nullptr && I >= packed_min))) {
+    if (n == 12 && m == 4 && !extra && t_hi == 0 && (force_packed || (variant == nullptr && I >= kPackedMinInstances))) {
         auto kern = tvlqr_riccati_packed_kernel<12, 4>;
         const int smem = (int)sizeof(RicPackSmem<12, 4>);
         if (cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, smem) != cudaSuccess)
@@ -962,7 +907,7 @@ static int tvlqr_riccati_impl(int n, int m, const double* At, const double* Bt, 
     IRS_DISPATCH_DIMS(n, m, {
         if (per_block) {
             if constexpr (N_ % 2 == 0 && M_ % 2 == 0) {
-                if ((!no_tiles || t_hi > 0) && !extra) {
+                if (!extra) {
                     tvlqr_riccati_tiled_kernel<N_, M_>
                         <<<(unsigned)I, kTvlqrTiledThreads, sizeof(TvlqrTiledSmem<N_, M_>), st>>>(a);
                     return check_launch("tvlqr_riccati_tiled_kernel");

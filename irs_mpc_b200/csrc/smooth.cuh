@@ -23,20 +23,6 @@ enum SmoothFlags {
                                     // kFlagProjectAbsolute; replayed absolute points: set explicitly)
 };
 
-// Sample-sharded run with the exchange started by the ACCUMULATE kernel (smooth_tc.cuh, push_point_if_last): the block
-// that completes the last chunk of a nominal point reduces the point's chunks and stores the fp64 block into every
-// rank's exchange buffer while the rest of the launch is still sampling; the fit kernel then only waits for the
-// arrival flags (peer_exchange_point, prepushed).  world == 0: off.
-struct PeerPushArgs {
-    double* const* peer_bufs;     // [world] device array: base of each rank's exchange buffer
-    int* const* peer_flags;       // [world] device array: base of each rank's flag array [world][flag_stride]
-    const int* epoch;             // local: exchanges completed so far (advanced by the fit kernel)
-    unsigned int* counters;       // local: [P] chunks of a point finished in this launch (reset by the pushing block)
-    long long slot_stride;
-    int flag_stride;
-    int rank, world;
-};
-
 struct SmoothArgs {
     const double* x_nom;   // [P, n] nominal states
     const double* u_nom;   // [P, m] nominal inputs
@@ -52,7 +38,6 @@ struct SmoothArgs {
     int nreg;              // n + m: live entries of sigma_scaled
     SysParams prm;
     float sigma_scaled[16];   // kBoxMullerScale * sigma[c] (Philox mode), lives in the constant bank
-    PeerPushArgs push;        // exchange started by this kernel (sample-sharded tensor-core launches); world == 0: off
 };
 constexpr int kMaxRegressors = 16;
 
@@ -534,7 +519,6 @@ struct PeerFusedArgs {
     int mode;
     int p0, P_total;
     long long out_stride;
-    int prepushed;                // kPeerExchange: the accumulate kernel has reduced and pushed this rank's blocks already
 };
 enum PeerMode { kPeerNone = 0, kPeerExchange = 1, kPeerGather = 2 };
 
@@ -626,57 +610,6 @@ __device__ __forceinline__ double sum_chunks_in_order(const float* src, int C, i
     return s;
 }
 
-// The exchange of a sample-sharded step STARTED by the accumulate kernel.  Called by all BT threads of a block after
-// they have written the packed block of item (p, c): the block that completes the LAST chunk of p (device-scope
-// fence + one atomic per item: the "last block" pattern) reduces the point's chunks in fixed order — the same sums
-// peer_exchange_point would form — stores them into slot `rank` of every rank's exchange buffer, raises the arrival
-// flag of p on every rank and resets the point's counter for the next launch.  The stores travel while the other
-// blocks are still sampling.  flag_s: one int of shared memory.
-template <int BT>
-__device__ __forceinline__ void push_point_if_last(const SmoothArgs& a, int p, int width, int tid, int* flag_s) {
-    const PeerPushArgs& x = a.push;
-    // one release per BLOCK: the barrier orders the block's stores before thread 0, whose (cumulative) device-scope
-    // acq_rel atomic orders them before the count — the pattern of a cooperative-groups grid barrier.  A fence in
-    // every thread cost 54 us per launch, fence + atomic in one thread 30 us (MEMBAR.SC.GPU + CCTL.IVALL).
-    __syncthreads();
-    if (tid == 0) {
-        // release: the block's stores (ordered before this thread by the barrier) before the count; acquire: the
-        // other blocks' stores before the reads of the block that sees the last count
-        unsigned int before;
-        asm volatile("atom.add.release.gpu.global.u32 %0, [%1], 1;" : "=r"(before) : "l"(x.counters + p) : "memory");
-        const int last = before == (unsigned)(a.C - 1) ? 1 : 0;
-        if (last) asm volatile("fence.acq_rel.gpu;" ::: "memory");      // (an acquire invalidates the SM's L1: last block only)
-        *flag_s = last;
-    }
-    __syncthreads();
-    if (*flag_s == 0) return;
-    const int epoch = *reinterpret_cast<const volatile int*>(x.epoch) + 1;
-    const long long mine = ((long long)(epoch & 1) * x.world + x.rank) * x.slot_stride + (long long)p * width;
-    for (int e = tid; e < width; e += BT) {
-        const float* src = a.partials + ((long long)p * a.C) * width + e;
-        double s = 0.0;
-        int c = 0;
-        for (; c + 8 <= a.C; c += 8) {      // as sum_chunks_in_order, through L2 (written by other SMs in this launch)
-            float v[8];
-#pragma unroll
-            for (int k = 0; k < 8; ++k) v[k] = __ldcg(src + (long long)(c + k) * width);
-#pragma unroll
-            for (int k = 0; k < 8; ++k) s += (double)v[k];
-        }
-        for (; c < a.C; ++c) s += (double)__ldcg(src + (long long)c * width);
-        for (int r = 0; r < x.world; ++r) x.peer_bufs[r][mine + e] = s;      // local for r == rank
-    }
-    __syncthreads();
-    if (tid == 0) {
-        __threadfence_system();             // ONE fence: the block's (barrier-ordered) remote stores before the flags
-        for (int r = 0; r < x.world; ++r) {
-            int* remote = x.peer_flags[r] + (long long)x.rank * x.flag_stride + p;
-            asm volatile("st.relaxed.sys.global.s32 [%0], %1;" ::"l"(remote), "r"(epoch) : "memory");
-        }
-        x.counters[p] = 0u;
-    }
-}
-
 // ---------------------------------------------------------------------------------------------
 // Sample-sharded exchange FUSED into the finalize kernel (one process per GPU, peer-mapped exchange
 // buffers over NVLink / NVSwitch; torch symmetric memory provides the address exchange only).
@@ -704,21 +637,17 @@ __device__ __forceinline__ int peer_exchange_point(const FinalizeArgs& a, int p,
     const int epoch = *reinterpret_cast<volatile int*>(x.epoch) + 1;
     const long long slot0 = (long long)(epoch & 1) * x.world * x.slot_stride;
     const long long mine = slot0 + (long long)x.rank * x.slot_stride + (long long)p * width;
-    if (!x.prepushed) {
-        for (int e = tid; e < width; e += BT) {
-            const double s = sum_chunks_in_order(a.partials + ((long long)p * a.C) * width + e, a.C, width);
-            for (int r = 0; r < x.world; ++r) x.peer_bufs[r][mine + e] = s;      // local for r == rank
-        }
-        // the barrier orders the block's stores before the flag threads, whose system-scope RELEASE stores are
-        // cumulative: `world` fences per block instead of one per thread (each is a MEMBAR.SYS + L1 invalidate)
-        __syncthreads();
+    for (int e = tid; e < width; e += BT) {
+        const double s = sum_chunks_in_order(a.partials + ((long long)p * a.C) * width + e, a.C, width);
+        for (int r = 0; r < x.world; ++r) x.peer_bufs[r][mine + e] = s;      // local for r == rank
     }
+    // the barrier orders the block's stores before the flag threads, whose system-scope RELEASE stores are
+    // cumulative: `world` fences per block instead of one per thread (each is a MEMBAR.SYS + L1 invalidate)
+    __syncthreads();
     int late = 0;
     if (tid < x.world) {
-        if (!x.prepushed) {
-            int* remote = x.peer_flags[tid] + (long long)x.rank * x.flag_stride + p;
-            asm volatile("st.release.sys.global.s32 [%0], %1;" ::"l"(remote), "r"(epoch) : "memory");
-        }
+        int* remote = x.peer_flags[tid] + (long long)x.rank * x.flag_stride + p;
+        asm volatile("st.release.sys.global.s32 [%0], %1;" ::"l"(remote), "r"(epoch) : "memory");
         const int* local = x.peer_flags[x.rank] + (long long)tid * x.flag_stride + p;
         unsigned long long t0;
         asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t0));

@@ -206,7 +206,6 @@ __global__ void __launch_bounds__(128, IRS_TC_MIN_BLOCKS) smooth_zero_order_tc_k
     __shared__ float scratch[C::kRows * kScr];           // s_r[i] = D[r][z_1 col i] - D[r][z_2 col i] of r's member
     __shared__ uint16_t idx_s[C::NACC];                  // packed output e -> (i << 8) | j
     __shared__ float mom_s[C::kWarps][kMom];             // per-warp first moments of the item
-    __shared__ int push_flag_s;                          // this block completed a nominal point (push_point_if_last)
 
     const int tid = threadIdx.x, lane = tid & 31;
     // broadcast from lane 0 so that the compiler knows the warp index is warp-uniform: ring addresses,
@@ -658,8 +657,6 @@ __global__ void __launch_bounds__(128, IRS_TC_MIN_BLOCKS) smooth_zero_order_tc_k
                 out[C::NACC + tid] = v;
             }
         }
-        // sample-sharded run: the block that completes a nominal point starts the point's exchange
-        if (a.push.world > 0) push_point_if_last<C::kThreads>(a, (int)(item / a.C), C::WIDTH, tid, &push_flag_s);
         // (the next item's barriers order these scratch / mom_s reads before the next writes)
     }
     asm volatile("tcgen05.fence::before_thread_sync;");

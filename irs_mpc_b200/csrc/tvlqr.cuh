@@ -864,9 +864,6 @@ __global__ void __launch_bounds__(32 * kRolloutWarps) rollout_kernel(const Rollo
     constexpr int kSlot = CLOSED ? m * n + m : m;        // K_t | k_t   or   u_t
     constexpr int kPer = (kSlot + 31) / 32;
     __shared__ double slot[kRolloutWarps][2][kSlot];
-    // learned dynamics: the warp evaluates the network together (Mlp::step_warp), every lane carries the state
-    constexpr bool kWarpStep = is_mlp<Sys>::value;
-    __shared__ float act_s[kRolloutWarps][kWarpStep ? 2 * kMlpMaxHidden : 1];
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     const int inst = blockIdx.x * kRolloutWarps + warp;
     if (inst >= a.I) return;
@@ -895,18 +892,18 @@ __global__ void __launch_bounds__(32 * kRolloutWarps) rollout_kernel(const Rollo
     publish(0);
     __syncwarp();
     double x[n], u[m], xn[n];
-    if (lane == 0 || kWarpStep) {
+    if (lane == 0) {
 #pragma unroll
         for (int q = 0; q < n; ++q) {
             x[q] = a.x0[(long long)inst * n + q];
-            if (lane == 0) a.x_trj[((long long)inst * (a.T + 1)) * n + q] = x[q];
+            a.x_trj[((long long)inst * (a.T + 1)) * n + q] = x[q];
         }
     }
     for (int t = 0; t < a.T; ++t) {
         const long long it = (long long)inst * a.T + t;
         const double* sl = slot[warp][t & 1];
         if (t + 1 < a.T) fetch(t + 1);                 // in flight while lane 0 computes
-        if (lane == 0 || kWarpStep) {
+        if (lane == 0) {
             if (CLOSED) {
 #pragma unroll
                 for (int i = 0; i < m; ++i) {
@@ -919,18 +916,15 @@ __global__ void __launch_bounds__(32 * kRolloutWarps) rollout_kernel(const Rollo
 #pragma unroll
                 for (int i = 0; i < m; ++i) u[i] = sl[i];
             }
-        }
-        if constexpr (kWarpStep) sys.step_warp(x, u, xn, act_s[warp], act_s[warp] + kMlpMaxHidden, lane);
-        if (lane == 0 || kWarpStep) {
-            if constexpr (!kWarpStep) sys.template step<false>(x, u, xn);
-            if (CLOSED && lane == 0) {
+            sys.template step<false>(x, u, xn);
+            if (CLOSED) {
 #pragma unroll
                 for (int i = 0; i < m; ++i) a.u_trj[it * m + i] = u[i];
             }
 #pragma unroll
             for (int q = 0; q < n; ++q) {
                 x[q] = xn[q];
-                if (lane == 0) a.x_trj[((long long)inst * (a.T + 1) + t + 1) * n + q] = x[q];
+                a.x_trj[((long long)inst * (a.T + 1) + t + 1) * n + q] = x[q];
             }
         }
         if (t + 1 < a.T) publish((t + 1) & 1);

@@ -79,13 +79,6 @@ class PeerExchange:
     no NCCL call on the data path.  torch's symmetric-memory allocator is used for the address
     exchange only (plumbing).
 
-    Optional (IRS_PEER_EARLY_PUSH=1, systems whose zero-order Gram runs on the tensor cores): the exchange is STARTED
-    by the accumulate kernel (`accumulate`: the block that completes the last chunk of a point reduces and pushes the
-    point's block while the rest of the launch is still sampling) and the fit kernel only waits for the arrival
-    flags (`finalize(..., prepushed=True)`) — bit-identical sums.  Measured SLOWER than the exchange inside the fit
-    kernel (one release atomic + two block barriers per work item cost the sampling kernel 19 us per launch: 0.166
-    against 0.161 ms per step on two GPUs, 0.175 against 0.166 on eight), hence off by default.
-
     The epoch lives in device memory and is advanced by the kernel, flags are indexed by point: a
     changed horizon (fewer or more points per call) keeps the ranks in step, and the call sequence can
     be replayed from a CUDA graph.  A peer that does not deliver within `timeout_s` makes the points
@@ -110,52 +103,21 @@ class PeerExchange:
         self._hflags = symm_mem.rendezvous(self.flags, group)
         self.epoch = torch.zeros((1,), dtype=torch.int32, device=dev)
         self.counter = torch.zeros((1,), dtype=torch.int32, device=dev)
-        self.point_counters = torch.zeros((self.points,), dtype=torch.int32, device=dev)
         torch.cuda.synchronize()
         self._hflags.barrier()          # every rank's flags are zero before anyone raises one
 
     def fits(self, P, width):
         return P * width <= self.slot_stride and P <= self.flag_stride and width == self.width
 
-    @staticmethod
-    def early_push(system, order, kw):
-        """The accumulate kernel of this launch can start the exchange (tensor-core Gram, not switched off)."""
-        import os
-        if os.environ.get("IRS_PEER_EARLY_PUSH", "0") != "1" or order != smoothing.ZERO_ORDER:
-            return False
-        return _lib.lib().irs_smooth_push_supported(system.system_id, order) != 0
-
-    def accumulate(self, system, x_nom, u_nom, N, ws, sigma=None, noise=None, seed=0, it=1, stream_id=0, p0=0, i0=0,
-                   flags=0):
-        """smoothing.accumulate (zero order) whose kernel also reduces and pushes every completed point's block."""
-        import ctypes
-        P = x_nom.shape[0]
-        prm, nprm = system._params()
-        if system.batch_differs_from_scalar:
-            flags |= 1
-        ws.centered = bool(flags & (smoothing.FLAG_PROJECT_ABSOLUTE | smoothing.FLAG_CENTERED))
-        sig = None
-        if noise is None:
-            sig = np.ascontiguousarray(np.asarray(sigma, dtype=np.float32))
-            if sig.shape != (system.dim_x + system.dim_u,):
-                raise ValueError("sigma must have n + m = %d entries" % (system.dim_x + system.dim_u))
-            sig = sig.ctypes.data_as(ctypes.c_void_p)
-        _lib.call("irs_smooth_zero_order_accumulate_push", system.system_id, prm, nprm, flags, _device.ptr(x_nom),
-                  _device.ptr(u_nom), P, int(N), sig, _device.ptr(noise), int(seed), int(it), int(stream_id), int(p0),
-                  int(i0), ws.C, ws.S, _device.ptr(ws.partials), self._hbuf.buffer_ptrs_dev,
-                  self._hflags.buffer_ptrs_dev, _device.ptr(self.epoch), _device.ptr(self.point_counters),
-                  self.slot_stride, self.flag_stride, self.rank, self.world, _device.stream_ptr())
-
-    def finalize(self, system, order, x_nom, u_nom, ws, n_total, prepushed=False):
-        """Enqueue the fused reduce + exchange + fit of this step (all ranks, same order).  prepushed: the blocks
-        were sent by `accumulate`; the kernel only waits for the flags, sums over the ranks and fits."""
+    def finalize(self, system, order, x_nom, u_nom, ws, n_total):
+        """Enqueue the fused reduce + exchange + fit of this step (all ranks, same order)."""
         P = x_nom.shape[0]
         prm, nprm = system._params()
         _lib.call("irs_smooth_finalize_peer", system.system_id, prm, nprm, order, _device.ptr(x_nom),
                   _device.ptr(u_nom), P, ws.C, _device.ptr(ws.partials), self._hbuf.buffer_ptrs_dev,
                   self._hflags.buffer_ptrs_dev, _device.ptr(self.epoch), _device.ptr(self.counter),
                   self.slot_stride, self.flag_stride, self.rank, self.world, self.timeout_s, float(n_total),
-                  1 if ws.centered else 0, 1 if prepushed else 0, _device.ptr(ws.At), _device.ptr(ws.Bt),
+                  1 if ws.centered else 0, _device.ptr(ws.At), _device.ptr(ws.Bt),
                   _device.ptr(ws.ct), _device.ptr(ws.status), _device.stream_ptr())
         return ws.At, ws.Bt, ws.ct, ws.status
 
@@ -369,17 +331,11 @@ class ShardedLinearizer:
         ws = self._workspace(T, N_local, fill=True)
         px = self._peer_exchange(T, ws.width)
 
-        early = px is not None and PeerExchange.early_push(self.system, self.order, kw)
-
         def enqueue():
-            if early:
-                px.accumulate(self.system, x_nom, u_nom, N_local, ws, i0=rank * N_local, **kw)
-                px.finalize(self.system, self.order, x_nom, u_nom, ws, world * N_local, prepushed=True)
-            elif px is not None:
-                smoothing.accumulate(self.system, self.order, x_nom, u_nom, N_local, ws, i0=rank * N_local, **kw)
+            smoothing.accumulate(self.system, self.order, x_nom, u_nom, N_local, ws, i0=rank * N_local, **kw)
+            if px is not None:
                 px.finalize(self.system, self.order, x_nom, u_nom, ws, world * N_local)
             else:
-                smoothing.accumulate(self.system, self.order, x_nom, u_nom, N_local, ws, i0=rank * N_local, **kw)
                 mine = smoothing.reduce_chunks(self.system, self.order, ws)
                 everyone = gather_ranks(mine, self.group)
                 smoothing.finalize(self.system, self.order, x_nom, u_nom, ws, world * N_local,
@@ -388,7 +344,7 @@ class ShardedLinearizer:
         key = None
         if px is not None and kw.get("noise") is None and kw.get("sigma") is not None:
             # everything a captured kernel reads besides (seed, it, sigma) must be part of the key
-            key = (self.system.system_id, self.order, T, N_local, world, rank, kw.get("flags", 0), early,
+            key = (self.system.system_id, self.order, T, N_local, world, rank, kw.get("flags", 0),
                    kw.get("stream_id", 0), kw.get("p0", 0), x_nom.data_ptr(), u_nom.data_ptr(), id(px), ws.S,
                    tuple(float(v) for v in self.system.device_params()))
 

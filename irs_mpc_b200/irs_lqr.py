@@ -32,7 +32,6 @@ _USE_PIPELINE = os.environ.get("IRS_PIPELINE", "1") != "0"     # see _SampledIrs
 _PIPELINE_MIN_STEPS = 8                                        # timesteps per segment below which it does not pay
 _PIPELINE_SEGMENTS = int(os.environ.get("IRS_PIPELINE_SEGMENTS", "0"))      # 0 = sized from the work per launch
 START_BOUND_TOL = 1e-6      # tolerance of the start-state box test in local_descent
-_DESCENT_CHUNK = int(os.environ.get("IRS_DESCENT_CHUNK", "0"))           # see _SampledIrsLqr._descent_chunk
 
 
 class IrsLqrParameters:
@@ -249,16 +248,12 @@ class IrsLqr:
     def _linearize_and_riccati(self, db, x_nom, u_nom):
         """Linearization along the nominal trajectory, then the backward pass -> db["K"], db["k"]."""
         T, n, m = self.T, self.dim_x, self.dim_u
-        At, Bt, ct, status = self._descent_tv_matrices(x_nom, u_nom)
+        At, Bt, ct, status = self._tv_matrices_device(x_nom, u_nom)
         _lib.call("irs_tvlqr_riccati", n, m, _device.ptr(At), _device.ptr(Bt), _device.ptr(ct),
                   _device.ptr(self._dQ), _device.ptr(self._dQd), _device.ptr(self._dR),
                   _device.ptr(self._dxd), 0, 1, T, _device.ptr(db["K"]), _device.ptr(db["k"]),
                   _device.ptr(db["rstatus"]), _device.stream_ptr())
         return At, Bt, ct, status
-
-    def _descent_tv_matrices(self, x_nom, u_nom):
-        """The linearization inside local_descent (subclasses may plan it differently from get_TV_matrices)."""
-        return self._tv_matrices_device(x_nom, u_nom)
 
     def _graph_key(self):
         """None when this call sequence cannot be replayed from a CUDA graph (see _SampledIrsLqr)."""
@@ -479,11 +474,7 @@ class _SampledIrsLqr(IrsLqr):
     def __init__(self, system, params, sampling):
         super().__init__(system, params)
         self.sampling = sampling
-        self._ws_d = None
         self._key_cache = None
-
-    def _descent_tv_matrices(self, x_nom, u_nom):
-        return self._tv_matrices_device(x_nom, u_nom, descent=True)
 
     def _replay_noise(self, x_nom, u_nom):
         """Call the user's closure once per timestep (as the reference does) and upload."""
@@ -495,17 +486,9 @@ class _SampledIrsLqr(IrsLqr):
             rows.append(np.hstack((np.asarray(dx), np.asarray(du))).astype(np.float32))
         return _device.to_device(np.stack(rows), torch.float32)
 
-    def _tv_matrices_device(self, x_nom, u_nom, descent=False):
+    def _tv_matrices_device(self, x_nom, u_nom):
         s = self.sampling
         if isinstance(s, GaussianSampling):
-            if descent and self._descent_chunk():
-                # the linearization inside local_descent: its own workspace with the descent's chunk plan
-                # (one-pass and pipelined descents then sum in the same order: bit-identical)
-                ws = self._descent_workspace()
-                smoothing.accumulate(self.system, self.order, x_nom, u_nom, s.num_samples, ws,
-                                     sigma=s.sigma(self.iter), seed=s.seed, it=self.iter, stream_id=s.stream_id,
-                                     flags=s.flags())
-                return smoothing.finalize(self.system, self.order, x_nom, u_nom, ws, s.num_samples)
             At, Bt, ct, status, self._ws = smoothing.linearize(
                 self.system, self.order, x_nom, u_nom, s.num_samples, self._ws,
                 sigma=s.sigma(self.iter), seed=s.seed, it=self.iter, stream_id=s.stream_id,
@@ -530,28 +513,6 @@ class _SampledIrsLqr(IrsLqr):
         closer_to_nominal = float((mean - nominal).abs().sum().item()) < float(mean.abs().sum().item())
         return smoothing.FLAG_CENTERED if closer_to_nominal else 0
 
-
-    def _descent_chunk(self):
-        """Samples per chunk of the linearization INSIDE local_descent (0 = library default, which is
-        also the measured optimum: a pipelined descent samples the horizon in launches of a few timesteps,
-        and smaller chunks give such a launch more work items per SM, but at configs[2] the extra partial
-        blocks and item epilogues cost more than the fuller SMs gain — 362 us per descent with 4096-sample
-        chunks against 390-400 with 1024 and 420-435 with 512).  IRS_DESCENT_CHUNK selects another plan."""
-        if not isinstance(self.sampling, GaussianSampling) or self.order != smoothing.ZERO_ORDER:
-            return 0
-        C, _ = smoothing.plan(self.system.system_id, self.order, self.T, self.sampling.num_samples)
-        if self.T * C < 2 * RESIDENT_BLOCKS:
-            return 0
-        return _DESCENT_CHUNK
-
-    def _descent_workspace(self):
-        s = self.sampling
-        chunk = self._descent_chunk()
-        key = (self.system.system_id, self.order, self.T, s.num_samples, chunk)
-        if self._ws_d is None or self._ws_d.key != key:
-            self._ws_d = smoothing.Workspace(self.system, self.order, self.T, s.num_samples, chunk)
-        return self._ws_d
-
     def _pipeline_segments(self):
         """Timestep segments [(lo, hi), ...], late timesteps first, or None for the one-pass sequence.
         The backward Riccati pass needs the late timesteps first, so the horizon is linearized in a
@@ -567,7 +528,7 @@ class _SampledIrsLqr(IrsLqr):
         n, m, T = self.dim_x, self.dim_u, self.T
         if not _USE_PIPELINE or not isinstance(self.sampling, GaussianSampling) or n % 2 or m % 2:
             return None
-        C, _ = smoothing.plan(self.system.system_id, self.order, T, self.sampling.num_samples, self._descent_chunk())
+        C, _ = smoothing.plan(self.system.system_id, self.order, T, self.sampling.num_samples)
         return pipeline_segments(T, C, _PIPELINE_SEGMENTS)
 
     def _linearize_and_riccati(self, db, x_nom, u_nom):
@@ -576,13 +537,10 @@ class _SampledIrsLqr(IrsLqr):
             return super()._linearize_and_riccati(db, x_nom, u_nom)
         s = self.sampling
         T, n, m = self.T, self.dim_x, self.dim_u
-        if self._descent_chunk():
-            ws = self._descent_workspace()
-        else:
-            key = (self.system.system_id, self.order, T, s.num_samples)
-            if self._ws is None or self._ws.key != key:
-                self._ws = smoothing.Workspace(self.system, self.order, T, s.num_samples)
-            ws = self._ws
+        key = (self.system.system_id, self.order, T, s.num_samples)
+        if self._ws is None or self._ws.key != key:
+            self._ws = smoothing.Workspace(self.system, self.order, T, s.num_samples)
+        ws = self._ws
         if "carry" not in db:
             db["carry"] = _device.empty((n * n + n,))
             db["side"] = torch.cuda.Stream(priority=-1)        # the sequential Riccati chain

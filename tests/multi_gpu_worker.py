@@ -103,19 +103,6 @@ def main():
         A2, B2, c2, st2 = sh.linearize_n(x, u, N, **kw)
     smoothing.check_status(st2)
     report("peer exchange stable over 20 steps", torch.equal(A2, An) and torch.equal(c2, cn))
-    # the exchange started by the accumulate kernel (IRS_PEER_EARLY_PUSH=1) against the exchange inside the fit
-    # kernel (default): same sums, same bits
-    from irs_mpc_b200.distributed import PeerExchange
-    early_off = not PeerExchange.early_push(s, smoothing.ZERO_ORDER, kw)
-    os.environ["IRS_PEER_EARLY_PUSH"] = "1"
-    sh_push = ShardedLinearizer(s, smoothing.ZERO_ORDER, peer_memory=True)
-    for k in range(3):
-        Af, Bf, cf, stf = sh_push.linearize_n(x, u, N, **kw)
-    early_on = PeerExchange.early_push(s, smoothing.ZERO_ORDER, kw)
-    del os.environ["IRS_PEER_EARLY_PUSH"]
-    smoothing.check_status(stf)
-    report("early push == exchange in the fit", torch.equal(Af, An) and torch.equal(Bf, Bn) and torch.equal(cf, cn)
-           and early_on and early_off, "(opt-in path exercised: %s)" % early_on)
 
     # 2b. a horizon that shrinks and grows again on a LIVE linearizer (shrinking-horizon MPC): the
     #     exchange is reused, the ranks stay in step, and every size still equals the NCCL path

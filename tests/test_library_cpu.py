@@ -25,7 +25,7 @@ def test_header_symbols_exported_and_bound(built_lib):
         assert hasattr(built_lib, name), "library does not export %s" % name
         assert name in _lib.SIGNATURES, "no ctypes signature for %s" % name
     assert sorted(_lib.SIGNATURES) == names
-    assert built_lib.irs_abi_version() == _lib.ABI_VERSION == 3
+    assert built_lib.irs_abi_version() == _lib.ABI_VERSION == 4
 
 
 def test_system_dims_and_partial_width(built_lib):

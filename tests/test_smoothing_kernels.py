@@ -42,9 +42,9 @@ Which test reaches which instantiation through `irs_smooth_zero_order_accumulate
 |   (the centred un-shift always takes the block kernel)              | test_finalize_centred_unshift_...            |
 | finalize_first_order_kernel<Sys>                                    | test_first_order_means                       |
 
-The engine is chosen with irs_set_gram_engine and restored on leaving the `engine` block.  IRS_TC_BLOCKS_PER_SM is not used: it is read
-once per process, so item counts per block come from the shapes instead (P = 409,600 at N = 1000 makes every
-persistent block walk far more than the quadrotor's 64-item nominal batch).
+The engine is chosen with irs_set_gram_engine and restored on leaving the `engine` block.  The persistent
+tensor-core grid is sized from the kernel's occupancy, so item counts per block come from the shapes (P = 409,600
+at N = 1000 makes every persistent block walk far more than the quadrotor's 64-item nominal batch).
 """
 import numpy as np
 import pytest

@@ -16,15 +16,12 @@ from irs_mpc_b200.all import (GaussianSampling, IrsLqrParameters, IrsLqrZeroOrde
                               QuadrotorDynamics)
 
 cfg = ec.quadrotor(T=100)
-CASES = [("auto", True, 0, None)]
-for chunk in (0, 2048, 1024, 512):
-    for segs in (3, 4, 5, 6):
-        CASES.append(("%d equal" % segs, True, segs, chunk))
-CASES += [("one pass", False, 0, 0), ("one pass", False, 0, 1024), ("auto", True, 0, None)]
-for label, pipeline, segs, chunk in CASES:
+CASES = [("auto", True, 0)]
+for segs in (3, 4, 5, 6):
+    CASES.append(("%d equal" % segs, True, segs))
+CASES += [("one pass", False, 0), ("auto", True, 0)]
+for label, pipeline, segs in CASES:
     mod._USE_PIPELINE, mod._PIPELINE_SEGMENTS = pipeline, segs
-    if chunk is not None:
-        mod._DESCENT_CHUNK = chunk
     system = QuadrotorDynamics(cfg["h"])
     params = IrsLqrParameters()
     for key in ("Q", "Qd", "R", "x0", "xd_trj", "u_trj_initial", "xbound", "ubound"):
@@ -41,5 +38,5 @@ for label, pipeline, segs, chunk in CASES:
         xn, un = solver.local_descent(x, u)
         c = solver.evaluate_cost(xn, un)
     dt = (time.perf_counter() - t0) / K
-    print("%-9s chunk %-5s %s: %.1f us per descent + cost = %.0f iterations/s (cost %.6f)"
-          % (label, solver._descent_chunk(), solver._pipeline_segments(), dt * 1e6, 1 / dt, c), flush=True)
+    print("%-9s %s: %.1f us per descent + cost = %.0f iterations/s (cost %.6f)"
+          % (label, solver._pipeline_segments(), dt * 1e6, 1 / dt, c), flush=True)

@@ -50,19 +50,11 @@ def main():
         smoothing.finalize(s, 0, x, u, ws, N)
 
     res = {"accumulate": timed(acc), "accumulate+local finalize": timed(local)}
-    from irs_mpc_b200.distributed import PeerExchange
-    pxx = PeerExchange(T, ws.width)
-    res["accumulate with the push of completed points (no fit)"] = timed(
-        lambda k: pxx.accumulate(s, x, u, N, ws, seed=k, i0=rank * N, **kw))
     for graphs in (False, True):
         _graph.USE_GRAPHS = graphs
         sh = ShardedLinearizer(s, 0, peer_memory=True)
         res["fused peer finalize, graphs=%s" % graphs] = timed(lambda k: sh.linearize_n(x, u, N, seed=k, **kw))
     _graph.USE_GRAPHS = True
-    os.environ["IRS_PEER_EARLY_PUSH"] = "1"
-    she = ShardedLinearizer(s, 0, peer_memory=True)
-    res["exchange started by the sampling kernel (IRS_PEER_EARLY_PUSH=1), graphs=True"] = timed(lambda k: she.linearize_n(x, u, N, seed=k, **kw))
-    del os.environ["IRS_PEER_EARLY_PUSH"]
     shn = ShardedLinearizer(s, 0, peer_memory=False)
     res["NCCL all-gather path"] = timed(lambda k: shn.linearize_n(x, u, N, seed=k, **kw))
     _graph.USE_GRAPHS = True
