@@ -282,6 +282,38 @@ int irs_tvlqr_linear_rollout(int n, int m, const double* At, const double* Bt, c
                              const double* K, const double* k, const double* x0, int I, int T,
                              double* xs, double* us, void* stream);
 
+/* solve_tvlqr for any state and input dimension within the limits, not only those of the built-in
+ * systems (irs_tvlqr_riccati and the box solve are instantiated for those alone).  Same problem, same
+ * array layouts and the same conventions as the entries above; n and m are run-time arguments and every
+ * pair within the limits is accepted, the built-in pairs included.  Arguments are checked on the host
+ * before any launch (null pointers, n and m out of range, I < 1, T < 1, box strides, the box QP's horizon).
+ *  - irs_tvlqr_any_limits: the largest n and m (32 each).  Host only.
+ *  - irs_tvlqr_riccati_any: irs_tvlqr_riccati / irs_tvlqr_riccati_ex (Hinv_out [I,T,m,m] and P_out
+ *    [I,T+1,n,n] may each be null).  H_t is factored by a Cholesky decomposition; status[i] = 1 if a
+ *    pivot is not > 0, a K_t or k_t is not finite, or the final P holds a NaN.
+ *  - irs_tvlqr_linear_rollout_any: irs_tvlqr_linear_rollout.
+ *  - irs_tvlqr_box_qp_any: irs_tvlqr_box_solve with mpc = 0 (one QP from x0; no cost output).  K, Hinv,
+ *    P are irs_tvlqr_riccati_any's outputs for the penalty-augmented weights (Q + diag(dx)/2,
+ *    Qd + diag(dx)/2, R + diag(du)); Q, Qd, R are the problem's own weights (R is not read by the ADMM).
+ *    The ADMM state lives in shared memory: 8 (5 n T + 4 m T + 7 n + m) bytes must fit in 200 KiB
+ *    (T <= 88 at n = m = 32), otherwise the call fails before launch. */
+int irs_tvlqr_any_limits(int* max_n, int* max_m);
+int irs_tvlqr_riccati_any(int n, int m, const double* At, const double* Bt, const double* ct,
+                          const double* Q, const double* Qd, const double* R,
+                          const double* xd, long long xd_stride, int I, int T,
+                          double* K, double* k, int* status, double* Hinv_out, double* P_out, void* stream);
+int irs_tvlqr_linear_rollout_any(int n, int m, const double* At, const double* Bt, const double* ct,
+                                 const double* K, const double* k, const double* x0, int I, int T,
+                                 double* xs, double* us, void* stream);
+int irs_tvlqr_box_qp_any(int n, int m, const double* At, const double* Bt, const double* ct,
+                         const double* K, const double* Hinv, const double* P,
+                         const double* Q, const double* Qd, const double* R,
+                         const double* xd, long long xd_stride, const double* dx, const double* du,
+                         const double* xlo, const double* xhi, const double* ulo, const double* uhi,
+                         long long xbox_stride, long long ubox_stride, const double* x0,
+                         double alpha, double eps, int max_iter, int I, int T,
+                         double* x_trj, double* u_trj, int* status, int* iters, void* stream);
+
 /* IrsLqr.local_descent forward pass (irs_lqr/irs_lqr.py:169-184): u_t = K_t x_t + k_t on the TRUE
  * dynamics, plus IrsLqr.evaluate_cost (irs_lqr.py:121-137, terminal term uses Q).
  * x0 [I,n]; x_trj [I,T+1,n]; u_trj [I,T,m]; cost [I]. */

@@ -90,6 +90,12 @@ SIGNATURES = {
                             _vp, _vp, _vp, _vp, _ll, _ll, _vp, _vp, _vp, ctypes.c_double, ctypes.c_double, ctypes.c_double,
                             _i, _i, _i, _vp, _vp, _vp, _vp, _vp, _vp],
     "irs_tvlqr_linear_rollout": [_i, _i, _vp, _vp, _vp, _vp, _vp, _vp, _i, _i, _vp, _vp, _vp],
+    "irs_tvlqr_any_limits": [ctypes.POINTER(_i), ctypes.POINTER(_i)],
+    "irs_tvlqr_riccati_any": [_i, _i, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _ll, _i, _i, _vp, _vp, _vp, _vp, _vp, _vp],
+    "irs_tvlqr_linear_rollout_any": [_i, _i, _vp, _vp, _vp, _vp, _vp, _vp, _i, _i, _vp, _vp, _vp],
+    "irs_tvlqr_box_qp_any": [_i, _i, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _ll, _vp, _vp, _vp, _vp, _vp,
+                             _vp, _ll, _ll, _vp, ctypes.c_double, ctypes.c_double, _i, _i, _i, _vp, _vp, _vp, _vp,
+                             _vp],
     "irs_rollout_closed_loop": [_i, _c_double_p, _i, _vp, _vp, _vp, _vp, _ll, _vp, _vp, _i, _i,
                                 _vp, _vp, _vp, _vp],
     "irs_rollout_open_loop": [_i, _c_double_p, _i, _vp, _vp, _vp, _ll, _vp, _vp, _i, _i,

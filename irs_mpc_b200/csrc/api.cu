@@ -11,6 +11,7 @@
 #include "smooth_tc.cuh"
 #include "tvlqr.cuh"
 #include "tvlqr_box.cuh"
+#include "tvlqr_any.cuh"
 #include "cem.cuh"
 #include "smooth_mlp.cuh"
 
@@ -1022,6 +1023,89 @@ int irs_tvlqr_linear_rollout(int n, int m, const double* At, const double* Bt, c
     cudaStream_t st = (cudaStream_t)stream;
     IRS_DISPATCH_DIMS(n, m, (linear_rollout_kernel<N_, M_><<<(I + 63) / 64, 64, 0, st>>>(a, x0, xs, us)));
     return check_launch("linear_rollout_kernel");
+}
+
+// ---- run-time dimensions (tvlqr_any.cuh): every (n, m) up to kTvlqrAnyMaxDim, the built-in pairs included ----
+int irs_tvlqr_any_limits(int* max_n, int* max_m) {
+    IRS_REQUIRE(max_n && max_m, "null pointer argument");
+    *max_n = kTvlqrAnyMaxDim;
+    *max_m = kTvlqrAnyMaxDim;
+    return 0;
+}
+
+#define IRS_REQUIRE_ANY_DIMS(n, m)                                                                  \
+    IRS_REQUIRE(n >= 1 && n <= kTvlqrAnyMaxDim && m >= 1 && m <= kTvlqrAnyMaxDim,                   \
+                "TVLQR dims n=%d m=%d out of range: need 1 <= n, m <= %d", n, m, kTvlqrAnyMaxDim)
+
+int irs_tvlqr_riccati_any(int n, int m, const double* At, const double* Bt, const double* ct,
+                          const double* Q, const double* Qd, const double* R,
+                          const double* xd, long long xd_stride, int I, int T,
+                          double* K, double* k, int* status, double* Hinv_out, double* P_out, void* stream) {
+    IRS_REQUIRE_ANY_DIMS(n, m);
+    IRS_REQUIRE(At && Bt && ct && Q && Qd && R && xd && K && k && status, "null pointer argument");
+    IRS_REQUIRE(I >= 1 && T >= 1, "need I >= 1 and T >= 1");
+    IRS_REQUIRE(xd_stride >= 0, "need xd_stride >= 0");
+    TvlqrAnyArgs a{TvlqrArgs{At, Bt, ct, Q, Qd, R, xd, xd_stride, K, k, status, I, T, Hinv_out, P_out, 0, 0, nullptr},
+                   n, m};
+    const size_t smem = tvlqr_riccati_any_smem_bytes(n, m);      // 109 KiB at n = m = 32
+    if (cudaFuncSetAttribute(tvlqr_riccati_any_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem) !=
+        cudaSuccess)
+        return check_launch("cudaFuncSetAttribute(tvlqr_riccati_any_kernel)");
+    tvlqr_riccati_any_kernel<<<(unsigned)I, tvlqr_any_threads(n, m), smem, (cudaStream_t)stream>>>(a);
+    return check_launch("tvlqr_riccati_any_kernel");
+}
+
+int irs_tvlqr_linear_rollout_any(int n, int m, const double* At, const double* Bt, const double* ct,
+                                 const double* K, const double* k, const double* x0, int I, int T,
+                                 double* xs, double* us, void* stream) {
+    IRS_REQUIRE_ANY_DIMS(n, m);
+    IRS_REQUIRE(At && Bt && ct && K && k && x0 && xs && us, "null pointer argument");
+    IRS_REQUIRE(I >= 1 && T >= 1, "need I >= 1 and T >= 1");
+    TvlqrArgs a{At, Bt, ct, nullptr, nullptr, nullptr, nullptr, 0, const_cast<double*>(K),
+                const_cast<double*>(k), nullptr, I, T};
+    linear_rollout_any_kernel<<<(unsigned)((I + kRolloutAnyWarps - 1) / kRolloutAnyWarps), 32 * kRolloutAnyWarps, 0,
+                                (cudaStream_t)stream>>>(a, n, m, x0, xs, us);
+    return check_launch("linear_rollout_any_kernel");
+}
+
+int irs_tvlqr_box_qp_any(int n, int m, const double* At, const double* Bt, const double* ct,
+                         const double* K, const double* Hinv, const double* P,
+                         const double* Q, const double* Qd, const double* R,
+                         const double* xd, long long xd_stride, const double* dx, const double* du,
+                         const double* xlo, const double* xhi, const double* ulo, const double* uhi,
+                         long long xbox_stride, long long ubox_stride, const double* x0,
+                         double alpha, double eps, int max_iter, int I, int T,
+                         double* x_trj, double* u_trj, int* status, int* iters, void* stream) {
+    IRS_REQUIRE_ANY_DIMS(n, m);
+    IRS_REQUIRE(At && Bt && ct && K && Hinv && P && Q && Qd && R && xd && dx && du && xlo && xhi && ulo && uhi &&
+                    x0 && x_trj && u_trj && status && iters, "null pointer argument");
+    IRS_REQUIRE(I >= 1 && T >= 1 && max_iter >= 1, "need I >= 1, T >= 1, max_iter >= 1");
+    IRS_REQUIRE(xd_stride >= 0, "need xd_stride >= 0");
+    IRS_REQUIRE(alpha > 0.0 && alpha < 2.0 && eps > 0.0, "need 0 < alpha < 2 and eps > 0");
+    IRS_REQUIRE((xbox_stride == 0 || xbox_stride == n) && (ubox_stride == 0 || ubox_stride == m),
+                "box strides must be 0 (constant box) or n / m (one box per timestep)");
+    // the ADMM state stays in shared memory under the limit of launch_box_mpc; the per-step matrices join it
+    // when they fit too
+    constexpr size_t kLimit = 200 * 1024;
+    const size_t with_cache = box_qp_any_smem_bytes(n, m, T, true);
+    const bool cache = with_cache <= kLimit;
+    const size_t smem = cache ? with_cache : box_qp_any_smem_bytes(n, m, T, false);
+    if (smem > kLimit) {
+        int t_max = 0;
+        while (box_qp_any_smem_bytes(n, m, t_max + 1, false) <= kLimit) ++t_max;
+        set_error("horizon T=%d too long for the shared-memory resident ADMM state at n=%d m=%d: "
+                  "the longest is T=%d (%zu bytes of shared memory at most)", T, n, m, t_max, kLimit);
+        return 1;
+    }
+    BoxQpAnyArgs a{At, Bt, ct, K, Hinv, P, Q, Qd, xd, xd_stride, dx, du, xlo, xhi, ulo, uhi, xbox_stride,
+                   ubox_stride, x0, alpha, eps, max_iter, x_trj, u_trj, status, iters, I, T, n, m};
+    (void)R;      // the ADMM step only needs the augmented matrices; R is part of the problem's description
+    cudaStream_t st = (cudaStream_t)stream;
+    auto kern = cache ? box_qp_any_kernel<true> : box_qp_any_kernel<false>;
+    if (cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem) != cudaSuccess)
+        return check_launch("cudaFuncSetAttribute(box_qp_any_kernel)");
+    kern<<<(unsigned)I, 32, smem, st>>>(a);
+    return check_launch("box_qp_any_kernel");
 }
 
 int irs_rollout_closed_loop(int system, const double* params_host, int nparams,

@@ -17,7 +17,17 @@ to the quasistatic drivers and is not implemented.
 Start state: the reference also boxes xt[0] = x0 (:113-114), so an x0 outside x_bound_abs[:, 0] makes
 the QP infeasible; reproduced (ValueError).  xinit / uinit are initial guesses of an iterative solver;
 the solves here are direct (or warm-started internally) and ignore them.
+
+Dimensions: the reference takes (At, Bt, ...) of any shape.  The kernels of csrc/tvlqr.cuh and
+csrc/tvlqr_box.cuh are unrolled over the dimensions of the built-in systems, (2,1), (5,2), (6,2) and
+(12,4), and those pairs take them.  Every other pair with 1 <= n, m <= 32 (`tvlqr_any_limits`) takes the
+kernels of csrc/tvlqr_any.cuh, which get n and m at run time: the same recursion, rollout and ADMM, so
+the same minimiser.  Beyond the limits solve_tvlqr raises NotImplementedError.  A bounded solve at
+n = m = 32 accepts horizons up to T = 88 (the ADMM state is kept in shared memory).
 """
+import ctypes
+import functools
+
 import numpy as np
 import torch
 
@@ -135,6 +145,73 @@ class _DimsOnlySystem:
         return _lib.params_array(self._p)
 
 
+@functools.lru_cache(maxsize=None)
+def tvlqr_any_limits():
+    """(max_n, max_m) of the run-time-dimension kernels (csrc/tvlqr_any.cuh).  Host only."""
+    max_n, max_m = ctypes.c_int(), ctypes.c_int()
+    _lib.call("irs_tvlqr_any_limits", ctypes.byref(max_n), ctypes.byref(max_m))
+    return max_n.value, max_m.value
+
+
+def _builtin_dims(n, m):
+    """True: (n, m) is a built-in system's pair and takes the compile-time kernels; False: the run-time
+    kernels; NotImplementedError beyond their limits."""
+    if (n, m) in _DimsOnlySystem._BY_DIMS:
+        return True
+    max_n, max_m = tvlqr_any_limits()
+    if not (1 <= n <= max_n and 1 <= m <= max_m):
+        raise NotImplementedError("TVLQR with n=%d states and m=%d inputs: the kernels take 1 <= n <= %d and "
+                                  "1 <= m <= %d" % (n, m, max_n, max_m))
+    return False
+
+
+def riccati_any_device(At, Bt, ct, Q, Qd, R, xd, xd_stride, hessians=False):
+    """riccati_device for any (n, m) within tvlqr_any_limits -> K, k, status and, with hessians, also
+    Hinv [I,T,m,m] and P [I,T+1,n,n] (else None, None)."""
+    I, T, n, _ = At.shape
+    m = Bt.shape[3]
+    K = _device.empty((I, T, m, n))
+    k = _device.empty((I, T, m))
+    status = _device.empty((I,), torch.int32)
+    Hinv = _device.empty((I, T, m, m)) if hessians else None
+    P = _device.empty((I, T + 1, n, n)) if hessians else None
+    _lib.call("irs_tvlqr_riccati_any", n, m, _device.ptr(At), _device.ptr(Bt), _device.ptr(ct),
+              _device.ptr(Q), _device.ptr(Qd), _device.ptr(R), _device.ptr(xd), int(xd_stride),
+              I, T, _device.ptr(K), _device.ptr(k), _device.ptr(status),
+              _device.ptr(Hinv) if hessians else None, _device.ptr(P) if hessians else None, _device.stream_ptr())
+    return K, k, status, Hinv, P
+
+
+def box_qp_any_device(At, Bt, ct, dQ, dQd, dR, Q, Qd, R, dxd, xd_stride, x0, xlo, xhi, ulo, uhi,
+                      rho0=BOX_RHO0, alpha=BOX_ALPHA, eps=BOX_EPS, max_iter=BOX_MAX_ITER):
+    """One bounded QP from x0 (box_solve_device with mpc=False) for any (n, m) within tvlqr_any_limits.
+    Returns device tensors (x_trj [I,T+1,n], u_trj [I,T,m], status [I], iters [I])."""
+    I, T, n, _ = At.shape
+    m = Bt.shape[3]
+    dx, du = box_penalties(Q, R, rho0)
+    Qe = _device.to_device(np.asarray(Q, dtype=np.float64) + 0.5 * np.diag(dx))
+    Qde = _device.to_device(np.asarray(Qd, dtype=np.float64) + 0.5 * np.diag(dx))
+    Re = _device.to_device(np.asarray(R, dtype=np.float64) + np.diag(du))      # halved inside the kernel
+    K, _, rstatus, Hinv, P = riccati_any_device(At, Bt, ct, Qe, Qde, Re, dxd, xd_stride, hessians=True)
+    x_trj = _device.empty((I, T + 1, n))
+    u_trj = _device.empty((I, T, m))
+    status = _device.empty((I,), torch.int32)
+    iters = _device.empty((I,), torch.int32)
+    d = {name: _device.to_device(np.ascontiguousarray(v, dtype=np.float64))
+         for name, v in (("dx", dx), ("du", du), ("xlo", xlo), ("xhi", xhi), ("ulo", ulo), ("uhi", uhi))}
+    xbox_stride = n if np.ndim(xlo) == 2 else 0
+    ubox_stride = m if np.ndim(ulo) == 2 else 0
+    if (xbox_stride and np.shape(xlo) != (T + 1, n)) or (ubox_stride and np.shape(ulo) != (T, m)):
+        raise ValueError("time-varying boxes must be [T+1, n] (states) and [T, m] (inputs)")
+    _lib.call("irs_tvlqr_box_qp_any", n, m, _device.ptr(At), _device.ptr(Bt), _device.ptr(ct), _device.ptr(K),
+              _device.ptr(Hinv), _device.ptr(P), _device.ptr(dQ), _device.ptr(dQd), _device.ptr(dR),
+              _device.ptr(dxd), int(xd_stride), _device.ptr(d["dx"]), _device.ptr(d["du"]), _device.ptr(d["xlo"]),
+              _device.ptr(d["xhi"]), _device.ptr(d["ulo"]), _device.ptr(d["uhi"]), xbox_stride, ubox_stride,
+              _device.ptr(x0), float(alpha), float(eps), int(max_iter), I, T, _device.ptr(x_trj),
+              _device.ptr(u_trj), _device.ptr(status), _device.ptr(iters), _device.stream_ptr())
+    return x_trj, u_trj, status | rstatus, iters
+
+
 def _box_rows(bound, rows, dim, name):
     """The reference indexes its bounds by timestep (x_bound_abs[0, t]: tv_lqr.py:113-116): accepts
     [2, rows, dim] (or [2, dim], broadcast over the horizon) -> (lo, hi), each [dim] when the box is
@@ -170,6 +247,7 @@ def solve_tvlqr(At, Bt, ct, Q, Qd, R, x0, x_trj_d, solver=None, indices_u_into_x
     At = np.asarray(At, dtype=np.float64)
     Bt = np.asarray(Bt, dtype=np.float64)
     T, n, m = At.shape[0], At.shape[1], Bt.shape[2]
+    builtin = _builtin_dims(n, m)
     ct = np.asarray(ct, dtype=np.float64).reshape(T, n)
     dA = _device.to_device(At[None])
     dB = _device.to_device(Bt[None])
@@ -177,10 +255,13 @@ def solve_tvlqr(At, Bt, ct, Q, Qd, R, x0, x_trj_d, solver=None, indices_u_into_x
     dQ, dQd, dR = _device.to_device(Q), _device.to_device(Qd), _device.to_device(R)
     dxd = _device.to_device(np.asarray(x_trj_d, dtype=np.float64)[:T + 1])
     dx0 = _device.to_device(np.asarray(x0, dtype=np.float64)[None])
-    K, k, status = riccati_device(dA, dB, dc, dQ, dQd, dR, dxd, 0)
+    if builtin:
+        K, k, status = riccati_device(dA, dB, dc, dQ, dQd, dR, dxd, 0)
+    else:
+        K, k, status, _, _ = riccati_any_device(dA, dB, dc, dQ, dQd, dR, dxd, 0)
     xs = _device.empty((1, T + 1, n))
     us = _device.empty((1, T, m))
-    _lib.call("irs_tvlqr_linear_rollout", n, m, _device.ptr(dA), _device.ptr(dB), _device.ptr(dc),
+    _lib.call("irs_tvlqr_linear_rollout" if builtin else "irs_tvlqr_linear_rollout_any", n, m, _device.ptr(dA), _device.ptr(dB), _device.ptr(dc),
               _device.ptr(K), _device.ptr(k), _device.ptr(dx0), 1, T, _device.ptr(xs),
               _device.ptr(us), _device.stream_ptr())
     if int(status.item()) != 0:
@@ -204,8 +285,11 @@ def solve_tvlqr(At, Bt, ct, Q, Qd, R, x0, x_trj_d, solver=None, indices_u_into_x
     if not (x_active or u_active):
         return xs, us
     # an absolute bound is active: box-constrained QP (tv_lqr.py:113-118, :132-134)
-    xb, ub, _, bstatus, _ = box_solve_device(_DimsOnlySystem(n, m), False, dA, dB, dc, dQ, dQd, dR, Q, Qd, R,
-                                             dxd, 0, dx0, xlo, xhi, ulo, uhi)
+    if builtin:
+        xb, ub, _, bstatus, _ = box_solve_device(_DimsOnlySystem(n, m), False, dA, dB, dc, dQ, dQd, dR, Q, Qd, R,
+                                                 dxd, 0, dx0, xlo, xhi, ulo, uhi)
+    else:
+        xb, ub, bstatus, _ = box_qp_any_device(dA, dB, dc, dQ, dQd, dR, Q, Qd, R, dxd, 0, dx0, xlo, xhi, ulo, uhi)
     if int(bstatus.item()) != 0:
         raise ValueError(TVLQR_FAILED)
     return _device.to_numpy(xb[0]), _device.to_numpy(ub[0])
