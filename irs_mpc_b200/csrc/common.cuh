@@ -134,6 +134,72 @@ __device__ __forceinline__ float2 ffma2(float2 a, float2 b, float2 c) {
     return *reinterpret_cast<float2*>(&ud);
 }
 
+// ---------------------------------------------------------------------------------------------
+// fp32 arithmetic with every rounding explicit, on one value (float) or on both halves of a float2 in
+// one instruction (FADD2 / FMUL2 / FFMA2).  Nothing is contracted or re-associated, so one source
+// rounds identically on either type, lane by lane.  ptxas folds a splat into the .F32 (broadcast)
+// operand selector and a negated pair into the operand's sign modifier: neither costs an instruction.
+// ---------------------------------------------------------------------------------------------
+template <typename V>
+struct Lanes;
+
+template <>
+struct Lanes<float> {
+    static __device__ __forceinline__ float splat(float a) { return a; }
+    static __device__ __forceinline__ float neg(float a) { return -a; }
+    static __device__ __forceinline__ float add(float a, float b) { return __fadd_rn(a, b); }
+    static __device__ __forceinline__ float sub(float a, float b) { return __fsub_rn(a, b); }
+    static __device__ __forceinline__ float mul(float a, float b) { return __fmul_rn(a, b); }
+    static __device__ __forceinline__ float fma(float a, float b, float c) { return __fmaf_rn(a, b, c); }
+    static __device__ __forceinline__ float rcp(float a) { return Math<float>::rcp(a); }
+};
+
+#define IRS_F32X2_BINARY(OP)                                                                            \
+    float2 d;                                                                                           \
+    asm("{\n\t.reg .b64 a, b, d;\n\tmov.b64 a, {%2, %3};\n\tmov.b64 b, {%4, %5};\n\t" OP             \
+        ".rn.f32x2 d, a, b;\n\tmov.b64 {%0, %1}, d;\n\t}"                                               \
+        : "=f"(d.x), "=f"(d.y)                                                                          \
+        : "f"(a.x), "f"(a.y), "f"(b.x), "f"(b.y));                                                      \
+    return d;
+
+template <>
+struct Lanes<float2> {
+    static __device__ __forceinline__ float2 splat(float a) { return make_float2(a, a); }
+    static __device__ __forceinline__ float2 neg(float2 a) { return make_float2(-a.x, -a.y); }
+    static __device__ __forceinline__ float2 add(float2 a, float2 b) { IRS_F32X2_BINARY("add") }
+    static __device__ __forceinline__ float2 sub(float2 a, float2 b) { IRS_F32X2_BINARY("sub") }
+    static __device__ __forceinline__ float2 mul(float2 a, float2 b) { IRS_F32X2_BINARY("mul") }
+    static __device__ __forceinline__ float2 fma(float2 a, float2 b, float2 c) {
+        float2 d;
+        asm("{\n\t.reg .b64 a, b, c, d;\n\tmov.b64 a, {%2, %3};\n\tmov.b64 b, {%4, %5};\n\tmov.b64 c, {%6, %7};\n\t"
+            "fma.rn.f32x2 d, a, b, c;\n\tmov.b64 {%0, %1}, d;\n\t}"
+            : "=f"(d.x), "=f"(d.y)
+            : "f"(a.x), "f"(a.y), "f"(b.x), "f"(b.y), "f"(c.x), "f"(c.y));
+        return d;
+    }
+    static __device__ __forceinline__ float2 rcp(float2 a) { return make_float2(Math<float>::rcp(a.x), Math<float>::rcp(a.y)); }
+};
+#undef IRS_F32X2_BINARY
+
+// box_muller_raw on the word pairs (wa0, wb0) -> e01 and (wa1, wb1) -> e23 with the float arithmetic of the
+// two packed: the bits of two box_muller_raw calls.
+__device__ __forceinline__ void box_muller_raw_x2(uint32_t wa0, uint32_t wb0, uint32_t wa1, uint32_t wb1,
+                                                  float2& e01, float2& e23) {
+    using L = Lanes<float2>;
+    const float2 u = L::sub(L::splat(2.0f), make_float2(unit_float(wa0), unit_float(wa1)));
+    const float2 ang = L::mul(make_float2(unit_float(wb0), unit_float(wb1)), L::splat(6.283185307179586f));
+    float l2a, l2b, ra, rb;
+    asm("lg2.approx.ftz.f32 %0, %1;" : "=f"(l2a) : "f"(u.x));
+    asm("lg2.approx.ftz.f32 %0, %1;" : "=f"(l2b) : "f"(u.y));
+    asm("sqrt.approx.ftz.f32 %0, %1;" : "=f"(ra) : "f"(-l2a));
+    asm("sqrt.approx.ftz.f32 %0, %1;" : "=f"(rb) : "f"(-l2b));
+    float sa, ca, sb, cb;
+    __sincosf(ang.x, &sa, &ca);
+    __sincosf(ang.y, &sb, &cb);
+    e01 = L::mul(L::splat(ra), make_float2(ca, sa));
+    e23 = L::mul(L::splat(rb), make_float2(cb, sb));
+}
+
 __device__ __forceinline__ float warp_sum(float v) {
 #pragma unroll
     for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);

@@ -78,6 +78,23 @@ __device__ __forceinline__ void philox_normals(const SmoothArgs& a, int p, unsig
     }
 }
 
+// Counter block j of philox_normals (w[4 j .. 4 j + 3]) for an antithetic pair evaluated in packed FP32
+// (smooth_tc.cuh: kTcPaired): zz[q] = (w[4 j + q], w[4 j + q]), the bits of philox_normals in both halves of
+// a register pair; Box-Muller and the sigma scaling run packed.  Entries past d are left unset.
+template <class Sys>
+__device__ __forceinline__ void philox_normals_x2(const SmoothArgs& a, int p, unsigned long long ctr0, int j,
+                                                  float2 (&zz)[4]) {
+    uint32_t r[4];
+    philox4x32((uint32_t)ctr0, a.p0 + (uint32_t)p, (a.iter << 8) | (uint32_t)j, a.stream, a.seed_lo, a.seed_hi, r);
+    float2 e01, e23;
+    box_muller_raw_x2(r[0], r[1], r[2], r[3], e01, e23);
+    const float e[4] = {e01.x, e01.y, e23.x, e23.y};
+#pragma unroll
+    for (int q = 0; q < 4; ++q)
+        if (4 * j + q < Sys::D)
+            zz[q] = Lanes<float2>::mul(Lanes<float2>::splat(a.sigma_scaled[4 * j + q]), Lanes<float2>::splat(e[q]));
+}
+
 // Deltas of sample i of nominal point p: replayed from a.noise or drawn from the Philox stream.
 // MODE: -1 = decided at run time, 0 = Philox, 1 = replay (a compile-time mode keeps the test and the
 // other path's code out of the hot loop).

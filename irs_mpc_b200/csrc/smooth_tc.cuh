@@ -181,8 +181,11 @@ enum TcMode { kTcPhilox = 0, kTcReplay = 1, kTcPaired = 2 };
 // the nominal point (kFlagProjectAbsolute, or replayed absolute points with kFlagCentered) and their
 // first moments [sum z' | sum dF] are appended to the packed block — per-lane fp32 sums of a few dozen
 // values each, reduced by shuffles, so they carry far less rounding noise than a running sum.
+// The packed pair evaluation asks for five resident blocks explicitly: left at the common cap, ptxas gives it 101
+// registers (four blocks per SM); at 96 it needs no spills and one more instruction per pair.
 template <class Sys, int NSTAGE, int MODE, bool CENTERED>
-__global__ void __launch_bounds__(128, IRS_TC_MIN_BLOCKS) smooth_zero_order_tc_kernel(const SmoothArgs a) {
+__global__ void __launch_bounds__(128, MODE == kTcPaired && has_step_pair<Sys>::value ? 5 : IRS_TC_MIN_BLOCKS)
+    smooth_zero_order_tc_kernel(const SmoothArgs a) {
     // three_cart pairs whose regressors are projected stage both members in one tile
     constexpr bool DUAL = MODE == kTcPaired && Sys::kHasProjection;
     using C = TcCfg<Sys, DUAL>;
@@ -410,6 +413,31 @@ __global__ void __launch_bounds__(128, IRS_TC_MIN_BLOCKS) smooth_zero_order_tc_k
                 sys.template step<false>(xu, xu + n, f);
             }
         };
+        // w = [z | f(x̄ + z) - f(x̄ - z)] of an antithetic pair, both members evaluated at once in the two halves
+        // of packed FP32 registers: half the issue slots of two scalar evaluations, the same bits.  z arrives in
+        // both halves of a register pair, so (x̄ + z, x̄ - z) is one FADD2 whose operand negates the high half.
+        auto pair_row = [&](unsigned long long pair, float (&w)[C::RS]) {
+            if constexpr (has_step_pair<Sys>::value) {
+                float2 xu2[d], f2[n];
+#pragma unroll
+                for (int j = 0; j < (d + 3) / 4; ++j) {     // block by block: a block's z pairs die at once
+                    float2 zz[4];
+                    philox_normals_x2<Sys>(a, p, pair, j, zz);
+                    const float4 v = nom4[j];
+                    const float xb[4] = {v.x, v.y, v.z, v.w};
+#pragma unroll
+                    for (int k = 0; k < 4; ++k) {
+                        if (4 * j + k < d) {
+                            w[4 * j + k] = zz[k].x;
+                            xu2[4 * j + k] = Lanes<float2>::add(Lanes<float2>::splat(xb[k]), make_float2(zz[k].x, -zz[k].y));
+                        }
+                    }
+                }
+                sys.step_pair(xu2, xu2 + n, f2);
+#pragma unroll
+                for (int q = 0; q < n; ++q) w[d + q] = f2[q].x - f2[q].y;
+            }
+        };
         // w[d ..] = scale (f - fbar)
         auto minus_nominal_response = [&](const float (&f)[n], float (&w)[C::RS], float scale) {
 #pragma unroll
@@ -519,25 +547,29 @@ __global__ void __launch_bounds__(128, IRS_TC_MIN_BLOCKS) smooth_zero_order_tc_k
                 if constexpr (DUAL) two_rows = pair_rows;
                 if (!two_rows) {
                     if (have_plus) {
-                        philox_normals<Sys, C::RS>(a, p, pair, w);
-                        float xu[kXU], fp[n];
-                        load_xu(xu);
-#pragma unroll
-                        for (int q = 0; q < d; ++q) xu[q] += w[q];
-                        dynamics(xu, fp);
-                        if (have_minus) {
-                            float fm[n];
+                        if (has_step_pair<Sys>::value && have_minus) {
+                            pair_row(pair, w);
+                        } else {
+                            philox_normals<Sys, C::RS>(a, p, pair, w);
+                            float xu[kXU], fp[n];
                             load_xu(xu);
 #pragma unroll
-                            for (int q = 0; q < d; ++q) xu[q] -= w[q];
-                            dynamics(xu, fm);
+                            for (int q = 0; q < d; ++q) xu[q] += w[q];
+                            dynamics(xu, fp);
+                            if (have_minus) {
+                                float fm[n];
+                                load_xu(xu);
 #pragma unroll
-                            for (int q = 0; q < n; ++q) w[d + q] = fp[q] - fm[q];
-                        } else {
-                            // lone + member at the end of an odd chunk: [z / sqrt 2 | sqrt 2 (f+ - fbar)]
-                            minus_nominal_response(fp, w, 1.41421356237309505f);
+                                for (int q = 0; q < d; ++q) xu[q] -= w[q];
+                                dynamics(xu, fm);
 #pragma unroll
-                            for (int q = 0; q < d; ++q) w[q] *= 0.70710678118654752f;
+                                for (int q = 0; q < n; ++q) w[d + q] = fp[q] - fm[q];
+                            } else {
+                                // lone + member at the end of an odd chunk: [z / sqrt 2 | sqrt 2 (f+ - fbar)]
+                                minus_nominal_response(fp, w, 1.41421356237309505f);
+#pragma unroll
+                                for (int q = 0; q < d; ++q) w[q] *= 0.70710678118654752f;
+                            }
                         }
                     } else {
                         zero_row(w);

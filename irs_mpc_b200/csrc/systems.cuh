@@ -161,8 +161,63 @@ struct Quadrotor {
         Math<R>::sincos(x[5], sc[4], sc[5]);
         step_trig<BATCH>(x, u, sc, o);
     }
+    // Both members of an antithetic pair at once, x = (x̄ + z, x̄ − z) in the two halves of every float2
+    // (smooth_tc.cuh, kTcPaired): each half gets the bits step<false> gives that member alone.
+    __device__ __forceinline__ void step_pair(const float2* x, const float2* u, float2* o) const {
+        float2 sc[6];
+#pragma unroll
+        for (int j = 0; j < 3; ++j) {
+            Math<float>::sincos(x[3 + j].x, sc[2 * j].x, sc[2 * j + 1].x);
+            Math<float>::sincos(x[3 + j].y, sc[2 * j].y, sc[2 * j + 1].y);
+        }
+        step_lanes(x, u, sc, o);
+    }
     template <bool BATCH>
     __device__ __forceinline__ void step_trig(const R* x, const R* u, const R* sc, R* o) const {
+        if constexpr (std::is_same<R, float>::value) step_lanes(x, u, sc, o);
+        else step_trig_fp64(x, u, sc, o);
+    }
+    // The fp32 step on one sample (V = float) or on two (V = float2), every rounding explicit: the
+    // contractions are those nvcc chose for the expression form below, so both keep their former bits.
+    template <typename V>
+    __device__ __forceinline__ void step_lanes(const V* x, const V* u, const V* sc, V* o) const {
+        using L = Lanes<V>;
+        const V sr = sc[0], cr = sc[1], sp = sc[2], cp = sc[3], sy = sc[4], cy = sc[5];
+        const V icp = L::rcp(cp);
+        const V rd0 = x[9], rd1 = x[10], rd2 = x[11];
+        const V hh = L::splat(h);
+        const V s03 = L::add(u[0], u[3]), s12 = L::add(u[1], u[2]);
+        const V Fz = L::mul(L::splat(kF), L::add(s03, s12));
+        const V M0 = L::mul(L::splat(LkF), L::sub(L::add(u[2], u[3]), L::add(u[0], u[1])));
+        const V M1 = L::mul(L::splat(LkF), L::sub(s12, s03));
+        const V M2 = L::mul(L::splat(kM), L::sub(L::add(u[1], u[3]), L::add(u[0], u[2])));
+        const V a = L::mul(Fz, L::splat(inv_mass));
+        const V spcr = L::mul(sp, cr);
+        o[6] = L::fma(hh, L::mul(a, L::fma(sy, sr, L::mul(cy, spcr))), x[6]);
+        o[7] = L::fma(hh, L::mul(a, L::fma(sy, spcr, L::neg(L::mul(cy, sr)))), x[7]);
+        o[8] = L::fma(hh, L::fma(a, L::mul(cp, cr), L::splat(-g)), x[8]);
+        const V cprd2 = L::mul(cp, rd2);
+        const V p = L::fma(L::neg(sp), rd2, rd0);
+        const V q = L::fma(cr, rd1, L::mul(sr, cprd2));
+        const V r = L::fma(cr, cprd2, L::neg(L::mul(sr, rd1)));
+        const V pd_I0 = L::fma(L::splat(dI12), L::mul(q, r), M0);       // pd * I0
+        const V qd = L::mul(L::fma(L::splat(dI20), L::mul(r, p), M1), L::splat(inv_I1));
+        const V rdd = L::mul(L::fma(L::splat(dI01), L::mul(p, q), M2), L::splat(inv_I2));
+        const V tp = L::mul(sp, icp);
+        const V icp2 = L::mul(icp, icp);
+        const V srq_crr = L::fma(sr, q, L::mul(cr, r));
+        const V crq_srr = L::fma(cr, q, L::neg(L::mul(sr, r)));
+        const V srqd_crrd = L::fma(sr, qd, L::mul(cr, rdd));
+        o[9] = L::fma(hh, L::fma(rd1, L::mul(icp2, srq_crr),
+                                 L::fma(rd0, L::mul(tp, crq_srr), L::fma(pd_I0, L::splat(inv_I0), L::mul(tp, srqd_crrd)))),
+                      x[9]);
+        o[10] = L::fma(hh, L::fma(L::neg(rd0), srq_crr, L::fma(cr, qd, L::neg(L::mul(sr, rdd)))), x[10]);
+        o[11] = L::fma(hh, L::fma(rd1, L::mul(L::mul(tp, icp), srq_crr), L::fma(rd0, L::mul(icp, crq_srr), L::mul(icp, srqd_crrd))),
+                       x[11]);
+#pragma unroll
+        for (int i = 0; i < 6; ++i) o[i] = L::fma(hh, x[6 + i], x[i]);     // kinematics; next_angle for i >= 3
+    }
+    __device__ __forceinline__ void step_trig_fp64(const R* x, const R* u, const R* sc, R* o) const {
         const R sr = sc[0], cr = sc[1], sp = sc[2], cp = sc[3], sy = sc[4], cy = sc[5];
         const R icp = Math<R>::rcp(cp);
         const R rd0 = x[9], rd1 = x[10], rd2 = x[11];
@@ -512,6 +567,12 @@ template <class Sys>
 struct is_mlp : std::false_type {};
 template <typename R, int N_, int M_>
 struct is_mlp<Mlp<R, N_, M_>> : std::true_type {};
+
+// systems with step_pair (both members of an antithetic pair in packed FP32)
+template <class Sys>
+struct has_step_pair : std::false_type {};
+template <>
+struct has_step_pair<Quadrotor<float>> : std::true_type {};
 
 // Host-side dimension table (kept in sync with the functors by static_asserts in api.cu).
 struct SystemDims {
