@@ -6,4 +6,4 @@ Host side: Python, same call surface as hjsuh94/irs_mpc (`DynamicalSystem`, `Irs
 """
 from . import _lib  # noqa: F401
 
-__all__ = ["all", "dynamical_system", "irs_lqr", "sampling", "smoothing", "systems", "tv_lqr"]
+__all__ = ["all", "dynamical_system", "irs_lqr", "sampling", "smoothing", "systems", "tv_lqr", "user_system"]

@@ -19,13 +19,17 @@ USE_GRAPHS = os.environ.get("IRS_CUDA_GRAPH", "1") != "0"
 
 
 class GraphRunner:
-    def __init__(self):
+    """lib: the library whose entry points the captured sequence calls (the accumulate node is looked up
+    in that library's capture state)."""
+
+    def __init__(self, lib=_lib.MAIN):
+        self._lib = lib
         self._slots = {}
 
     def reset(self):
         for slot in self._slots.values():
             if slot[1] is not None:
-                _lib.call("irs_graph_destroy", slot[1])
+                self._lib.call("irs_graph_destroy", slot[1])
         self._slots = {}
 
     def run(self, name, key, enqueue, update=None):
@@ -38,7 +42,7 @@ class GraphRunner:
         slot = self._slots.get(name)
         if slot is None or slot[0] != key:
             if slot is not None and slot[1] is not None:
-                _lib.call("irs_graph_destroy", slot[1])
+                self._lib.call("irs_graph_destroy", slot[1])
             self._slots[name] = [key, None, 1]        # key, graph handle, eager calls so far
             enqueue()
             return
@@ -50,7 +54,7 @@ class GraphRunner:
             side = torch.cuda.Stream()
             side.wait_stream(torch.cuda.current_stream())
             with torch.cuda.stream(side):
-                _lib.call("irs_graph_begin", side.cuda_stream)
+                self._lib.call("irs_graph_begin", side.cuda_stream)
                 handle = ctypes.c_void_p()
                 try:
                     enqueue()
@@ -58,13 +62,13 @@ class GraphRunner:
                     # end the capture (a stream must not stay in capture mode), drop the partial graph and
                     # let the ORIGINAL exception propagate
                     try:
-                        _lib.call("irs_graph_end", side.cuda_stream, ctypes.byref(handle))
-                        _lib.call("irs_graph_destroy", handle)
+                        self._lib.call("irs_graph_end", side.cuda_stream, ctypes.byref(handle))
+                        self._lib.call("irs_graph_destroy", handle)
                     except _lib.IrsCudaError:
                         pass
                     raise
-                _lib.call("irs_graph_end", side.cuda_stream, ctypes.byref(handle))
+                self._lib.call("irs_graph_end", side.cuda_stream, ctypes.byref(handle))
             slot[1] = handle
         if update is not None:
             update(slot[1])
-        _lib.call("irs_graph_launch", slot[1], _device.stream_ptr())
+        self._lib.call("irs_graph_launch", slot[1], _device.stream_ptr())

@@ -110,39 +110,66 @@ SIGNATURES = {
 }
 _RESTYPES = {"irs_last_error": ctypes.c_char_p}
 
-_lib = None
-
 
 class IrsCudaError(RuntimeError):
     pass
 
 
+class Library:
+    """One build of the C ABI: the main library, or the library of a user-written system
+    (user_system.py), which exports the same entry points.  Loaded on first use."""
+
+    _by_path = {}
+
+    def __init__(self, path):
+        self.path = path
+        self._handle = None
+
+    @classmethod
+    def at(cls, path):
+        """The one Library object of `path` (one dlopen per library and process)."""
+        path = os.path.abspath(path)
+        if path not in cls._by_path:
+            cls._by_path[path] = cls(path)
+        return cls._by_path[path]
+
+    def handle(self):
+        """Load (once) and return the ctypes handle.  Raises if the library has not been built."""
+        if self._handle is None:
+            if not os.path.exists(self.path):
+                raise ImportError(
+                    "irs_mpc_b200: %s not found. Build it with `python -c 'import __graft_entry__ as g; "
+                    "g.build()'` (needs nvcc). There is no CPU fallback." % self.path)
+            handle = ctypes.CDLL(self.path)
+            for name, argtypes in SIGNATURES.items():
+                fn = getattr(handle, name)
+                fn.argtypes = argtypes
+                fn.restype = _RESTYPES.get(name, ctypes.c_int)
+            if handle.irs_abi_version() != ABI_VERSION:
+                raise ImportError("irs_mpc_b200: ABI version mismatch in %s" % self.path)
+            self._handle = handle
+        return self._handle
+
+    def call(self, name, *args):
+        """Invoke an entry point; translate a non-zero status into IrsCudaError(message)."""
+        handle = self.handle()
+        rc = getattr(handle, name)(*args)
+        if rc != 0:
+            raise IrsCudaError("%s failed: %s" % (name, handle.irs_last_error().decode()))
+        return rc
+
+
+MAIN = Library.at(LIB_PATH)
+
+
 def lib():
-    """Load (once) and return the ctypes handle.  Raises if the library has not been built."""
-    global _lib
-    if _lib is None:
-        if not os.path.exists(LIB_PATH):
-            raise ImportError(
-                "irs_mpc_b200: %s not found. Build it with `python -c 'import __graft_entry__ as g; "
-                "g.build()'` (needs nvcc). There is no CPU fallback." % LIB_PATH)
-        handle = ctypes.CDLL(LIB_PATH)
-        for name, argtypes in SIGNATURES.items():
-            fn = getattr(handle, name)
-            fn.argtypes = argtypes
-            fn.restype = _RESTYPES.get(name, ctypes.c_int)
-        if handle.irs_abi_version() != ABI_VERSION:
-            raise ImportError("irs_mpc_b200: ABI version mismatch in %s" % LIB_PATH)
-        _lib = handle
-    return _lib
+    """Load (once) and return the ctypes handle of the main library."""
+    return MAIN.handle()
 
 
 def call(name, *args):
-    """Invoke an entry point; translate a non-zero status into IrsCudaError(message)."""
-    handle = lib()
-    rc = getattr(handle, name)(*args)
-    if rc != 0:
-        raise IrsCudaError("%s failed: %s" % (name, handle.irs_last_error().decode()))
-    return rc
+    """Invoke an entry point of the main library."""
+    return MAIN.call(name, *args)
 
 
 def params_array(values):

@@ -9,3 +9,4 @@ from .sampling import GaussianSampling  # noqa: F401
 from .systems import (BicycleDynamics, MlpDynamics, PendulumDynamics, QuadrotorDynamics,  # noqa: F401
                       ThreeCartDynamics)
 from .tv_lqr import get_solver, solve_tvlqr  # noqa: F401
+from .user_system import CudaSourceDynamics  # noqa: F401

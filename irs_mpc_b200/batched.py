@@ -91,7 +91,7 @@ class BatchedIrsLqrZeroOrder:
     # -- device launches ------------------------------------------------------------------------
     def _rollout_open(self, x0, u, x_out, cost_out):
         prm, nprm = self.system._params()
-        _lib.call("irs_rollout_open_loop", self.system.system_id, prm, nprm, _device.ptr(u),
+        self.system.lib.call("irs_rollout_open_loop", self.system.system_id, prm, nprm, _device.ptr(u),
                   _device.ptr(x0), _device.ptr(self._dxd), self._xd_stride, _device.ptr(self._dQ),
                   _device.ptr(self._dR), self.I, self.T, _device.ptr(x_out), _device.ptr(cost_out),
                   _device.stream_ptr())
@@ -115,12 +115,12 @@ class BatchedIrsLqrZeroOrder:
         (x_new [I,T+1,n], u_new [I,T,m], cost_new [I]).  No host synchronisation."""
         I, T, n, m = self.I, self.T, self.dim_x, self.dim_u
         At, Bt, ct, self._sstatus = self.linearize()
-        _lib.call("irs_tvlqr_riccati", n, m, _device.ptr(At), _device.ptr(Bt), _device.ptr(ct),
+        self.system.lib.call("irs_tvlqr_riccati", n, m, _device.ptr(At), _device.ptr(Bt), _device.ptr(ct),
                   _device.ptr(self._dQ), _device.ptr(self._dQd), _device.ptr(self._dR),
                   _device.ptr(self._dxd), self._xd_stride, I, T, _device.ptr(self._K),
                   _device.ptr(self._k), _device.ptr(self._rstatus), _device.stream_ptr())
         prm, nprm = self.system._params()
-        _lib.call("irs_rollout_closed_loop", self.system.system_id, prm, nprm, _device.ptr(self._K),
+        self.system.lib.call("irs_rollout_closed_loop", self.system.system_id, prm, nprm, _device.ptr(self._K),
                   _device.ptr(self._k), _device.ptr(self.x_trj[:, 0, :].contiguous()),
                   _device.ptr(self._dxd), self._xd_stride, _device.ptr(self._dQ), _device.ptr(self._dR),
                   I, T, _device.ptr(self._x_new), _device.ptr(self._u_new), _device.ptr(self._cost_new),
@@ -128,7 +128,7 @@ class BatchedIrsLqrZeroOrder:
         if self._box is not None:
             from .tv_lqr import BOUND_TOL
             xlo, xhi, ulo, uhi = self._box
-            _lib.call("irs_tvlqr_plan_check", n, m, _device.ptr(At), _device.ptr(Bt), _device.ptr(ct),
+            self.system.lib.call("irs_tvlqr_plan_check", n, m, _device.ptr(At), _device.ptr(Bt), _device.ptr(ct),
                       _device.ptr(self._K), _device.ptr(self._k), _device.ptr(self._x_new), _device.ptr(xlo),
                       _device.ptr(xhi), _device.ptr(ulo), _device.ptr(uhi), BOUND_TOL, I, T, 0,
                       _device.ptr(self._violated), _device.ptr(self._plan_scratch), _device.stream_ptr())

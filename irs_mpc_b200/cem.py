@@ -104,7 +104,7 @@ class CrossEntropyMethod:
         x_trj = _device.empty((B, self.T + 1, self.dim_x))
         cost = _device.empty((B,))
         prm, nprm = self.system._params()
-        _lib.call("irs_rollout_open_loop", self.system.system_id, prm, nprm, _device.ptr(ud),
+        self.system.lib.call("irs_rollout_open_loop", self.system.system_id, prm, nprm, _device.ptr(ud),
                   _device.ptr(x0d), _device.ptr(self._dxd), 0, _device.ptr(self._dQ),
                   _device.ptr(self._dR), B, self.T, _device.ptr(x_trj), _device.ptr(cost),
                   _device.stream_ptr())
@@ -118,7 +118,7 @@ class CrossEntropyMethod:
         x = _device.to_device(np.asarray(x_trj, dtype=np.float64).reshape(1, self.T + 1, self.dim_x))
         u = _device.to_device(np.asarray(u_trj, dtype=np.float64).reshape(1, self.T, self.dim_u))
         cost = _device.empty((1,))
-        _lib.call("irs_evaluate_cost", self.dim_x, self.dim_u, _device.ptr(x), _device.ptr(u),
+        self.system.lib.call("irs_evaluate_cost", self.dim_x, self.dim_u, _device.ptr(x), _device.ptr(u),
                   _device.ptr(self._dxd), 0, _device.ptr(self._dQ), _device.ptr(self._dR), 1, self.T,
                   _device.ptr(cost), _device.stream_ptr())
         return float(cost.item())
@@ -137,7 +137,7 @@ class CrossEntropyMethod:
         cost = _device.empty((B,))
         prm, nprm = self.system._params()
         # 2. roll all of them out and cost them: one kernel launch
-        _lib.call("irs_rollout_open_loop", self.system.system_id, prm, nprm, _device.ptr(ud),
+        self.system.lib.call("irs_rollout_open_loop", self.system.system_id, prm, nprm, _device.ptr(ud),
                   _device.ptr(x0d), _device.ptr(self._dxd), 0, _device.ptr(self._dQ),
                   _device.ptr(self._dR), B, T, _device.ptr(x_cand), _device.ptr(cost), _device.stream_ptr())
         # 3.-4. the n_elite cheapest, mean and std over them — on the device; out = [mean | std | x of the mean]
@@ -145,10 +145,10 @@ class CrossEntropyMethod:
         out = _device.empty((2 * T * m + (T + 1) * n + 1,))
         mean, std = out[:T * m].view(1, T, m), out[T * m:2 * T * m]
         x_new = out[2 * T * m:2 * T * m + (T + 1) * n].view(1, T + 1, n)
-        _lib.call("irs_cem_refit", _device.ptr(cost), _device.ptr(ud), B, T, m, int(self.n_elite),
+        self.system.lib.call("irs_cem_refit", _device.ptr(cost), _device.ptr(ud), B, T, m, int(self.n_elite),
                   _device.ptr(elite), _device.ptr(mean), _device.ptr(std), _device.stream_ptr())
         # rollout of the new mean (cem.py:183)
-        _lib.call("irs_rollout_open_loop", self.system.system_id, prm, nprm, _device.ptr(mean),
+        self.system.lib.call("irs_rollout_open_loop", self.system.system_id, prm, nprm, _device.ptr(mean),
                   _device.ptr(x0d), _device.ptr(self._dxd), 0, _device.ptr(self._dQ),
                   _device.ptr(self._dR), 1, T, _device.ptr(x_new), _device.ptr(out[-1:]), _device.stream_ptr())
         h = _device.to_numpy(out)

@@ -45,7 +45,11 @@ static std::vector<MlpEntry> g_mlps;
 static std::mutex g_mlp_mutex;
 
 static int load_params(int system, const double* params_host, int nparams, SysParams* out) {
+#ifndef IRS_USER_SYSTEM
     static const int expected[kNumSystems] = {1, 1, 9, 2, 2};
+#else
+    static const int expected[kNumSystems] = {1, 1, 9, 2, 2, IRS_USER_NPARAMS};
+#endif
     IRS_REQUIRE(system >= 0 && system < kNumSystems, "unknown system id %d", system);
     IRS_REQUIRE(params_host != nullptr && nparams == expected[system],
                 "system %d expects %d parameters, got %d", system, expected[system], nparams);
@@ -117,6 +121,10 @@ static int gram_engine() {
 }
 static bool use_tensor_cores(int system) {
     const int e = gram_engine();
+#ifdef IRS_USER_SYSTEM
+    // user system: CUDA cores up to 8 regressors (as for pendulum and bicycle), tcgen05 above
+    if (e == -1) return system == kUser && UserSystem<float>::D > 8;
+#endif
     if (e == -1) return system == kQuadrotor || system == kThreeCart;   // measured: see DESIGN.md
     return e == 1;
 }
@@ -222,6 +230,30 @@ static int launch_zero_order_tc(const SmoothArgs& a, cudaStream_t st) {
     }
     return launch_zero_order_tc_centered<Sys, false>(a, st);
 }
+
+#ifdef IRS_USER_SYSTEM
+// CUDA-core Gram engine of the user system: the whole block in every thread's registers up to 8 regressors;
+// above that its rows are split over the four warps of a block (the quadrotor's layout), which needs a split
+// that gives every warp the same number of outputs.
+static int launch_zero_order_user(const SmoothArgs& a, cudaStream_t st) {
+    using Sys = UserSystem<float>;
+    if constexpr (Sys::D <= 8) {
+        return launch_zero_order<Sys, 1>(a, st);
+    } else {
+        using C = ZeroOrderCfg<Sys, 4>;
+        constexpr int NP = role_pairs(C::d, C::Wp, 4, 0);
+        if constexpr (role_pairs(C::d, C::Wp, 4, 1) == NP && role_pairs(C::d, C::Wp, 4, 2) == NP &&
+                      role_pairs(C::d, C::Wp, 4, 3) == NP) {
+            IRS_REQUIRE(a.S % 128 == 0, "chunk size must be a multiple of 128");
+            return launch_zero_order<Sys, 4>(a, st);
+        } else {
+            set_error("the CUDA-core Gram engine cannot split the rows of d = %d regressors evenly over four warps: "
+                      "use the tensor-core engine (irs_set_gram_engine(-1) or (1))", Sys::D);
+            return 1;
+        }
+    }
+}
+#endif
 
 static int fill_smooth_args(SmoothArgs* a, int system, const double* params_host, int nparams,
                             int flags, const double* x_nom, const double* u_nom, int P, long long N,
@@ -357,6 +389,9 @@ static int jacobian_batch_impl(int system, const double* params_host, int nparam
     if (load_params(system, params_host, nparams, &prm)) return 1;
     IRS_REQUIRE(system != kThreeCart,
                 "three_cart is not differentiable and has no Jacobian (three_cart_dynamics.py:20)");
+#ifdef IRS_USER_SYSTEM
+    IRS_REQUIRE(UserSystem<double>::kHasJacobian, "the user system was built without a Jacobian body");
+#endif
     IRS_REQUIRE(B >= 0, "negative batch");
     if (B == 0) return 0;
     IRS_REQUIRE(x && u && J, "null pointer argument");
@@ -366,12 +401,26 @@ static int jacobian_batch_impl(int system, const double* params_host, int nparam
     return check_launch("jacobian_batch_kernel");
 }
 
+#ifndef IRS_USER_SYSTEM
 #define IRS_DISPATCH_DIMS(n, m, ...)                                                \
     if (n == 2 && m == 1) { constexpr int N_ = 2, M_ = 1; __VA_ARGS__; }            \
     else if (n == 5 && m == 2) { constexpr int N_ = 5, M_ = 2; __VA_ARGS__; }       \
     else if (n == 12 && m == 4) { constexpr int N_ = 12, M_ = 4; __VA_ARGS__; }     \
     else if (n == 6 && m == 2) { constexpr int N_ = 6, M_ = 2; __VA_ARGS__; }       \
     else { irs::set_error("unsupported TVLQR dims n=%d m=%d", n, m); return 1; }
+#else
+// A user library holds the compile-time LQR kernels of its own system's pair only.  The Riccati pass and the
+// linear rollout of a pair that is not a built-in one take the run-time-dimension kernels (tvlqr_any.cuh):
+// the templated Riccati kernel's Cholesky is built for m in {1, 2, 4}, the tiled and packed kernels for fixed
+// shapes.
+#define IRS_DISPATCH_DIMS(n, m, ...)                                                                     \
+    if (n == IRS_USER_N && m == IRS_USER_M) { constexpr int N_ = IRS_USER_N, M_ = IRS_USER_M; __VA_ARGS__; } \
+    else { irs::set_error("unsupported TVLQR dims n=%d m=%d (this library is built for n=%d m=%d)", n, m,  \
+                          IRS_USER_N, IRS_USER_M); return 1; }
+#define IRS_USER_BUILTIN_DIMS                                                                             \
+    ((IRS_USER_N == 2 && IRS_USER_M == 1) || (IRS_USER_N == 5 && IRS_USER_M == 2) ||                      \
+     (IRS_USER_N == 12 && IRS_USER_M == 4) || (IRS_USER_N == 6 && IRS_USER_M == 2))
+#endif
 
 }  // namespace irs
 
@@ -483,13 +532,18 @@ int irs_smooth_zero_order_accumulate(int system, const double* params_host, int 
     cudaStream_t st = (cudaStream_t)stream;
     if (use_tensor_cores(system)) {
         switch (system) {
+#ifndef IRS_USER_SYSTEM
             case kPendulum: return launch_zero_order_tc<Pendulum<float>>(a, st);
             case kBicycle: return launch_zero_order_tc<Bicycle<float>>(a, st);
             case kThreeCart: return launch_zero_order_tc<ThreeCart<float>>(a, st);
             case kQuadrotor: return launch_zero_order_tc<Quadrotor<float>>(a, st);
+#else
+            case kUser: return launch_zero_order_tc<UserSystem<float>>(a, st);
+#endif
         }
     }
     switch (system) {
+#ifndef IRS_USER_SYSTEM
         case kPendulum: return launch_zero_order<Pendulum<float>, 1>(a, st);
         case kBicycle: return launch_zero_order<Bicycle<float>, 1>(a, st);
         case kThreeCart: return launch_zero_order<ThreeCart<float>, 1>(a, st);
@@ -500,6 +554,9 @@ int irs_smooth_zero_order_accumulate(int system, const double* params_host, int 
             IRS_REQUIRE(S % 128 == 0, "quadrotor chunk size must be a multiple of 128");
             // 16 regressors: the Gram rows are split over the 4 warps of a block sharing one sample tile
             return launch_zero_order<Quadrotor<float>, 4>(a, st);
+#else
+        case kUser: return launch_zero_order_user(a, st);
+#endif
     }
     set_error("unknown system id %d", system);
     return 1;
@@ -520,6 +577,7 @@ int irs_smooth_first_order_accumulate(int system, const double* params_host, int
     cudaStream_t st = (cudaStream_t)stream;
     const unsigned grid = (unsigned)((long long)P * C);
     switch (system) {
+#ifndef IRS_USER_SYSTEM
         case kPendulum:
             g_last_smooth_func = (const void*)smooth_first_order_kernel<Pendulum<float>>;
             smooth_first_order_kernel<Pendulum<float>><<<grid, 128, 0, st>>>(a);
@@ -536,6 +594,17 @@ int irs_smooth_first_order_accumulate(int system, const double* params_host, int
             g_last_smooth_func = (const void*)smooth_first_order_kernel<Mlp21<float>>;
             smooth_first_order_kernel<Mlp21<float>><<<grid, 128, 0, st>>>(a);
             break;
+#else
+        case kUser:
+            if constexpr (UserSystem<float>::kHasJacobian) {
+                g_last_smooth_func = (const void*)smooth_first_order_kernel<UserSystem<float>>;
+                smooth_first_order_kernel<UserSystem<float>><<<grid, 128, 0, st>>>(a);
+                break;
+            } else {
+                set_error("the user system was built without a Jacobian body: no first-order smoothing");
+                return 1;
+            }
+#endif
         default: set_error("unknown system id %d", system); return 1;
     }
     return check_launch("smooth_first_order_kernel");
@@ -568,10 +637,21 @@ static int finalize_resident_blocks(int system, int order, int* out) {
                                  &per_sm, finalize_zero_order_kernel<Sys, kFinalizeThreads>, kFinalizeThreads, 0)));
     } else {
         switch (system) {
+#ifndef IRS_USER_SYSTEM
             case kPendulum: e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, finalize_first_order_kernel<Pendulum<double>>, kFinalizeThreads, 0); break;
             case kBicycle: e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, finalize_first_order_kernel<Bicycle<double>>, kFinalizeThreads, 0); break;
             case kQuadrotor: e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, finalize_first_order_kernel<Quadrotor<double>>, kFinalizeThreads, 0); break;
             case kMlp21: e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, finalize_first_order_kernel<Mlp21<double>>, kFinalizeThreads, 0); break;
+#else
+            case kUser:
+                if constexpr (UserSystem<double>::kHasJacobian) {
+                    e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, finalize_first_order_kernel<UserSystem<double>>, kFinalizeThreads, 0);
+                    break;
+                } else {
+                    set_error("system %d has no first-order path", system);
+                    return 1;
+                }
+#endif
             default: set_error("system %d has no first-order path", system); return 1;
         }
     }
@@ -636,10 +716,21 @@ static int smooth_finalize_impl(int system, const double* params_host, int npara
         }
     } else {
         switch (system) {
+#ifndef IRS_USER_SYSTEM
             case kPendulum: finalize_first_order_kernel<Pendulum<double>><<<grid, kFinalizeThreads, 0, st>>>(a); break;
             case kBicycle: finalize_first_order_kernel<Bicycle<double>><<<grid, kFinalizeThreads, 0, st>>>(a); break;
             case kQuadrotor: finalize_first_order_kernel<Quadrotor<double>><<<grid, kFinalizeThreads, 0, st>>>(a); break;
             case kMlp21: finalize_first_order_kernel<Mlp21<double>><<<grid, kFinalizeThreads, 0, st>>>(a); break;
+#else
+            case kUser:
+                if constexpr (UserSystem<double>::kHasJacobian) {
+                    finalize_first_order_kernel<UserSystem<double>><<<grid, kFinalizeThreads, 0, st>>>(a);
+                    break;
+                } else {
+                    set_error("the user system was built without a Jacobian body: no first-order smoothing");
+                    return 1;
+                }
+#endif
             default: set_error("unknown system id %d", system); return 1;
         }
     }
@@ -718,10 +809,21 @@ int irs_exact_linearize(int system, const double* params_host, int nparams,
     IRS_REQUIRE(P >= 1, "need at least one nominal point");
     cudaStream_t st = (cudaStream_t)stream;
     switch (system) {
+#ifndef IRS_USER_SYSTEM
         case kPendulum: exact_linearize_kernel<Pendulum<double>><<<(P + 63) / 64, 64, 0, st>>>(prm, x_nom, u_nom, P, At, Bt, ct); break;
         case kBicycle: exact_linearize_kernel<Bicycle<double>><<<(P + 63) / 64, 64, 0, st>>>(prm, x_nom, u_nom, P, At, Bt, ct); break;
         case kQuadrotor: exact_linearize_kernel<Quadrotor<double>><<<(P + 63) / 64, 64, 0, st>>>(prm, x_nom, u_nom, P, At, Bt, ct); break;
         case kMlp21: exact_linearize_kernel<Mlp21<double>><<<(P + 63) / 64, 64, 0, st>>>(prm, x_nom, u_nom, P, At, Bt, ct); break;
+#else
+        case kUser:
+            if constexpr (UserSystem<double>::kHasJacobian) {
+                exact_linearize_kernel<UserSystem<double>><<<(P + 63) / 64, 64, 0, st>>>(prm, x_nom, u_nom, P, At, Bt, ct);
+                break;
+            } else {
+                set_error("the user system was built without a Jacobian body: no exact linearization");
+                return 1;
+            }
+#endif
         default: set_error("unknown system id %d", system); return 1;
     }
     return check_launch("exact_linearize_kernel");
@@ -874,6 +976,10 @@ static int tvlqr_riccati_impl(int n, int m, const double* At, const double* Bt, 
                     "segmented Riccati needs even n, m (n=%d, m=%d)", n, m);
         IRS_REQUIRE((t_lo == 0 && t_hi == T) || carry != nullptr, "a partial segment needs the carry buffer");
     }
+#if defined(IRS_USER_SYSTEM) && !IRS_USER_BUILTIN_DIMS
+    IRS_REQUIRE(t_hi == 0, "segmented Riccati is not built for n=%d m=%d", n, m);
+    return irs_tvlqr_riccati_any(n, m, At, Bt, ct, Q, Qd, R, xd, xd_stride, I, T, K, k, status, Hinv_out, P_out, stream);
+#else
     cudaStream_t st = (cudaStream_t)stream;
     // few instances: one block per instance (latency); many: one warp per instance (throughput) —
     // except where the register-tiled block kernel applies (even n, m): it moves half the shared-memory
@@ -897,6 +1003,7 @@ static int tvlqr_riccati_impl(int n, int m, const double* At, const double* Bt, 
     constexpr long long kPackedMinInstances = 1000;
     const char* variant = getenv("IRS_TVLQR_VARIANT");
     const bool force_packed = variant != nullptr && !strcmp(variant, "packed");
+#if !defined(IRS_USER_SYSTEM) || (IRS_USER_N == 12 && IRS_USER_M == 4)
     if (n == 12 && m == 4 && !extra && t_hi == 0 && (force_packed || (variant == nullptr && I >= kPackedMinInstances))) {
         auto kern = tvlqr_riccati_packed_kernel<12, 4>;
         const int smem = (int)sizeof(RicPackSmem<12, 4>);
@@ -905,6 +1012,9 @@ static int tvlqr_riccati_impl(int n, int m, const double* At, const double* Bt, 
         kern<<<(unsigned)((I + kRicPackPerBlock - 1) / kRicPackPerBlock), kRicPackThreads, smem, st>>>(a);
         return check_launch("tvlqr_riccati_packed_kernel");
     }
+#else
+    (void)force_packed;
+#endif
     IRS_DISPATCH_DIMS(n, m, {
         if (per_block) {
             if constexpr (N_ % 2 == 0 && M_ % 2 == 0) {
@@ -922,6 +1032,7 @@ static int tvlqr_riccati_impl(int n, int m, const double* At, const double* Bt, 
         }
     });
     return check_launch("tvlqr_riccati_kernel");
+#endif
 }
 
 int irs_tvlqr_riccati(int n, int m, const double* At, const double* Bt, const double* ct,
@@ -1003,11 +1114,15 @@ int irs_tvlqr_box_solve(int system, const double* params_host, int nparams, int 
     a.x_trj = x_trj;  a.u_trj = u_trj;  a.cost = cost;  a.status = status;  a.iters = iters;  a.I = I;  a.T = T;
     cudaStream_t st = (cudaStream_t)stream;
     switch (system) {
+#ifndef IRS_USER_SYSTEM
         case kPendulum: return launch_box_mpc<Pendulum<double>>(a, st);
         case kBicycle: return launch_box_mpc<Bicycle<double>>(a, st);
         case kQuadrotor: return launch_box_mpc<Quadrotor<double>>(a, st);
         case kThreeCart: return launch_box_mpc<ThreeCart<double>>(a, st);
         case kMlp21: return launch_box_mpc<Mlp21<double>>(a, st);
+#else
+        case kUser: return launch_box_mpc<UserSystem<double>>(a, st);
+#endif
     }
     set_error("unknown system id %d", system);
     return 1;
@@ -1018,11 +1133,15 @@ int irs_tvlqr_linear_rollout(int n, int m, const double* At, const double* Bt, c
                              double* xs, double* us, void* stream) {
     IRS_REQUIRE(At && Bt && ct && K && k && x0 && xs && us, "null pointer argument");
     IRS_REQUIRE(I >= 1 && T >= 1, "need I >= 1 and T >= 1");
+#if defined(IRS_USER_SYSTEM) && !IRS_USER_BUILTIN_DIMS
+    return irs_tvlqr_linear_rollout_any(n, m, At, Bt, ct, K, k, x0, I, T, xs, us, stream);
+#else
     TvlqrArgs a{At, Bt, ct, nullptr, nullptr, nullptr, nullptr, 0, const_cast<double*>(K),
                 const_cast<double*>(k), nullptr, I, T};
     cudaStream_t st = (cudaStream_t)stream;
     IRS_DISPATCH_DIMS(n, m, (linear_rollout_kernel<N_, M_><<<(I + 63) / 64, 64, 0, st>>>(a, x0, xs, us)));
     return check_launch("linear_rollout_kernel");
+#endif
 }
 
 // ---- run-time dimensions (tvlqr_any.cuh): every (n, m) up to kTvlqrAnyMaxDim, the built-in pairs included ----

@@ -513,10 +513,14 @@ constexpr FinalizeTables make_finalize_tables(int n, int m) {
         for (int c = 0; c <= r; ++c, ++e) { t.tri_r[e] = (unsigned char)r;  t.tri_c[e] = (unsigned char)c; }
     return t;
 }
-// indexed by SystemId: pendulum, bicycle, quadrotor, three_cart, learned 2/1
+// indexed by SystemId: pendulum, bicycle, quadrotor, three_cart, learned 2/1 (, the user system)
 __device__ const FinalizeTables g_finalize_tables[kNumSystems] = {
     make_finalize_tables(2, 1), make_finalize_tables(5, 2), make_finalize_tables(12, 4), make_finalize_tables(6, 2),
+#ifdef IRS_USER_SYSTEM
+    make_finalize_tables(2, 1), make_finalize_tables(IRS_USER_N, IRS_USER_M)};
+#else
     make_finalize_tables(2, 1)};
+#endif
 
 // Fused sample-sharded exchange (one process per GPU, peer-mapped buffers over NVLink): see
 // peer_exchange_point below.  world == 0: not sharded.

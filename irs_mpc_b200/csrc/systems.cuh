@@ -17,7 +17,17 @@
 
 namespace irs {
 
+#ifndef IRS_USER_SYSTEM
 enum SystemId { kPendulum = 0, kBicycle = 1, kQuadrotor = 2, kThreeCart = 3, kMlp21 = 4, kNumSystems = 5 };
+#else
+// A library built around one user-written system (irs_mpc_b200/user_system.py generates the translation
+// unit): its functor is irs::UserSystem<R>, defined after this header with IRS_USER_N states, IRS_USER_M
+// inputs and IRS_USER_NPARAMS parameters (h first).  The system dispatch of such a library holds that system
+// alone.
+enum SystemId { kPendulum = 0, kBicycle = 1, kQuadrotor = 2, kThreeCart = 3, kMlp21 = 4, kUser = 5, kNumSystems = 6 };
+template <typename R>
+struct UserSystem;
+#endif
 
 // ---------------------------------------------------------------------------------------------
 // parameter i in the functor's scalar type: fp32 reads the host-rounded mirror
@@ -585,11 +595,22 @@ inline SystemDims system_dims(int id) {
         case kQuadrotor: return {12, 4, IRS_QUAD_NJ};
         case kThreeCart: return {6, 2, 0};
         case kMlp21: return {2, 1, 6};
+#ifdef IRS_USER_SYSTEM
+        case kUser: return {IRS_USER_N, IRS_USER_M, IRS_USER_N * (IRS_USER_N + IRS_USER_M)};
+#endif
         default: return {0, 0, 0};
     }
 }
 
 // Dispatch a generic lambda-like functor over the system id:  IRS_DISPATCH_SYSTEM(id, R, Sys, {...})
+#ifdef IRS_USER_SYSTEM
+#define IRS_DISPATCH_SYSTEM(id, R, SYS, ...)                                                        \
+    switch (id) {                                                                                   \
+        case irs::kUser: { using SYS = irs::UserSystem<R>; __VA_ARGS__; break; }                    \
+        default: irs::set_error("this library holds the user system (id %d) only, got id %d", (int)irs::kUser, id); \
+                 return 1;                                                                          \
+    }
+#else
 #define IRS_DISPATCH_SYSTEM(id, R, SYS, ...)                                   \
     switch (id) {                                                              \
         case irs::kPendulum: { using SYS = irs::Pendulum<R>; __VA_ARGS__; break; }   \
@@ -599,5 +620,6 @@ inline SystemDims system_dims(int id) {
         case irs::kMlp21: { using SYS = irs::Mlp21<R>; __VA_ARGS__; break; }         \
         default: irs::set_error("unknown system id %d", id); return 1;         \
     }
+#endif
 
 }  // namespace irs

@@ -190,6 +190,9 @@ class ShardedLinearizer:
     def __init__(self, system, order, group=None, peer_memory=None, peer_timeout_s=None):
         """peer_memory: None = use the fused peer-memory exchange when symmetric memory can be set up
         (NCCL all-gather otherwise), False = always NCCL, True = require it."""
+        if getattr(system, "lib", _lib.MAIN) is not _lib.MAIN:
+            raise NotImplementedError("sharded multi-GPU linearization is built for the library's own systems; "
+                                      "a CudaSourceDynamics runs on one GPU")
         self.system, self.order, self.group = system, order, group
         self._ws = None
         self._peer_memory = peer_memory

@@ -40,6 +40,13 @@ class CudaDynamicalSystem(DynamicalSystem):
     system_id = -1
     system_name = ""
     batch_differs_from_scalar = False   # only three_cart (SURVEY Appendix A-4)
+    lib = _lib.MAIN                     # the library holding the functor (user systems: their own)
+    riccati_segments = True             # the library has the segmented Riccati kernel for (dim_x, dim_u)
+
+    @property
+    def system_key(self):
+        """Tells systems apart in workspace and CUDA-graph cache keys (user systems all have one id)."""
+        return self.system_id
 
     def device_params(self):
         """Parameter vector in the order documented in include/irs_mpc_b200.h."""
@@ -62,7 +69,7 @@ class CudaDynamicalSystem(DynamicalSystem):
         out = _device.empty((B, self.dim_x), dtype)
         prm, nprm = self._params()
         fn = "irs_dynamics_batch_f64" if dtype == torch.float64 else "irs_dynamics_batch_f32"
-        _lib.call(fn, self.system_id, prm, nprm, int(batch_variant), _device.ptr(xd),
+        self.lib.call(fn, self.system_id, prm, nprm, int(batch_variant), _device.ptr(xd),
                   _device.ptr(ud), _device.ptr(out), B, _device.stream_ptr())
         return _device.to_numpy(out).astype(np.float64)
 
@@ -86,7 +93,7 @@ class CudaDynamicalSystem(DynamicalSystem):
         J = _device.empty((B, self.dim_x, self.dim_x + self.dim_u), dtype)
         prm, nprm = self._params()
         fn = "irs_jacobian_xu_batch_f64" if dtype == torch.float64 else "irs_jacobian_xu_batch_f32"
-        _lib.call(fn, self.system_id, prm, nprm, _device.ptr(xd), _device.ptr(ud), _device.ptr(J),
+        self.lib.call(fn, self.system_id, prm, nprm, _device.ptr(xd), _device.ptr(ud), _device.ptr(J),
                   B, _device.stream_ptr())
         return _device.to_numpy(J).astype(np.float64)
 

@@ -77,7 +77,7 @@ class IrsLqr:
         self._dxd = _device.to_device(np.asarray(self.xd_trj, dtype=np.float64)[:self.T + 1])
         self._ws = None
         self._db = None
-        self._graphs = GraphRunner()
+        self._graphs = GraphRunner(system.lib)
         self._last_descent = None
 
         self.x_trj = self.rollout(self.x0, self.u_trj)
@@ -100,7 +100,8 @@ class IrsLqr:
             raise RuntimeError(
                 "Could not evaluate dynamics. irs_mpc_b200 runs the dynamics as CUDA functors: the "
                 "system must derive from CudaDynamicalSystem (pendulum, bicycle, quadrotor, "
-                "three_cart); there is no CPU fallback for arbitrary Python dynamics.")
+                "three_cart, or your own dynamics as CUDA C++ source in CudaSourceDynamics); there is "
+                "no CPU fallback for arbitrary Python dynamics.")
         try:
             system.dynamics(np.zeros(system.dim_x), np.zeros(system.dim_u))
         except _lib.IrsCudaError:
@@ -123,7 +124,7 @@ class IrsLqr:
         x_trj = _device.empty((1, self.T + 1, self.dim_x))
         cost = _device.empty((1,))
         prm, nprm = self.system._params()
-        _lib.call("irs_rollout_open_loop", self.system.system_id, prm, nprm, _device.ptr(u),
+        self.system.lib.call("irs_rollout_open_loop", self.system.system_id, prm, nprm, _device.ptr(u),
                   _device.ptr(x0d), _device.ptr(self._dxd), 0, _device.ptr(self._dQ),
                   _device.ptr(self._dR), 1, self.T, _device.ptr(x_trj), _device.ptr(cost),
                   _device.stream_ptr())
@@ -139,7 +140,7 @@ class IrsLqr:
         x = _device.to_device(np.asarray(x_trj, dtype=np.float64).reshape(1, self.T + 1, self.dim_x))
         u = _device.to_device(np.asarray(u_trj, dtype=np.float64).reshape(1, self.T, self.dim_u))
         cost = _device.empty((1,))
-        _lib.call("irs_evaluate_cost", self.dim_x, self.dim_u, _device.ptr(x), _device.ptr(u),
+        self.system.lib.call("irs_evaluate_cost", self.dim_x, self.dim_u, _device.ptr(x), _device.ptr(u),
                   _device.ptr(self._dxd), 0, _device.ptr(self._dQ), _device.ptr(self._dR), 1, self.T,
                   _device.ptr(cost), _device.stream_ptr())
         return float(cost.item())
@@ -223,12 +224,12 @@ class IrsLqr:
             gains.record(main)
             side.wait_event(gains)
             with torch.cuda.stream(side):
-                _lib.call("irs_tvlqr_plan_rows", n, m, _device.ptr(At), _device.ptr(Bt), _device.ptr(ct),
+                self.system.lib.call("irs_tvlqr_plan_rows", n, m, _device.ptr(At), _device.ptr(Bt), _device.ptr(ct),
                           _device.ptr(K), _device.ptr(k), 1, T, _device.ptr(db["plan_scratch"]),
                           _device.stream_ptr())
                 rows_done = torch.cuda.Event()
                 rows_done.record(side)
-        _lib.call("irs_rollout_closed_loop", self.system.system_id, prm, nprm, _device.ptr(K),
+        self.system.lib.call("irs_rollout_closed_loop", self.system.system_id, prm, nprm, _device.ptr(K),
                   _device.ptr(k), _device.ptr(x_all), _device.ptr(self._dxd), 0,
                   _device.ptr(self._dQ), _device.ptr(self._dR), 1, T, _device.ptr(db["x_new"]),
                   _device.ptr(db["u_new"]), _device.ptr(db["cost"]), _device.stream_ptr())
@@ -236,7 +237,7 @@ class IrsLqr:
             # would any of the reference's T re-solved QPs (irs_lqr.py:169-182) have had an active bound?
             xlo, xhi, ulo, uhi = db["box"]
             torch.cuda.current_stream().wait_event(rows_done)
-            _lib.call("irs_tvlqr_plan_check", n, m, _device.ptr(At), _device.ptr(Bt), _device.ptr(ct),
+            self.system.lib.call("irs_tvlqr_plan_check", n, m, _device.ptr(At), _device.ptr(Bt), _device.ptr(ct),
                       _device.ptr(K), _device.ptr(k), _device.ptr(db["x_new"]), _device.ptr(xlo),
                       _device.ptr(xhi), _device.ptr(ulo), _device.ptr(uhi), BOUND_TOL, 1, T, 1,
                       _device.ptr(db["violated"]), _device.ptr(db["plan_scratch"]), _device.stream_ptr())
@@ -249,7 +250,7 @@ class IrsLqr:
         """Linearization along the nominal trajectory, then the backward pass -> db["K"], db["k"]."""
         T, n, m = self.T, self.dim_x, self.dim_u
         At, Bt, ct, status = self._tv_matrices_device(x_nom, u_nom)
-        _lib.call("irs_tvlqr_riccati", n, m, _device.ptr(At), _device.ptr(Bt), _device.ptr(ct),
+        self.system.lib.call("irs_tvlqr_riccati", n, m, _device.ptr(At), _device.ptr(Bt), _device.ptr(ct),
                   _device.ptr(self._dQ), _device.ptr(self._dQd), _device.ptr(self._dR),
                   _device.ptr(self._dxd), 0, 1, T, _device.ptr(db["K"]), _device.ptr(db["k"]),
                   _device.ptr(db["rstatus"]), _device.stream_ptr())
@@ -337,19 +338,19 @@ class IrsLqr:
 
         def riccati():
             At, Bt, ct, _ = state["lin"]
-            _lib.call("irs_tvlqr_riccati", n, m, _device.ptr(At), _device.ptr(Bt), _device.ptr(ct),
+            self.system.lib.call("irs_tvlqr_riccati", n, m, _device.ptr(At), _device.ptr(Bt), _device.ptr(ct),
                       _device.ptr(self._dQ), _device.ptr(self._dQd), _device.ptr(self._dR), _device.ptr(self._dxd), 0, 1, T,
                       _device.ptr(db["K"]), _device.ptr(db["k"]), _device.ptr(db["rstatus"]), _device.stream_ptr())
 
         def rollout():
-            _lib.call("irs_rollout_closed_loop", self.system.system_id, prm, nprm, _device.ptr(db["K"]), _device.ptr(db["k"]),
+            self.system.lib.call("irs_rollout_closed_loop", self.system.system_id, prm, nprm, _device.ptr(db["K"]), _device.ptr(db["k"]),
                       _device.ptr(x_all), _device.ptr(self._dxd), 0, _device.ptr(self._dQ), _device.ptr(self._dR), 1, T,
                       _device.ptr(db["x_new"]), _device.ptr(db["u_new"]), _device.ptr(db["cost"]), _device.stream_ptr())
 
         def plan_check():
             At, Bt, ct, _ = state["lin"]
             xlo, xhi, ulo, uhi = db["box"]
-            _lib.call("irs_tvlqr_plan_check", n, m, _device.ptr(At), _device.ptr(Bt), _device.ptr(ct), _device.ptr(db["K"]),
+            self.system.lib.call("irs_tvlqr_plan_check", n, m, _device.ptr(At), _device.ptr(Bt), _device.ptr(ct), _device.ptr(db["K"]),
                       _device.ptr(db["k"]), _device.ptr(db["x_new"]), _device.ptr(xlo), _device.ptr(xhi), _device.ptr(ulo),
                       _device.ptr(uhi), BOUND_TOL, 1, T, 0, _device.ptr(db["violated"]), _device.ptr(db["plan_scratch"]),
                       _device.stream_ptr())
@@ -424,10 +425,17 @@ class IrsLqr:
         return self.x_trj, self.u_trj, self.cost
 
 
+def _require_jacobian(system, solver):
+    if not getattr(system, "has_jacobian", True):
+        raise NotImplementedError("%s needs the Jacobian of the dynamics: %r was built without one"
+                                  % (solver, getattr(system, "system_name", system)))
+
+
 class IrsLqrExact(IrsLqr):
     """irs_lqr/irs_lqr_exact.py:6-31 — Jacobian at the nominal point, evaluated in fp64."""
 
     def __init__(self, system, params):
+        _require_jacobian(system, "IrsLqrExact")
         super().__init__(system, params)
 
     def _tv_matrices_device(self, x_nom, u_nom):
@@ -436,7 +444,7 @@ class IrsLqrExact(IrsLqr):
         Bt = _device.empty((P, n, m))
         ct = _device.empty((P, n))
         prm, nprm = self.system._params()
-        _lib.call("irs_exact_linearize", self.system.system_id, prm, nprm, _device.ptr(x_nom),
+        self.system.lib.call("irs_exact_linearize", self.system.system_id, prm, nprm, _device.ptr(x_nom),
                   _device.ptr(u_nom), P, _device.ptr(At), _device.ptr(Bt), _device.ptr(ct),
                   _device.stream_ptr())
         status = torch.zeros((P,), dtype=torch.int32, device=x_nom.device)
@@ -472,6 +480,8 @@ class _SampledIrsLqr(IrsLqr):
     order = None
 
     def __init__(self, system, params, sampling):
+        if self.order == smoothing.FIRST_ORDER:
+            _require_jacobian(system, "IrsLqrFirstOrder")
         super().__init__(system, params)
         self.sampling = sampling
         self._key_cache = None
@@ -526,9 +536,10 @@ class _SampledIrsLqr(IrsLqr):
         bit-identical to the one-pass sequence (global point index in the Philox counter, carried
         (P, p) between segments)."""
         n, m, T = self.dim_x, self.dim_u, self.T
-        if not _USE_PIPELINE or not isinstance(self.sampling, GaussianSampling) or n % 2 or m % 2:
+        if not _USE_PIPELINE or not isinstance(self.sampling, GaussianSampling) or n % 2 or m % 2 \
+                or not self.system.riccati_segments:
             return None
-        C, _ = smoothing.plan(self.system.system_id, self.order, T, self.sampling.num_samples)
+        C, _ = smoothing.plan(self.system.system_id, self.order, T, self.sampling.num_samples, lib=self.system.lib)
         return pipeline_segments(T, C, _PIPELINE_SEGMENTS)
 
     def _linearize_and_riccati(self, db, x_nom, u_nom):
@@ -537,7 +548,7 @@ class _SampledIrsLqr(IrsLqr):
             return super()._linearize_and_riccati(db, x_nom, u_nom)
         s = self.sampling
         T, n, m = self.T, self.dim_x, self.dim_u
-        key = (self.system.system_id, self.order, T, s.num_samples)
+        key = (self.system.system_key, self.order, T, s.num_samples)
         if self._ws is None or self._ws.key != key:
             self._ws = smoothing.Workspace(self.system, self.order, T, s.num_samples)
         ws = self._ws
@@ -565,7 +576,7 @@ class _SampledIrsLqr(IrsLqr):
                 fitted.record(fin)
             side.wait_event(fitted)
             with torch.cuda.stream(side):
-                _lib.call("irs_tvlqr_riccati_segment", n, m, _device.ptr(ws.At), _device.ptr(ws.Bt),
+                self.system.lib.call("irs_tvlqr_riccati_segment", n, m, _device.ptr(ws.At), _device.ptr(ws.Bt),
                           _device.ptr(ws.ct), _device.ptr(self._dQ), _device.ptr(self._dQd),
                           _device.ptr(self._dR), _device.ptr(self._dxd), 0, 1, T, lo, hi,
                           _device.ptr(db["carry"]), _device.ptr(db["K"]), _device.ptr(db["k"]),
@@ -584,14 +595,14 @@ class _SampledIrsLqr(IrsLqr):
         c = self._key_cache
         if c is None or c[0] != prm or c[1] != (s.num_samples, s.flags()):
             c = (prm, (s.num_samples, s.flags()),
-                 (self.system.system_id, self.order, self.T, s.num_samples, s.flags(), tuple(float(v) for v in prm)))
+                 (self.system.system_key, self.order, self.T, s.num_samples, s.flags(), tuple(float(v) for v in prm)))
             self._key_cache = c
         return c[2]
 
     def _graph_update(self, graph):
         s = self.sampling
         _, sig_ptr = s.sigma32(self.iter)
-        _lib.call("irs_graph_update_smoothing", graph, sig_ptr, s.seed, int(self.iter), s.stream_id)
+        self.system.lib.call("irs_graph_update_smoothing", graph, sig_ptr, s.seed, int(self.iter), s.stream_id)
 
     def _enqueue_linearize(self, ws):
         s = self.sampling
@@ -608,7 +619,7 @@ class _SampledIrsLqr(IrsLqr):
         s = self.sampling
         if not isinstance(s, GaussianSampling):
             return super().get_TV_matrices(x_trj, u_trj)
-        key = (self.system.system_id, self.order, self.T, s.num_samples)
+        key = (self.system.system_key, self.order, self.T, s.num_samples)
         if self._ws is None or self._ws.key != key:
             self._ws = smoothing.Workspace(self.system, self.order, self.T, s.num_samples)
         ws = self._ws
@@ -646,16 +657,16 @@ class IrsLqrZeroOrder(_SampledIrsLqr):
             raise ValueError("expected dxdu [N, %d] and deltaf [N, %d]" % (d, n))
         N = dxdu.shape[0]
         Z, F = _device.to_device(dxdu), _device.to_device(deltaf)
-        width = _lib.lib().irs_partial_width(self.system.system_id, smoothing.ZERO_ORDER)
+        width = self.system.lib.handle().irs_partial_width(self.system.system_id, smoothing.ZERO_ORDER)
         block = torch.zeros((1, width), dtype=torch.float64, device=Z.device)
-        _lib.call("irs_gram_block_f64", n, m, _device.ptr(Z), _device.ptr(F), N, _device.ptr(block),
+        self.system.lib.call("irs_gram_block_f64", n, m, _device.ptr(Z), _device.ptr(F), N, _device.ptr(block),
                   _device.stream_ptr())
         zero_x, zero_u = torch.zeros((1, n), dtype=torch.float64, device=Z.device), \
             torch.zeros((1, m), dtype=torch.float64, device=Z.device)
         At, Bt, ct = _device.empty((1, n, n)), _device.empty((1, n, m)), _device.empty((1, n))
         status = _device.empty((1,), torch.int32)
         prm, nprm = self.system._params()
-        _lib.call("irs_smooth_finalize", self.system.system_id, prm, nprm, smoothing.ZERO_ORDER, _device.ptr(zero_x),
+        self.system.lib.call("irs_smooth_finalize", self.system.system_id, prm, nprm, smoothing.ZERO_ORDER, _device.ptr(zero_x),
                   _device.ptr(zero_u), 1, 1, None, _device.ptr(block), 1, 0, float(N), 0, _device.ptr(At),
                   _device.ptr(Bt), _device.ptr(ct), _device.ptr(status), _device.stream_ptr())
         smoothing.check_status(status)

@@ -96,6 +96,6 @@ def project_samples(system, x, dx, u, du):
     u_abs = np.asarray(u, dtype=np.float64) + np.asarray(du, dtype=np.float64)
     xd = _device.to_device(x_abs, torch.float64)
     prm, nprm = system._params()
-    _lib.call("irs_project_batch_f64", system.system_id, prm, nprm, _device.ptr(xd), xd.shape[0],
+    system.lib.call("irs_project_batch_f64", system.system_id, prm, nprm, _device.ptr(xd), xd.shape[0],
               _device.stream_ptr())
     return _device.to_numpy(xd), u_abs

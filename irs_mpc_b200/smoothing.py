@@ -19,11 +19,11 @@ FIRST_ORDER = 1
 FLAG_PROJECT_ABSOLUTE, FLAG_PROJECT_DELTA, FLAG_ANTITHETIC, FLAG_CENTERED = 2, 4, 8, 16
 
 
-def plan(system_id, order, P, N, chunk_samples=0):
+def plan(system_id, order, P, N, chunk_samples=0, lib=_lib.MAIN):
     """(C, S): C chunks of S samples per nominal point; chunk_samples = 0 is the library default."""
     C = ctypes.c_int(0)
     S = ctypes.c_longlong(0)
-    _lib.call("irs_smooth_plan", system_id, order, P, N, int(chunk_samples), ctypes.byref(C), ctypes.byref(S))
+    lib.call("irs_smooth_plan", system_id, order, P, N, int(chunk_samples), ctypes.byref(C), ctypes.byref(S))
     return C.value, S.value
 
 
@@ -35,9 +35,9 @@ class Workspace:
     API moves exactly one host->device and one device->host copy per linearization."""
 
     def __init__(self, system, order, P, N, chunk_samples=0):
-        self.key = (system.system_id, order, P, N) if not chunk_samples else (system.system_id, order, P, N, chunk_samples)
-        self.C, self.S = plan(system.system_id, order, P, N, chunk_samples)
-        self.width = _lib.lib().irs_partial_width(system.system_id, order)
+        self.key = (system.system_key, order, P, N) if not chunk_samples else (system.system_key, order, P, N, chunk_samples)
+        self.C, self.S = plan(system.system_id, order, P, N, chunk_samples, lib=system.lib)
+        self.width = system.lib.handle().irs_partial_width(system.system_id, order)
         n, m = system.dim_x, system.dim_u
         self.P, self.n, self.m = P, n, m
         self.partials = _device.empty((P, self.C, self.width), torch.float32)
@@ -122,7 +122,7 @@ def accumulate(system, order, x_nom, u_nom, N, ws, sigma=None, noise=None, seed=
         sig = sig.ctypes.data_as(ctypes.c_void_p)
     fn = ("irs_smooth_zero_order_accumulate" if order == ZERO_ORDER
           else "irs_smooth_first_order_accumulate")
-    _lib.call(fn, system.system_id, prm, nprm, flags, _device.ptr(x_nom), _device.ptr(u_nom), P,
+    system.lib.call(fn, system.system_id, prm, nprm, flags, _device.ptr(x_nom), _device.ptr(u_nom), P,
               int(N), sig, _device.ptr(noise), int(seed), int(it), int(stream_id),
               int(p0), int(i0), ws.C, ws.S, _device.ptr(partials), _device.stream_ptr())
 
@@ -132,7 +132,7 @@ def reduce_chunks(system, order, ws, out=None):
     P = ws.partials.shape[0]
     if out is None:
         out = _device.empty((P, ws.width))
-    _lib.call("irs_smooth_reduce_chunks", system.system_id, order, _device.ptr(ws.partials), P, ws.C,
+    system.lib.call("irs_smooth_reduce_chunks", system.system_id, order, _device.ptr(ws.partials), P, ws.C,
               _device.ptr(out), _device.stream_ptr())
     return out
 
@@ -150,7 +150,7 @@ def finalize(system, order, x_nom, u_nom, ws, n_total, partials=None, reduced=No
         x_nom, u_nom, part = x_nom[lo:hi], u_nom[lo:hi], part[lo:hi]
         At, Bt, ct, status = At[lo:hi], Bt[lo:hi], ct[lo:hi], status[lo:hi]
     P = x_nom.shape[0]
-    _lib.call("irs_smooth_finalize", system.system_id, prm, nprm, order, _device.ptr(x_nom),
+    system.lib.call("irs_smooth_finalize", system.system_id, prm, nprm, order, _device.ptr(x_nom),
               _device.ptr(u_nom), P, ws.C, _device.ptr(part), _device.ptr(reduced), nranks,
               int(rank_stride), float(n_total), 1 if ws.centered else 0, _device.ptr(At), _device.ptr(Bt),
               _device.ptr(ct), _device.ptr(status), _device.stream_ptr())
@@ -160,7 +160,7 @@ def finalize(system, order, x_nom, u_nom, ws, n_total, partials=None, reduced=No
 def linearize(system, order, x_nom, u_nom, N, ws=None, **kw):
     """x_nom [P,n], u_nom [P,m] (CUDA float64) -> (At, Bt, ct, status) CUDA tensors."""
     P = x_nom.shape[0]
-    if ws is None or ws.key != (system.system_id, order, P, N):
+    if ws is None or ws.key != (system.system_key, order, P, N):
         ws = Workspace(system, order, P, N)
     accumulate(system, order, x_nom, u_nom, N, ws, **kw)
     return finalize(system, order, x_nom, u_nom, ws, N) + (ws,)

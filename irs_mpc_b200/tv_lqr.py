@@ -54,14 +54,15 @@ def get_solver(solver_name):
     raise ValueError("Do not recognize solver.")
 
 
-def riccati_device(At, Bt, ct, Q, Qd, R, xd, xd_stride):
-    """Device-level backward pass.  At [I,T,n,n] ... -> K [I,T,m,n], k [I,T,m], status [I]."""
+def riccati_device(At, Bt, ct, Q, Qd, R, xd, xd_stride, lib=_lib.MAIN):
+    """Device-level backward pass.  At [I,T,n,n] ... -> K [I,T,m,n], k [I,T,m], status [I].
+    lib: the library to run it in (a user system's own library holds its (n, m))."""
     I, T, n, _ = At.shape
     m = Bt.shape[3]
     K = _device.empty((I, T, m, n))
     k = _device.empty((I, T, m))
     status = _device.empty((I,), torch.int32)
-    _lib.call("irs_tvlqr_riccati", n, m, _device.ptr(At), _device.ptr(Bt), _device.ptr(ct),
+    lib.call("irs_tvlqr_riccati", n, m, _device.ptr(At), _device.ptr(Bt), _device.ptr(ct),
               _device.ptr(Q), _device.ptr(Qd), _device.ptr(R), _device.ptr(xd), int(xd_stride),
               I, T, _device.ptr(K), _device.ptr(k), _device.ptr(status), _device.stream_ptr())
     return K, k, status
@@ -102,7 +103,7 @@ def box_solve_device(system, mpc, At, Bt, ct, dQ, dQd, dR, Q, Qd, R, dxd, xd_str
     Hinv = _device.empty((I, T, m, m))
     P = _device.empty((I, T + 1, n, n))
     rstatus = _device.empty((I,), torch.int32)
-    _lib.call("irs_tvlqr_riccati_ex", n, m, _device.ptr(At), _device.ptr(Bt), _device.ptr(ct),
+    system.lib.call("irs_tvlqr_riccati_ex", n, m, _device.ptr(At), _device.ptr(Bt), _device.ptr(ct),
               _device.ptr(Qe), _device.ptr(Qde), _device.ptr(Re), _device.ptr(dxd), int(xd_stride), I, T,
               _device.ptr(K), _device.ptr(k), _device.ptr(rstatus), _device.ptr(Hinv), _device.ptr(P),
               _device.stream_ptr())
@@ -118,7 +119,7 @@ def box_solve_device(system, mpc, At, Bt, ct, dQ, dQd, dR, Q, Qd, R, dxd, xd_str
     ubox_stride = m if np.ndim(ulo) == 2 else 0
     if (xbox_stride and np.shape(xlo) != (T + 1, n)) or (ubox_stride and np.shape(ulo) != (T, m)):
         raise ValueError("time-varying boxes must be [T+1, n] (states) and [T, m] (inputs)")
-    _lib.call("irs_tvlqr_box_solve", system.system_id, prm, nprm, 1 if mpc else 0, _device.ptr(At),
+    system.lib.call("irs_tvlqr_box_solve", system.system_id, prm, nprm, 1 if mpc else 0, _device.ptr(At),
               _device.ptr(Bt), _device.ptr(ct), _device.ptr(K), _device.ptr(Hinv), _device.ptr(P),
               _device.ptr(dQ), _device.ptr(dQd), _device.ptr(dR), _device.ptr(dxd), int(xd_stride),
               _device.ptr(d["dx"]), _device.ptr(d["du"]), _device.ptr(d["xlo"]), _device.ptr(d["xhi"]),
@@ -132,6 +133,7 @@ def box_solve_device(system, mpc, At, Bt, ct, dQ, dQd, dR, Q, Qd, R, dxd, xd_str
 class _DimsOnlySystem:
     """solve_tvlqr knows only (n, m): the bounded single-QP solve never evaluates the dynamics, but the
     kernel is instantiated per built-in system; pick the one with matching dimensions."""
+    lib = _lib.MAIN
     _BY_DIMS = {(2, 1): (0, [0.05]), (5, 2): (1, [0.1]), (12, 4): (2, [0.05, 0.775, 0.15, 9.81, 0.0015, 0.0025,
                                                                       0.0035, 1.0, 0.0245]),
                 (6, 2): (3, [0.05, 0.2])}
