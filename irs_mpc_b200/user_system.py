@@ -8,6 +8,7 @@
             o[0] = x[0] + h * x[2];  ...
         ''',
         jacobian=None,      # optional: a body writing J[N*D], row-major, columns [x | u]
+        autodiff=False,     # or True: the Jacobian of the step body by forward-mode dual numbers
         name="cartpole")
 
 The bodies are C++ over the scalar type R, instantiated as float (the sample work of the smoothing kernels)
@@ -21,6 +22,19 @@ C ABI, in which the user system has id 5 (kUser).  Every kernel of the hot path 
 accumulation, fits, Riccati, rollouts, the bounded descent — is then the one the built-in systems run.  The
 library is cached under a hash of everything it is built from (IRS_USER_CACHE, default: _user_cache/ next to
 this file); constructing the same system again loads it without compiling.
+
+autodiff=True derives the Jacobian from the step body alone (no jacobian body; giving both is a ValueError).  The
+body is then also evaluated over irs::ad::Dual<R, K> (csrc/dual.cuh): a value and K tangent lanes, packed FP32
+pairs in float.  jac_var seeds unit tangents on K consecutive columns of [x | u] per pass, P = ceil(D / 8) passes
+of K = ceil(D / P), and reads J off the tangents of o.  In such a body R is the dual type where it is
+differentiated, while h and p[] stay plain float / double.  Supported: construction from int, float, double and R;
+unary -; + - * / and += -= *= /= with R or a number on either side; comparisons (on the values); Math<R>::sincos /
+rcp / div (the values are Math<float>'s fast intrinsics or Math<double>'s); sqrt, exp, log, sin, cos, tan, asin,
+acos, atan, atan2, sinh, cosh, tanh, fabs, fmin, fmax, and pow with a constant exponent.  There is no conversion
+back to float, double or int: a body that drops the derivative (`float t = x[0];`) does not compile.  At kinks:
+branches follow the values; fabs at 0 takes the + branch; fmin / fmax take the derivative of the argument they
+select, the first one on a tie; sqrt at 0 gives the infinite derivative that math gives.  The Jacobian is checked
+against central differences at construction, as a hand-written body is.
 """
 import ctypes
 import functools
@@ -41,6 +55,7 @@ USER_SYSTEM_ID = 5
 MAX_REGRESSORS = 16         # kMaxRegressors (csrc/smooth.cuh): n + m
 MAX_PARAMS = 9              # SysParams::v[10] (csrc/common.cuh) holds h and nine more
 BUILTIN_PAIRS = ((2, 1), (5, 2), (12, 4), (6, 2))      # (n, m) with compile-time LQR kernels (api.cu)
+AUTODIFF_MAX_LANES = 8      # tangent lanes of one forward-mode pass (DESIGN.md 3.10.1)
 
 
 def cache_dir():
@@ -73,9 +88,17 @@ def _build_inputs_digest():
     return h.hexdigest()
 
 
-def generate_source(dim_x, dim_u, nparams, step, jacobian=None):
+def autodiff_passes(d):
+    """(P, K) of a forward-mode Jacobian over d columns: P passes of K tangent lanes, K at most 8."""
+    p = -(-d // AUTODIFF_MAX_LANES)
+    return p, -(-d // p)
+
+
+def generate_source(dim_x, dim_u, nparams, step, jacobian=None, autodiff=False):
     """The translation unit of a user library: the functor around the bodies, then csrc/api.cu.
     nparams counts h.  #line directives make the compiler's diagnostics point into the bodies."""
+    if autodiff:
+        return _generate_autodiff_source(dim_x, dim_u, nparams, step)
     n, m = dim_x, dim_u
     d = n + m
     lines = [
@@ -129,6 +152,93 @@ def generate_source(dim_x, dim_u, nparams, step, jacobian=None):
     return "\n".join(lines)
 
 
+def _generate_autodiff_source(dim_x, dim_u, nparams, step):
+    """generate_source with autodiff: the step body is written once, in UserStep<B>::eval over any scalar type
+    R, and UserSystem<B> derives from UserStep<B>.  step<BATCH> evaluates it over B; jac_var evaluates step<false>
+    over irs::ad::Dual<B, K> in P passes, each seeding unit tangents on K consecutive columns of [x | u]."""
+    n, m = dim_x, dim_u
+    d = n + m
+    np_ = max(1, nparams - 1)
+    passes, lanes = autodiff_passes(d)
+    lines = [
+        "// generated by irs_mpc_b200/user_system.py: a user-written system around csrc/api.cu, its Jacobian by",
+        "// forward-mode dual numbers (csrc/dual.cuh)",
+        "#define IRS_USER_SYSTEM 1",
+        "#define IRS_USER_AUTODIFF 1",
+        "#define IRS_USER_N %d" % n,
+        "#define IRS_USER_M %d" % m,
+        "#define IRS_USER_NPARAMS %d" % nparams,
+        '#include "systems.cuh"',
+        '#include "dual.cuh"',
+        "",
+        "namespace irs {",
+        "// the step body over any scalar R; h and p[] stay in the base type B (parameters carry no tangents)",
+        "template <typename B>",
+        "struct UserStep {",
+        "    static constexpr int N = %d, M = %d, D = %d;" % (n, m, d),
+        "    B h;",
+        "    B p[%d];" % np_,
+        "    template <bool BATCH, typename R>",
+        "    __device__ __forceinline__ void eval(const R* x, const R* u, R* o) const {",
+    ]
+    lines.append('#line 1 "step"')
+    lines.extend(step.splitlines() or [""])
+    lines.append('#line %d "user_system.cu"' % (len(lines) + 2))
+    lines += [
+        "    }",
+        "};",
+        "",
+        "template <typename R>",
+        "struct UserSystem : UserStep<R> {",
+        "    template <typename S> using Rebind = UserSystem<S>;",
+        "    static constexpr int N = %d, M = %d, D = %d, NJ = %d;" % (n, m, d, n * d),
+        "    static constexpr bool kHasJacobian = true;",
+        "    static constexpr int kTrigAhead = 0;",
+        "    static constexpr bool kHasProjection = false;",
+        "    // jac_var: P passes of K tangent lanes (P = ceil(D / 8), K = ceil(D / P))",
+        "    static constexpr int kPasses = %d, kLanes = %d;" % (passes, lanes),
+        "    __device__ explicit UserSystem(const SysParams& sp) {",
+        "        this->h = prm<R>(sp, 0);",
+        "#pragma unroll",
+        "        for (int i = 0; i < %d; ++i) this->p[i] = i + 1 < %d ? prm<R>(sp, i + 1) : R(0);" % (np_, nparams),
+        "    }",
+        "    template <bool BATCH>",
+        "    __device__ __forceinline__ void step(const R* x, const R* u, R* o) const {",
+        "        this->template eval<BATCH, R>(x, u, o);",
+        "    }",
+        "    // the whole Jacobian of step<false> varies: jac_var writes it, jac_assemble copies it",
+        "    __device__ __forceinline__ void jac_var(const R* x, const R* u, R* J) const {",
+        "        using DR = ad::Dual<R, kLanes>;",
+        "#pragma unroll",
+        "        for (int pass = 0; pass < kPasses; ++pass) {",
+        "            const int c0 = pass * kLanes;",
+        "            DR xd[N], ud[M], od[N];",
+        "#pragma unroll",
+        "            for (int q = 0; q < N; ++q) xd[q] = DR::seed(x[q], q - c0);",
+        "#pragma unroll",
+        "            for (int q = 0; q < M; ++q) ud[q] = DR::seed(u[q], N + q - c0);",
+        "            this->template eval<false, DR>(xd, ud, od);",
+        "#pragma unroll",
+        "            for (int i = 0; i < N; ++i)",
+        "#pragma unroll",
+        "                for (int k = 0; k < kLanes; ++k)",
+        "                    if (c0 + k < D) J[i * D + c0 + k] = od[i].tangent(k);",
+        "        }",
+        "    }",
+        "    __device__ __forceinline__ void jac_assemble(const R* v, R* J) const {",
+        "#pragma unroll",
+        "        for (int i = 0; i < N * D; ++i) J[i] = v[i];",
+        "    }",
+        "    __device__ __forceinline__ void project(R*) const {}",
+        "};",
+        "}  // namespace irs",
+        "",
+        '#include "api.cu"',
+        "",
+    ]
+    return "\n".join(lines)
+
+
 def _compile(src_path, out_path):
     """nvcc with the main library's flags; RuntimeError with the compiler's diagnostics on failure."""
     cmd = [_nvcc()] + _lib.NVCC_FLAGS + ["-I", _lib.INCLUDE, "-I", _lib.CSRC, "-o", out_path, src_path]
@@ -137,10 +247,12 @@ def _compile(src_path, out_path):
         raise RuntimeError("compiling the user system failed:\n" + (res.stderr or res.stdout))
 
 
-def build_library(dim_x, dim_u, nparams, step, jacobian=None, name="user"):
+def build_library(dim_x, dim_u, nparams, step, jacobian=None, name="user", autodiff=False):
     """Compile (or find in the cache) the library of one user system -> (path, seconds spent compiling,
-    source hash).  seconds is 0.0 on a cache hit."""
-    src = generate_source(dim_x, dim_u, nparams, step, jacobian)
+    source hash).  seconds is 0.0 on a cache hit.  autodiff: derive the Jacobian from the step body."""
+    if autodiff and jacobian is not None:
+        raise ValueError("give a jacobian body or autodiff=True, not both")
+    src = generate_source(dim_x, dim_u, nparams, step, jacobian, autodiff)
     src_digest = hashlib.sha256((src + _build_inputs_digest()).encode()).hexdigest()[:24]
     tag = re.sub(r"[^A-Za-z0-9_]", "_", str(name))[:40] or "user"
     root = cache_dir()
@@ -175,14 +287,15 @@ class CudaSourceDynamics(CudaDynamicalSystem):
     dim_x, dim_u: N and M, with N + M <= 16.  h: the step, visible as `h`.  params: at most nine further
     finite numbers, visible as p[0..]; `self.params` may be changed later (same count), which re-captures
     the solvers' CUDA graphs.  step: body computing o = f(x, u).  jacobian: optional body writing
-    J = d f / d(x, u) [N x (N+M)] row-major; when given it is checked against central differences of the
-    fp64 step at a few seeded points (this needs the GPU) and a mismatch is refused.  Without it, the
+    J = d f / d(x, u) [N x (N+M)] row-major.  autodiff: derive J from the step body by forward-mode dual
+    numbers instead (not together with jacobian).  Either Jacobian is checked against central differences of
+    the fp64 step at a few seeded points (this needs the GPU) and a mismatch is refused.  Without one, the
     Jacobian methods, IrsLqrFirstOrder and IrsLqrExact raise NotImplementedError.  Changing the source
     means a new object."""
 
     system_id = USER_SYSTEM_ID
 
-    def __init__(self, dim_x, dim_u, h, params=(), step=None, jacobian=None, name="user"):
+    def __init__(self, dim_x, dim_u, h, params=(), step=None, jacobian=None, autodiff=False, name="user"):
         super().__init__()
         if int(dim_x) != dim_x or int(dim_u) != dim_u or dim_x < 1 or dim_u < 1:
             raise ValueError("dim_x and dim_u must be positive integers, got %r and %r" % (dim_x, dim_u))
@@ -204,11 +317,12 @@ class CudaSourceDynamics(CudaDynamicalSystem):
         self.dim_x, self.dim_u = dim_x, dim_u
         self.params = params
         self.system_name = str(name)
-        self.has_jacobian = jacobian is not None
+        self.autodiff = bool(autodiff)
+        self.has_jacobian = jacobian is not None or self.autodiff
         self.riccati_segments = (dim_x, dim_u) in BUILTIN_PAIRS
         self._nparams = 1 + len(params)
         path, self.build_seconds, self.source_hash = build_library(dim_x, dim_u, self._nparams, step, jacobian,
-                                                                   name)
+                                                                   name, self.autodiff)
         self.cache_hit = self.build_seconds == 0.0
         self.library_path = path
         self.lib = _lib.Library.at(path)
@@ -232,14 +346,16 @@ class CudaSourceDynamics(CudaDynamicalSystem):
 
     def jacobian_xu_batch(self, x, u, *args, **kw):
         if not self.has_jacobian:
-            raise NotImplementedError("user system %r was built without a Jacobian body" % self.system_name)
+            raise NotImplementedError("user system %r was built without a Jacobian body or autodiff=True"
+                                      % self.system_name)
         return super().jacobian_xu_batch(x, u, *args, **kw)
 
     def jacobian_xu(self, x, u):
         return self.jacobian_xu_batch(np.asarray(x)[None, :], np.asarray(u)[None, :])[0]
 
     def _check_jacobian(self, points=4, seed=0):
-        """Refuse a Jacobian body that disagrees with central differences of the fp64 step."""
+        """Refuse a Jacobian (a body, or the dual-number derivative) that disagrees with central differences of
+        the fp64 step."""
         n, m = self.dim_x, self.dim_u
         d = n + m
         rng = np.random.default_rng(seed)
@@ -255,6 +371,6 @@ class CudaSourceDynamics(CudaDynamicalSystem):
         tol = 1e-5 * max(1.0, float(np.abs(fd).max()))
         if not np.all(err <= tol):
             p, i, j = np.unravel_index(int(np.argmax(err)), err.shape)
-            raise ValueError("the Jacobian body of %r disagrees with central differences of its step: "
+            raise ValueError("the Jacobian of %r disagrees with central differences of its step: "
                              "J[%d][%d] = %.6g at point %d, differences give %.6g"
                              % (self.system_name, i, j, J[p, i, j], p, fd[p, i, j]))
