@@ -41,6 +41,18 @@ int irs_mlp_register(int dim_x, int dim_u, int h1, int h2, const float* W1, cons
                      const float* b2, const float* W3, const float* b3, int* handle);
 int irs_mlp_release(int handle);
 
+/* Arrays of a user-written system (irs_mpc_b200/user_system.py: CudaSourceDynamics(arrays=...)).  A library of
+ * such a system reads its arrays from one registered array set: `count` float64 HOST values, all arrays back to
+ * back, copied to the current device as float64 and as float32 (each element rounded once from the float64).
+ * The system's params are then [h, p..., handle].  irs_user_arrays_update overwrites elements
+ * [offset, offset + count) of both copies, ordered on `stream`; kernels and captured graphs that read the set
+ * see the new values from then on.  irs_user_arrays_release frees the set (after synchronising with the
+ * device).  Values must be finite.  The main library exports these entry points and refuses every call. */
+#define IRS_USER_ARRAYS_MAX_ELEMS (1 << 24)
+int irs_user_arrays_register(const double* values, long long count, int* handle);
+int irs_user_arrays_update(int handle, long long offset, const double* values, long long count, void* stream);
+int irs_user_arrays_release(int handle);
+
 /* smoothing flags */
 enum {
   IRS_SAMPLES_BATCH_VARIANT = 1, /* samples use dynamics_batch semantics (irs_lqr_zero_order.py:51);

@@ -81,6 +81,9 @@ SIGNATURES = {
     "irs_tvlqr_riccati_ex": [_i, _i, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _ll, _i, _i, _vp, _vp, _vp, _vp, _vp, _vp],
     "irs_mlp_register": [_i, _i, _i, _i, _vp, _vp, _vp, _vp, _vp, _vp, _vp],
     "irs_mlp_release": [_i],
+    "irs_user_arrays_register": [_vp, _ll, ctypes.POINTER(_i)],
+    "irs_user_arrays_update": [_i, _ll, _vp, _ll, _vp],
+    "irs_user_arrays_release": [_i],
     "irs_cem_refit": [_vp, _vp, _i, _i, _i, _i, _vp, _vp, _vp, _vp],
     "irs_gram_block_f64": [_i, _i, _vp, _vp, _ll, _vp, _vp],
     "irs_tvlqr_plan_rows": [_i, _i, _vp, _vp, _vp, _vp, _vp, _i, _i, _vp, _vp],

@@ -44,6 +44,19 @@ struct MlpEntry {
 static std::vector<MlpEntry> g_mlps;
 static std::mutex g_mlp_mutex;
 
+#ifdef IRS_USER_SYSTEM
+// Registered array sets of the user system (irs_user_arrays_register): an fp64 copy and an fp32 copy of the
+// same elements, one set per handle.
+struct ArraySetEntry {
+    double* f64;
+    float* f32;
+    long long count;
+    int device;
+};
+static std::vector<ArraySetEntry> g_array_sets;
+static std::mutex g_array_mutex;
+#endif
+
 static int load_params(int system, const double* params_host, int nparams, SysParams* out) {
 #ifndef IRS_USER_SYSTEM
     static const int expected[kNumSystems] = {1, 1, 9, 2, 2};
@@ -54,7 +67,26 @@ static int load_params(int system, const double* params_host, int nparams, SysPa
     IRS_REQUIRE(params_host != nullptr && nparams == expected[system],
                 "system %d expects %d parameters, got %d", system, expected[system], nparams);
     memset(out, 0, sizeof(*out));
-    for (int i = 0; i < nparams; ++i) {
+    int nscalars = nparams;
+#ifdef IRS_USER_ARRAYS
+    if (system == kUser) {           // [h, p..., handle] -> the registered array set
+        nscalars = nparams - 1;
+        const int handle = (int)params_host[nparams - 1];
+        std::lock_guard<std::mutex> lock(g_array_mutex);
+        IRS_REQUIRE(handle >= 0 && handle < (int)g_array_sets.size() && g_array_sets[handle].f64 != nullptr,
+                    "unknown array set handle %d (irs_user_arrays_register)", handle);
+        const ArraySetEntry& e = g_array_sets[handle];
+        IRS_REQUIRE(e.count == IRS_USER_ARRAY_ELEMS, "array set %d holds %lld elements, the system reads %lld",
+                    handle, e.count, (long long)IRS_USER_ARRAY_ELEMS);
+        int dev = 0;
+        cudaGetDevice(&dev);
+        IRS_REQUIRE(dev == e.device, "array set %d was registered on device %d, current device is %d", handle,
+                    e.device, dev);
+        out->arrays64 = e.f64;
+        out->arrays32 = e.f32;
+    }
+#endif
+    for (int i = 0; i < nscalars; ++i) {
         out->v[i] = params_host[i];
         out->f[i] = (float)params_host[i];
     }
@@ -914,6 +946,87 @@ int irs_mlp_release(int handle) {
     g_mlps[handle].w2_tc = nullptr;
     return 0;
 }
+
+#ifdef IRS_USER_SYSTEM
+static int finite_values(const double* values, long long count) {
+    for (long long i = 0; i < count; ++i)
+        IRS_REQUIRE(values[i] - values[i] == 0.0, "array values must be finite (element %lld is %g)", i, values[i]);
+    return 0;
+}
+
+int irs_user_arrays_register(const double* values, long long count, int* handle) {
+    IRS_REQUIRE(values && handle, "null pointer argument");
+    IRS_REQUIRE(count >= 1 && count <= IRS_USER_ARRAYS_MAX_ELEMS, "an array set holds 1 to %lld elements, got %lld",
+                (long long)IRS_USER_ARRAYS_MAX_ELEMS, count);
+    if (finite_values(values, count)) return 1;
+    std::vector<float> f32((size_t)count);
+    for (long long i = 0; i < count; ++i) f32[(size_t)i] = (float)values[i];      // rounded once, from float64
+    ArraySetEntry e{nullptr, nullptr, count, 0};
+    cudaGetDevice(&e.device);
+    if (cudaMalloc(&e.f64, sizeof(double) * count) != cudaSuccess) return check_launch("cudaMalloc(array set)");
+    if (cudaMalloc(&e.f32, sizeof(float) * count) != cudaSuccess) {
+        cudaFree(e.f64);
+        return check_launch("cudaMalloc(array set)");
+    }
+    if (cudaMemcpy(e.f64, values, sizeof(double) * count, cudaMemcpyHostToDevice) != cudaSuccess ||
+        cudaMemcpy(e.f32, f32.data(), sizeof(float) * count, cudaMemcpyHostToDevice) != cudaSuccess) {
+        cudaFree(e.f64);
+        cudaFree(e.f32);
+        return check_launch("cudaMemcpy(array set)");
+    }
+    std::lock_guard<std::mutex> lock(g_array_mutex);
+    g_array_sets.push_back(e);
+    *handle = (int)g_array_sets.size() - 1;
+    return 0;
+}
+
+int irs_user_arrays_update(int handle, long long offset, const double* values, long long count, void* stream) {
+    IRS_REQUIRE(values, "null pointer argument");
+    std::lock_guard<std::mutex> lock(g_array_mutex);
+    IRS_REQUIRE(handle >= 0 && handle < (int)g_array_sets.size() && g_array_sets[handle].f64 != nullptr,
+                "unknown array set handle %d", handle);
+    const ArraySetEntry& e = g_array_sets[handle];
+    IRS_REQUIRE(offset >= 0 && count >= 1 && offset + count <= e.count,
+                "elements [%lld, %lld) lie outside array set %d of %lld elements", offset, offset + count, handle,
+                e.count);
+    int dev = 0;
+    cudaGetDevice(&dev);
+    IRS_REQUIRE(dev == e.device, "array set %d was registered on device %d, current device is %d", handle, e.device,
+                dev);
+    if (finite_values(values, count)) return 1;
+    std::vector<float> f32((size_t)count);
+    for (long long i = 0; i < count; ++i) f32[(size_t)i] = (float)values[i];
+    // pageable sources: each copy has read its source when the call returns (the host buffers may go), and
+    // runs in stream order, after the kernels enqueued before it
+    const cudaStream_t st = (cudaStream_t)stream;
+    if (cudaMemcpyAsync(e.f64 + offset, values, sizeof(double) * count, cudaMemcpyHostToDevice, st) != cudaSuccess ||
+        cudaMemcpyAsync(e.f32 + offset, f32.data(), sizeof(float) * count, cudaMemcpyHostToDevice, st) != cudaSuccess)
+        return check_launch("cudaMemcpyAsync(array set)");
+    return 0;
+}
+
+int irs_user_arrays_release(int handle) {
+    std::lock_guard<std::mutex> lock(g_array_mutex);
+    IRS_REQUIRE(handle >= 0 && handle < (int)g_array_sets.size() && g_array_sets[handle].f64 != nullptr,
+                "unknown array set handle %d", handle);
+    cudaFree(g_array_sets[handle].f64);      // synchronises with the device: no kernel still reads it
+    cudaFree(g_array_sets[handle].f32);
+    g_array_sets[handle].f64 = nullptr;
+    g_array_sets[handle].f32 = nullptr;
+    return 0;
+}
+#else
+// array sets belong to user-written systems: the main library exports the entry points so that one ABI
+// serves both kinds of library, and refuses
+static int no_array_sets() {
+    set_error("array sets belong to the library of a user-written system (CudaSourceDynamics); the main library "
+              "has none");
+    return 1;
+}
+int irs_user_arrays_register(const double*, long long, int*) { return no_array_sets(); }
+int irs_user_arrays_update(int, long long, const double*, long long, void*) { return no_array_sets(); }
+int irs_user_arrays_release(int) { return no_array_sets(); }
+#endif
 
 int irs_philox_dump(int P, long long N, int d, const float* sigma_host, unsigned long long seed,
                     unsigned iter, unsigned stream_id, unsigned p0, unsigned long long i0, int antithetic,

@@ -31,6 +31,11 @@ struct SysParams {
     const float* mlp;
     const unsigned short* mlp_w2;      // hidden layer as tensor-core operand: bf16 pieces [hi | lo] (smooth_mlp.cuh)
     int h1, h2;
+#ifdef IRS_USER_SYSTEM
+    // arrays of a user-written system (irs_user_arrays_register): the fp64 and fp32 copies of its array set
+    const double* arrays64;
+    const float* arrays32;
+#endif
 };
 
 // ---------------------------------------------------------------------------------------------

@@ -9,6 +9,7 @@
         ''',
         jacobian=None,      # optional: a body writing J[N*D], row-major, columns [x | u]
         autodiff=False,     # or True: the Jacobian of the step body by forward-mode dual numbers
+        arrays=None,        # optional: {name: array} read by the bodies from device memory
         name="cartpole")
 
 The bodies are C++ over the scalar type R, instantiated as float (the sample work of the smoothing kernels)
@@ -35,6 +36,17 @@ back to float, double or int: a body that drops the derivative (`float t = x[0];
 branches follow the values; fabs at 0 takes the + branch; fmin / fmax take the derivative of the argument they
 select, the first one on a tie; sqrt at 0 gives the infinite derivative that math gives.  The Jacobian is checked
 against central differences at construction, as a hand-written body is.
+
+arrays={name: values} gives the bodies read-only arrays in device memory: matrices, lookup tables, network weights.
+Each is real, finite and non-empty with 1 to 3 dimensions; all of them together hold at most 2^24 elements
+(MAX_ARRAY_ELEMENTS).  In a body, `name[i]` reads it flat (row-major), `name(i, j)` and `name(i, j, k)` by
+dimension, and `name_n0`, `name_n1`, `name_n2` are its extents (1 for a missing dimension) as compile-time
+constants.  Elements are in the base type, like h and p[]: float in the fp32 sample kernels, double elsewhere; they
+carry no tangents under autodiff.  An element is returned by value, so writing to an array does not compile.
+Only the names and shapes enter the generated source: systems that differ in array values share one library,
+and `set_array(name, values)` replaces one array's values (same shape) in place, without recompiling and without
+re-capturing a CUDA graph.  Names must be C identifiers that are neither C++ keywords nor names a body already
+sees (RESERVED_NAMES), and must not start with `irs` or `__`.
 """
 import ctypes
 import functools
@@ -48,7 +60,7 @@ import time
 
 import numpy as np
 
-from . import _lib
+from . import _device, _lib
 from .dynamical_system import CudaDynamicalSystem
 
 USER_SYSTEM_ID = 5
@@ -56,6 +68,91 @@ MAX_REGRESSORS = 16         # kMaxRegressors (csrc/smooth.cuh): n + m
 MAX_PARAMS = 9              # SysParams::v[10] (csrc/common.cuh) holds h and nine more
 BUILTIN_PAIRS = ((2, 1), (5, 2), (12, 4), (6, 2))      # (n, m) with compile-time LQR kernels (api.cu)
 AUTODIFF_MAX_LANES = 8      # tangent lanes of one forward-mode pass (DESIGN.md 3.10.1)
+MAX_ARRAY_ELEMENTS = 1 << 24        # IRS_USER_ARRAYS_MAX_ELEMS (include/irs_mpc_b200.h): int indices in a body
+# names a body already sees, the generated functor's members, and the math functions a body calls: an array
+# of such a name would shadow them
+RESERVED_NAMES = frozenset("""
+    x u o J h p R B N M D Math
+    NJ Rebind kHasJacobian kTrigAhead kHasProjection kPasses kLanes BATCH DR
+    step eval jac_var jac_assemble project UserStep UserSystem SysParams ArrayView prm user_arrays ad irs std
+    sqrt exp log sin cos tan asin acos atan atan2 sinh cosh tanh fabs fmin fmax pow floor ceil round trunc
+    fmod abs min max sincos rcp div
+""".split())
+CPP_KEYWORDS = frozenset("""
+    alignas alignof and and_eq asm auto bitand bitor bool break case catch char char8_t char16_t char32_t class
+    compl concept const consteval constexpr constinit const_cast continue co_await co_return co_yield decltype
+    default delete do double dynamic_cast else enum explicit export extern false float for friend goto if inline
+    int long mutable namespace new noexcept not not_eq nullptr operator or or_eq private protected public
+    register reinterpret_cast requires return short signed sizeof static static_assert static_cast struct switch
+    template this thread_local throw true try typedef typeid typename union unsigned using virtual void volatile
+    wchar_t while xor xor_eq
+""".split())
+_IDENTIFIER = re.compile(r"[A-Za-z_][A-Za-z0-9_]*\Z")
+
+
+def _check_array(name, values):
+    """values as a C-contiguous float64 array; ValueError naming the array unless real, finite, non-empty and
+    of 1 to 3 dimensions."""
+    try:
+        a = np.asarray(values)
+        if np.iscomplexobj(a):
+            raise TypeError("complex")
+        a = np.asarray(a, dtype=np.float64)
+    except (TypeError, ValueError):
+        raise ValueError("array %r must hold real numbers" % (name,)) from None
+    if not 1 <= a.ndim <= 3:
+        raise ValueError("array %r has %d dimensions; arrays have 1 to 3" % (name, a.ndim))
+    a = np.ascontiguousarray(a)
+    if a.size == 0:
+        raise ValueError("array %r is empty" % (name,))
+    if not np.all(np.isfinite(a)):
+        raise ValueError("array %r holds a value that is not finite" % (name,))
+    return a
+
+
+def check_arrays(arrays):
+    """The arrays of a user system, validated -> [(name, float64 array)] in the mapping's order (see the module
+    docstring for the rules).  Every violation is a ValueError naming the array."""
+    if arrays is None:
+        return []
+    if not hasattr(arrays, "items"):
+        raise ValueError("arrays must be a mapping from name to array, got %s" % type(arrays).__name__)
+    out, total = [], 0
+    for name, values in arrays.items():
+        if not isinstance(name, str) or not _IDENTIFIER.match(name):
+            raise ValueError("array name %r is not a C identifier" % (name,))
+        if name in RESERVED_NAMES or name in CPP_KEYWORDS:
+            raise ValueError("array name %r is taken: a body already sees that name" % name)
+        if name.startswith("irs") or name.startswith("__"):
+            raise ValueError("array name %r starts with a reserved prefix (irs, __)" % name)
+        out.append((name, _check_array(name, values)))
+        total += out[-1][1].size
+        if total > MAX_ARRAY_ELEMENTS:
+            raise ValueError("array %r brings the arrays to %d elements, more than the limit of %d"
+                             % (name, total, MAX_ARRAY_ELEMENTS))
+    extents = {"%s_n%d" % (name, k) for name, _ in out for k in range(3)}
+    for name, _ in out:
+        if name in extents:
+            raise ValueError("array name %r is the name of another array's extent" % name)
+    return out
+
+
+def _array_lines(arrays, scalar="R"):
+    """Members of the functor for checked arrays: extents, then one view per array into the copy in `scalar`."""
+    lines = []
+    for name, a in arrays:
+        n0, n1, n2 = tuple(a.shape) + (1,) * (3 - a.ndim)
+        lines.append("    static constexpr int %s_n0 = %d, %s_n1 = %d, %s_n2 = %d;" % (name, n0, name, n1, name, n2))
+        lines.append("    ArrayView<%s, %d, %d, %d, %d> %s;" % (scalar, a.ndim, n0, n1, n2, name))
+    return lines
+
+
+def _array_init_lines(arrays, prefix):
+    lines, off = [], 0
+    for name, a in arrays:
+        lines.append("        %s%s.data = user_arrays<R>(sp) + %d;" % (prefix, name, off))
+        off += a.size
+    return lines
 
 
 def cache_dir():
@@ -94,11 +191,23 @@ def autodiff_passes(d):
     return p, -(-d // p)
 
 
-def generate_source(dim_x, dim_u, nparams, step, jacobian=None, autodiff=False):
+def _array_defines(arrays, nparams):
+    """The defines of a unit with arrays: the handle is one more parameter after h and p[]."""
+    if not arrays:
+        return ["#define IRS_USER_NPARAMS %d" % nparams]
+    return ["#define IRS_USER_NPARAMS %d" % (nparams + 1),
+            "#define IRS_USER_ARRAYS 1",
+            "#define IRS_USER_ARRAY_ELEMS %d" % sum(a.size for _, a in arrays)]
+
+
+def generate_source(dim_x, dim_u, nparams, step, jacobian=None, autodiff=False, arrays=None):
     """The translation unit of a user library: the functor around the bodies, then csrc/api.cu.
-    nparams counts h.  #line directives make the compiler's diagnostics point into the bodies."""
+    nparams counts h.  #line directives make the compiler's diagnostics point into the bodies.  arrays: the
+    mapping of CudaSourceDynamics; only names and shapes enter the source (the handle of the array set follows
+    the scalar parameters)."""
+    arrays = check_arrays(arrays)
     if autodiff:
-        return _generate_autodiff_source(dim_x, dim_u, nparams, step)
+        return _generate_autodiff_source(dim_x, dim_u, nparams, step, arrays)
     n, m = dim_x, dim_u
     d = n + m
     lines = [
@@ -106,8 +215,9 @@ def generate_source(dim_x, dim_u, nparams, step, jacobian=None, autodiff=False):
         "#define IRS_USER_SYSTEM 1",
         "#define IRS_USER_N %d" % n,
         "#define IRS_USER_M %d" % m,
-        "#define IRS_USER_NPARAMS %d" % nparams,
+    ] + _array_defines(arrays, nparams) + [
         '#include "systems.cuh"',
+    ] + (['#include "user_arrays.cuh"'] if arrays else []) + [
         "",
         "namespace irs {",
         "template <typename R>",
@@ -119,9 +229,11 @@ def generate_source(dim_x, dim_u, nparams, step, jacobian=None, autodiff=False):
         "    static constexpr bool kHasProjection = false;",
         "    R h;",
         "    R p[%d];" % max(1, nparams - 1),
+    ] + _array_lines(arrays) + [
         "    __device__ explicit UserSystem(const SysParams& sp) : h(prm<R>(sp, 0)) {",
         "#pragma unroll",
         "        for (int i = 0; i < %d; ++i) p[i] = i + 1 < %d ? prm<R>(sp, i + 1) : R(0);" % (max(1, nparams - 1), nparams),
+    ] + _array_init_lines(arrays, "") + [
         "    }",
         "    template <bool BATCH>",
         "    __device__ __forceinline__ void step(const R* x, const R* u, R* o) const {",
@@ -152,7 +264,7 @@ def generate_source(dim_x, dim_u, nparams, step, jacobian=None, autodiff=False):
     return "\n".join(lines)
 
 
-def _generate_autodiff_source(dim_x, dim_u, nparams, step):
+def _generate_autodiff_source(dim_x, dim_u, nparams, step, arrays):
     """generate_source with autodiff: the step body is written once, in UserStep<B>::eval over any scalar type
     R, and UserSystem<B> derives from UserStep<B>.  step<BATCH> evaluates it over B; jac_var evaluates step<false>
     over irs::ad::Dual<B, K> in P passes, each seeding unit tangents on K consecutive columns of [x | u]."""
@@ -167,9 +279,10 @@ def _generate_autodiff_source(dim_x, dim_u, nparams, step):
         "#define IRS_USER_AUTODIFF 1",
         "#define IRS_USER_N %d" % n,
         "#define IRS_USER_M %d" % m,
-        "#define IRS_USER_NPARAMS %d" % nparams,
+    ] + _array_defines(arrays, nparams) + [
         '#include "systems.cuh"',
         '#include "dual.cuh"',
+    ] + (['#include "user_arrays.cuh"'] if arrays else []) + [
         "",
         "namespace irs {",
         "// the step body over any scalar R; h and p[] stay in the base type B (parameters carry no tangents)",
@@ -178,6 +291,7 @@ def _generate_autodiff_source(dim_x, dim_u, nparams, step):
         "    static constexpr int N = %d, M = %d, D = %d;" % (n, m, d),
         "    B h;",
         "    B p[%d];" % np_,
+    ] + _array_lines(arrays, "B") + [
         "    template <bool BATCH, typename R>",
         "    __device__ __forceinline__ void eval(const R* x, const R* u, R* o) const {",
     ]
@@ -201,6 +315,7 @@ def _generate_autodiff_source(dim_x, dim_u, nparams, step):
         "        this->h = prm<R>(sp, 0);",
         "#pragma unroll",
         "        for (int i = 0; i < %d; ++i) this->p[i] = i + 1 < %d ? prm<R>(sp, i + 1) : R(0);" % (np_, nparams),
+    ] + _array_init_lines(arrays, "this->") + [
         "    }",
         "    template <bool BATCH>",
         "    __device__ __forceinline__ void step(const R* x, const R* u, R* o) const {",
@@ -247,12 +362,13 @@ def _compile(src_path, out_path):
         raise RuntimeError("compiling the user system failed:\n" + (res.stderr or res.stdout))
 
 
-def build_library(dim_x, dim_u, nparams, step, jacobian=None, name="user", autodiff=False):
+def build_library(dim_x, dim_u, nparams, step, jacobian=None, name="user", autodiff=False, arrays=None):
     """Compile (or find in the cache) the library of one user system -> (path, seconds spent compiling,
-    source hash).  seconds is 0.0 on a cache hit.  autodiff: derive the Jacobian from the step body."""
+    source hash).  seconds is 0.0 on a cache hit.  autodiff: derive the Jacobian from the step body.
+    arrays: {name: values}; only the names and shapes select the library."""
     if autodiff and jacobian is not None:
         raise ValueError("give a jacobian body or autodiff=True, not both")
-    src = generate_source(dim_x, dim_u, nparams, step, jacobian, autodiff)
+    src = generate_source(dim_x, dim_u, nparams, step, jacobian, autodiff, arrays)
     src_digest = hashlib.sha256((src + _build_inputs_digest()).encode()).hexdigest()[:24]
     tag = re.sub(r"[^A-Za-z0-9_]", "_", str(name))[:40] or "user"
     root = cache_dir()
@@ -290,12 +406,15 @@ class CudaSourceDynamics(CudaDynamicalSystem):
     J = d f / d(x, u) [N x (N+M)] row-major.  autodiff: derive J from the step body by forward-mode dual
     numbers instead (not together with jacobian).  Either Jacobian is checked against central differences of
     the fp64 step at a few seeded points (this needs the GPU) and a mismatch is refused.  Without one, the
-    Jacobian methods, IrsLqrFirstOrder and IrsLqrExact raise NotImplementedError.  Changing the source
-    means a new object."""
+    Jacobian methods, IrsLqrFirstOrder and IrsLqrExact raise NotImplementedError.  arrays: {name: values} the
+    bodies read from device memory (module docstring), registered on the current device; set_array replaces
+    one array's values.  Changing the source, or an array's shape, means a new object."""
 
     system_id = USER_SYSTEM_ID
+    _array_handle = -1
 
-    def __init__(self, dim_x, dim_u, h, params=(), step=None, jacobian=None, autodiff=False, name="user"):
+    def __init__(self, dim_x, dim_u, h, params=(), step=None, jacobian=None, autodiff=False, name="user",
+                 arrays=None):
         super().__init__()
         if int(dim_x) != dim_x or int(dim_u) != dim_u or dim_x < 1 or dim_u < 1:
             raise ValueError("dim_x and dim_u must be positive integers, got %r and %r" % (dim_x, dim_u))
@@ -313,6 +432,7 @@ class CudaSourceDynamics(CudaDynamicalSystem):
             raise ValueError("step must be the C++ body of the dynamics")
         if jacobian is not None and (not isinstance(jacobian, str) or not jacobian.strip()):
             raise ValueError("jacobian must be a C++ body or None")
+        arrays = check_arrays(arrays)
         self.h = float(h)
         self.dim_x, self.dim_u = dim_x, dim_u
         self.params = params
@@ -322,7 +442,7 @@ class CudaSourceDynamics(CudaDynamicalSystem):
         self.riccati_segments = (dim_x, dim_u) in BUILTIN_PAIRS
         self._nparams = 1 + len(params)
         path, self.build_seconds, self.source_hash = build_library(dim_x, dim_u, self._nparams, step, jacobian,
-                                                                   name, self.autodiff)
+                                                                   name, self.autodiff, dict(arrays))
         self.cache_hit = self.build_seconds == 0.0
         self.library_path = path
         self.lib = _lib.Library.at(path)
@@ -331,6 +451,17 @@ class CudaSourceDynamics(CudaDynamicalSystem):
         if (n.value, m.value) != (dim_x, dim_u):
             raise RuntimeError("library %s holds a (%d, %d) system, expected (%d, %d)"
                                % (path, n.value, m.value, dim_x, dim_u))
+        # name -> (offset of its first element in the array set, current values)
+        self._arrays, offset = {}, 0
+        for aname, a in arrays:
+            self._arrays[aname] = (offset, a)
+            offset += a.size
+        if arrays:
+            _device.require_cuda()
+            handle = ctypes.c_int(-1)
+            flat = np.concatenate([a.ravel() for _, a in arrays])
+            self.lib.call("irs_user_arrays_register", flat.ctypes.data, flat.size, ctypes.byref(handle))
+            self._array_handle = handle.value
         if self.has_jacobian:
             self._check_jacobian()
 
@@ -342,7 +473,40 @@ class CudaSourceDynamics(CudaDynamicalSystem):
         if len(self.params) != self._nparams - 1:
             raise ValueError("system %r was built with %d parameters, now has %d"
                              % (self.system_name, self._nparams - 1, len(self.params)))
-        return [self.h] + [float(v) for v in self.params]
+        prm = [self.h] + [float(v) for v in self.params]
+        if self._arrays:
+            prm.append(float(self._array_handle))     # in the graph keys: systems with other values never share
+        return prm
+
+    @property
+    def arrays(self):
+        """{name: a read-only view of the current values (float64)}."""
+        out = {}
+        for name, (_, a) in self._arrays.items():
+            v = a.view()
+            v.flags.writeable = False
+            out[name] = v
+        return out
+
+    def set_array(self, name, values):
+        """Replace the values of array `name` (same shape).  The copy is ordered on the current stream: the next
+        call sees the new values, eager or replayed from a CUDA graph; nothing recompiles or re-captures."""
+        if name not in self._arrays:
+            raise ValueError("system %r has no array %r (it has %s)" % (self.system_name, name, sorted(self._arrays)))
+        offset, old = self._arrays[name]
+        a = _check_array(name, values)
+        if a.shape != old.shape:
+            raise ValueError("array %r has shape %s, got values of shape %s" % (name, old.shape, a.shape))
+        self.lib.call("irs_user_arrays_update", self._array_handle, offset, a.ctypes.data, a.size,
+                      _device.stream_ptr())
+        self._arrays[name] = (offset, a)
+
+    def __del__(self):
+        try:
+            if self._array_handle >= 0:
+                self.lib.call("irs_user_arrays_release", self._array_handle)
+        except Exception:      # interpreter shutdown: the library may be gone already
+            pass
 
     def jacobian_xu_batch(self, x, u, *args, **kw):
         if not self.has_jacobian:

@@ -26,7 +26,7 @@ not depend on how the solver strides its tasks over workers.
 import numpy as np
 import torch
 
-from . import _device, _lib, smoothing
+from . import _device, smoothing
 from .dynamical_system import CudaDynamicalSystem
 
 MODES = {"zero_order_AB": smoothing.ZERO_ORDER, "first_order": smoothing.FIRST_ORDER, "exact": None}
@@ -105,7 +105,7 @@ class GpuLinearizationWorker:
         if self.order is None:
             At, Bt, ct = _device.empty((k, n, n)), _device.empty((k, n, m)), _device.empty((k, n))
             prm, nprm = s._params()
-            _lib.call("irs_exact_linearize", s.system_id, prm, nprm, _device.ptr(xd), _device.ptr(ud), k,
+            s.lib.call("irs_exact_linearize", s.system_id, prm, nprm, _device.ptr(xd), _device.ptr(ud), k,
                       _device.ptr(At), _device.ptr(Bt), _device.ptr(ct), _device.stream_ptr())
             out[:, :, :n], out[:, :, n:] = _device.to_numpy(At), _device.to_numpy(Bt)
             return out
