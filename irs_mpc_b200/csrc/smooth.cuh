@@ -806,9 +806,12 @@ __device__ __forceinline__ void static_for(F&& f) {
 }
 
 // Fixed-order sums (ranks, then chunks: the order of sum_partials) of U entries of one point at once;
-// the loads of the U entries are independent, so they are in flight together.
+// the loads of the U entries are independent, so they are in flight together.  CB > 1: the loads of CB
+// chunks are issued before the first of their adds as well (one L2 round trip per CB chunks instead of
+// one per chunk; the adds keep their order, so the sums do not depend on CB).  CB * U floats of registers;
+// CB > 1 has a block barrier between the loads and the adds: every thread of the block must call it.
 // pbase = offset of the point inside a rank buffer (chunk 0), rel[u] = entry index, < 0 = none (sum 0).
-template <int U>
+template <int U, int CB = 1>
 __device__ __forceinline__ void sum_partials_multi(const PartialSource& a, long long pbase, const int (&rel)[U],
                                                    int width, double (&s)[U]) {
 #pragma unroll
@@ -823,12 +826,34 @@ __device__ __forceinline__ void sum_partials_multi(const PartialSource& a, long 
             for (int u = 0; u < U; ++u) s[u] += v[u];
         } else {
             const float* src = a.partials + r * a.rank_stride + pbase;
-            for (int c = 0; c < a.C; ++c, src += width) {
-                float v[U];
+            for (int c = 0; c < a.C; c += CB, src += CB * width) {
+                float v[CB][U];
 #pragma unroll
-                for (int u = 0; u < U; ++u) v[u] = rel[u] >= 0 ? src[rel[u]] : 0.f;
+                for (int k = 0; k < CB; ++k) {
+                    // past the last chunk: load the last one again and drop it (a branch around the load would
+                    // let the compiler convert each value right after its load, i.e. wait for it)
+                    const int kk = c + k < a.C ? k : a.C - 1 - c;
 #pragma unroll
-                for (int u = 0; u < U; ++u) s[u] += (double)v[u];
+                    for (int u = 0; u < U; ++u) v[k][u] = rel[u] >= 0 ? src[kk * width + rel[u]] : 0.f;
+                }
+                // Fence: without it the compiler interleaves the adds with the loads, and the first add to
+                // wait for its load holds back every load behind it.  A barrier alone does not stop that (the
+                // conversions are register work and move above it), so every value is OR-ed with the
+                // barrier's result, which is 0 (C >= 1): the adds now depend on the barrier, the loads stay
+                // above it, and the bits are untouched.  tools/finalize_phases.py reports the schedule.
+                if constexpr (CB > 1) {
+                    const int zero = __syncthreads_or(a.C < 1);
+#pragma unroll
+                    for (int k = 0; k < CB; ++k)
+#pragma unroll
+                        for (int u = 0; u < U; ++u) v[k][u] = __int_as_float(__float_as_int(v[k][u]) | zero);
+                }
+#pragma unroll
+                for (int k = 0; k < CB; ++k)
+                    if (c + k < a.C) {
+#pragma unroll
+                        for (int u = 0; u < U; ++u) s[u] += (double)v[k][u];
+                    }
             }
         }
     }
@@ -885,6 +910,35 @@ __device__ __forceinline__ void write_abc(const FinalizeArgs& a, int p, const do
     }
 }
 
+// Chunks whose loads a thread of finalize_zero_order_kernel has in flight at once (<= 3 entries per
+// thread: 96 floats of registers): a point's partials cost ceil(C / 32) L2 round trips instead of C
+// (C = 25 at N = 1e5: one).
+constexpr int kFinalizeChunksInFlight = 32;
+
+// Phase clock of finalize_zero_order_kernel (tools/finalize_phases.py builds the library with
+// -DIRS_FINALIZE_PHASES; the shipped library has no stamps): SM clock and global timer at each phase
+// boundary of block 0, read back through irs_finalize_phases().
+#ifdef IRS_FINALIZE_PHASES
+enum FinalizePhase { kPhStart, kPhSums, kPhGram, kPhNominal, kPhFactor, kPhSolve, kPhWritten, kNumFinalizePhases };
+__device__ unsigned long long g_finalize_phases[2 * kNumFinalizePhases];
+// Every lane of the warp runs the stamp and the stores are predicated: a branch would leave the warp
+// diverged after it, and the shuffles of the factorisation would then take their slow path.
+__device__ __forceinline__ void finalize_stamp(int k, bool on) {
+    unsigned long long ns;
+    asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(ns));
+    const unsigned long long clk = (unsigned long long)clock64();
+    asm volatile("{ .reg .pred p;  setp.ne.u32 p, %0, 0;  @p st.global.u64 [%1], %2;  @p st.global.u64 [%3], %4; }"
+                 :: "r"((unsigned)(on && blockIdx.x == 0)), "l"(g_finalize_phases + k), "l"(clk),
+                    "l"(g_finalize_phases + kNumFinalizePhases + k), "l"(ns) : "memory");
+}
+extern "C" int irs_finalize_phases(unsigned long long* out) {
+    return cudaMemcpyFromSymbol(out, g_finalize_phases, sizeof(g_finalize_phases)) == cudaSuccess ? 0 : 1;
+}
+#define IRS_FINALIZE_STAMP(k, cond) finalize_stamp(k, cond)
+#else
+#define IRS_FINALIZE_STAMP(k, cond) do { } while (0)
+#endif
+
 template <class Sys, int BT>
 __global__ void __launch_bounds__(BT, 1) finalize_zero_order_kernel(const FinalizeArgs a) {
     constexpr int n = Sys::N, m = Sys::M, d = Sys::D;
@@ -898,8 +952,10 @@ __global__ void __launch_bounds__(BT, 1) finalize_zero_order_kernel(const Finali
     __shared__ double mom[WIDTH - NACC > 0 ? WIDTH - NACC : 1];   // [sum z' (d) | sum dF' (n)]
     __shared__ double spread[d];      // diagonal of the CENTRED Gram: scale of the rank test
     __shared__ double rho[n];         // centred: f_batch(2 xbar, 2 ubar) - f(xbar, ubar), the response shift
+    __shared__ double colk[2][32];    // column k of the factor, for the lanes of warp 0
     const int tid = threadIdx.x, lane = tid & 31;
     const int p = blockIdx.x;
+    IRS_FINALIZE_STAMP(kPhStart, tid == 0);
     // 0. sample-sharded run: exchange this point's chunk-reduced block with the other ranks first
     PartialSource src = partial_source(a);
     bool peer_late = false;
@@ -908,7 +964,8 @@ __global__ void __launch_bounds__(BT, 1) finalize_zero_order_kernel(const Finali
     else if (a.peer.mode == kPeerGather) epoch = *reinterpret_cast<volatile int*>(a.peer.epoch) + 1;
     __shared__ int status_s;
     // 1. fixed-order sum over ranks and chunks, unpacked into the symmetric Gram and the rhs; a thread's
-    //    entries are summed together so that all their loads are in flight at once
+    //    entries over kFinalizeChunksInFlight chunks are summed together so that all their loads are in
+    //    flight at once
     {
         constexpr int NE = (WIDTH + BT - 1) / BT;
         int rel[NE];
@@ -916,7 +973,8 @@ __global__ void __launch_bounds__(BT, 1) finalize_zero_order_kernel(const Finali
         for (int q = 0; q < NE; ++q) rel[q] = tid + q * BT < WIDTH ? tid + q * BT : -1;
         double sums[NE];
         const long long pbase = (long long)p * (src.reduced != nullptr ? (long long)WIDTH : (long long)src.C * WIDTH);
-        sum_partials_multi<NE>(src, pbase, rel, WIDTH, sums);
+        sum_partials_multi<NE, kFinalizeChunksInFlight>(src, pbase, rel, WIDTH, sums);
+        IRS_FINALIZE_STAMP(kPhSums, tid == 0);
 #pragma unroll
         for (int q = 0; q < NE; ++q) {
             if (rel[q] >= NACC) {
@@ -971,6 +1029,7 @@ __global__ void __launch_bounds__(BT, 1) finalize_zero_order_kernel(const Finali
         }
     }
     __syncthreads();
+    IRS_FINALIZE_STAMP(kPhGram, tid == 0);
     // learned dynamics: warp 1 evaluates the network together (Mlp::step_warp, bit-identical to the functor)
     constexpr bool kWarpNominal = is_mlp<Sys>::value;
     __shared__ float mlp_act[kWarpNominal ? 2 * kMlpMaxHidden : 1];
@@ -994,45 +1053,71 @@ __global__ void __launch_bounds__(BT, 1) finalize_zero_order_kernel(const Finali
         } else {
             nominal_compute_to_smem<Sys>(a, p, nom);
         }
+        IRS_FINALIZE_STAMP(kPhNominal, tid == 32);
     } else if (tid < 32) {
-        // 2. Cholesky G = L L^T by warp 0, left-looking, lane = row with the row of the factor in
-        //    REGISTERS: row k reaches the other lanes by shuffles, every lane recomputes the pivot (same
-        //    operands, same order: identical bits), no shared-memory round trip inside the
-        //    factorisation.  A column whose diagonal is exactly zero (sigma = 0: regressor identically
-        //    zero) gets coefficient 0, which is what the min-norm lstsq of the reference returns for it.
+        // 2. Cholesky G = L L^T by warp 0, right-looking, lane = row with the row of the factor in
+        //    REGISTERS: once column k is scaled, its entries reach the other lanes (see below) and every
+        //    lane updates its later entries with them; the pivot of column k + 1 is then one shuffle away
+        //    and every lane computes its reciprocal square root (same operands: identical bits).  Each
+        //    entry receives its updates in ascending column order — the fmas of the left-looking
+        //    factorisation this replaces (and of the quad kernel), operand for operand — and only one
+        //    update lies between two pivots, not two chains of k of them.
+        //    A column whose diagonal is exactly zero (sigma = 0: regressor identically zero) gets
+        //    coefficient 0, which is what the min-norm lstsq of the reference returns for it.
         bool bad = false;
+        unsigned zero_mask = 0;
         double row[d];
 #pragma unroll
         for (int j = 0; j < d; ++j) row[j] = (lane < d && j <= lane) ? Gm[lane * d + j] : 0.0;
+        double piv = __shfl_sync(0xffffffffu, row[0], 0);      // G_kk - sum_{j<k} L_kj^2, updated by lane k
         static_for<0, d>([&](auto kc) {
             constexpr int k = decltype(kc)::value;
-            double lk[k > 0 ? k : 1];            // row k of the factor (entries j < k)
-            static_for<0, k>([&](auto jc) { constexpr int j = decltype(jc)::value;  lk[j] = __shfl_sync(0xffffffffu, row[j], k); });
-            const double d0 = __shfl_sync(0xffffffffu, row[k], k);      // the original diagonal entry G_kk
-            double dk = d0;
-            static_for<0, k>([&](auto jc) { constexpr int j = decltype(jc)::value;  dk = fma(-lk[j], lk[j], dk); });
-            bool zero_col = false;
+            const double d0 = Gm[k * d + k];      // the original diagonal entry G_kk (Gm is written after the loop)
+            double dk = piv;
             // pivot <= 1e-6 * G_kk: the column is (numerically) a combination of earlier ones; the
             // fp32 partial sums carry ~1e-7 relative noise, so anything below is rank deficiency.
             // (Centred accumulation: the noise is relative to the SPREAD of the column, i.e. the centred
             //  diagonal, and a pivot of the shifted Gram is never below that of the centred one.)
             const double scale_k = (WIDTH > NACC && a.centered) ? spread[k] : d0;
-            if (d0 == 0.0) { zero_col = true; dk = 1.0; }
-            else if (!(dk > 1e-6 * scale_k)) { bad = true; dk = 1.0; }
+            const bool zero_col = d0 == 0.0;
+            const bool dependent = !zero_col && !(dk > 1e-6 * scale_k);
+            bad = bad || dependent;
+            if (zero_col || dependent) dk = 1.0;
             const double ikk = rsqrt(dk);           // one special function on the critical path, not two
-            double sk = row[k];
-            static_for<0, k>([&](auto jc) { constexpr int j = decltype(jc)::value;  sk = fma(-row[j], lk[j], sk); });
-            if (lane > k) row[k] = zero_col ? 0.0 : sk * ikk;
-            if (lane == k) { row[k] = dk * ikk;  inv_diag[k] = ikk; }
-            if (zero_col)
-                for (int q = lane; q < n; q += 32) Bm[k * n + q] = 0.0;
+            // selects, not branches: no reconvergence point between two pivots
+            const double lik = zero_col ? 0.0 : row[k] * ikk, lkk = dk * ikk;
+            row[k] = lane > k ? lik : (lane == k ? lkk : row[k]);
+            if (lane == k) inv_diag[k] = ikk;
+            if (zero_col) zero_mask |= 1u << k;
+            // G_ic -= L_ik L_ck for every later column c.  The next pivot's column first, by shuffle, and
+            // its pivot is broadcast at once; the other columns read L_ck from shared memory (one store
+            // per lane instead of two shuffles per column; two buffers: a lane may store column k + 2
+            // once every lane has passed the barrier of column k + 1, i.e. finished reading column k).
+            if constexpr (k + 1 < d) {
+                const double l = __shfl_sync(0xffffffffu, row[k], k + 1);      // L_k+1,k
+                row[k + 1] = fma(-row[k], l, row[k + 1]);
+                piv = __shfl_sync(0xffffffffu, row[k + 1], k + 1);
+            }
+            if constexpr (k + 2 < d) {
+                double* col = colk[k & 1];
+                col[lane] = row[k];
+                __syncwarp();
+                static_for<k + 2, d>([&](auto cc) {
+                    constexpr int c = decltype(cc)::value;
+                    row[c] = fma(-row[k], col[c], row[c]);      // col[c] = L_ck
+                });
+            }
         });
+        for (int k = 0; k < d; ++k)
+            if ((zero_mask >> k) & 1u)
+                for (int q = lane; q < n; q += 32) Bm[k * n + q] = 0.0;
         if (lane < d) {
 #pragma unroll
             for (int j = 0; j < d; ++j)
                 if (j <= lane) Gm[lane * d + j] = row[j];      // the solves read the factor from shared memory
         }
         __syncwarp();
+        IRS_FINALIZE_STAMP(kPhFactor, lane == 0);
         // 3. solve L L^T X = B, one right-hand side per lane (reciprocal diagonal: no divisions)
         if (lane < n) {
             const int q = lane;
@@ -1060,6 +1145,7 @@ __global__ void __launch_bounds__(BT, 1) finalize_zero_order_kernel(const Finali
         }
         bad = __any_sync(0xffffffffu, bad);
         if (lane == 0) status_s = peer_late ? 2 : (bad ? 1 : 0);      // 2: a peer's block never arrived
+        IRS_FINALIZE_STAMP(kPhSolve, lane == 0);
     }
     __syncthreads();
     if (a.peer.mode == kPeerGather) {
@@ -1068,6 +1154,7 @@ __global__ void __launch_bounds__(BT, 1) finalize_zero_order_kernel(const Finali
     } else {
         if (tid == 0) a.status[p] = status_s;
         write_abc<Sys, BT>(a, p, sAB, nom, tid);
+        IRS_FINALIZE_STAMP(kPhWritten, tid == 0);
         if (a.peer.mode == kPeerExchange) peer_exchange_finish(a, epoch, tid);
     }
 }
