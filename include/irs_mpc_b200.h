@@ -341,7 +341,7 @@ int irs_rollout_open_loop(int system, const double* params_host, int nparams,
                           int I, int T, double* x_trj, double* cost, void* stream);
 
 /* CrossEntropyMethod.local_descent, steps 3-4 (irs_lqr/cem.py:173-182): marks the n_elite cheapest of the
- * B candidates (elite [B] int, ties by index, NaN last) and refits mean [T,m] / std [T,m] (population
+ * B candidates (elite [B] int, ties by index, NaN after +inf) and refits mean [T,m] / std [T,m] (population
  * standard deviation) of the candidate input trajectories u_candidates [B,T,m] over them.  cost [B] is the
  * output of irs_rollout_open_loop. */
 int irs_cem_refit(const double* cost, const double* u_candidates, int B, int T, int m, int n_elite,

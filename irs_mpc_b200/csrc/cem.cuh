@@ -7,26 +7,31 @@
 
 namespace irs {
 
-// elite[b] = 1 iff cost[b] is among the n_elite smallest (ties broken by index, NaN sorts last): the
-// rank of b is the number of candidates that come before it in that total order.  O(B^2) comparisons,
-// B ~ 1e3-1e4 (the reference uses an O(B) partial partition; any choice among equal costs is valid).
+// elite[b] = 1 iff b is among the first n_elite candidates in the order of the key (isnan(cost), cost,
+// index): every NaN after every other value, +inf included (as np.argpartition / np.argsort place it, so a
+// diverged rollout never displaces an infinite-cost one), equal costs (-0.0 == +0.0) and NaNs by index.
+// The rank of b is the number of candidates that come before it in that total order, so exactly n_elite
+// are marked.  O(B^2) comparisons, B ~ 1e3-1e4 (the reference uses an O(B) partial partition; any choice
+// among equal costs is valid).
 __global__ void __launch_bounds__(256) cem_rank_kernel(const double* cost, int B, int n_elite, int* elite) {
     __shared__ double tile[256];
     const int b = blockIdx.x * blockDim.x + threadIdx.x;
-    double mine = b < B ? cost[b] : 0.0;
-    if (!(mine == mine)) mine = 1.0 / 0.0;      // NaN -> +inf
+    const double mine = b < B ? cost[b] : 0.0;
+    const bool mine_nan = mine != mine;
     int rank = 0;
     for (int base = 0; base < B; base += 256) {
         const int j = base + threadIdx.x;
-        double v = j < B ? cost[j] : 1.0 / 0.0;
-        if (!(v == v)) v = 1.0 / 0.0;
         __syncthreads();
-        tile[threadIdx.x] = v;
+        tile[threadIdx.x] = j < B ? cost[j] : 0.0;
         __syncthreads();
         const int lim = B - base < 256 ? B - base : 256;
         for (int q = 0; q < lim; ++q) {
             const double v2 = tile[q];
-            rank += (v2 < mine || (v2 == mine && base + q < b)) ? 1 : 0;
+            const bool nan2 = v2 != v2;
+            const bool before = nan2 != mine_nan ? mine_nan                        // the non-NaN one first
+                              : nan2 ? base + q < b                                // both NaN: by index
+                              : v2 < mine || (v2 == mine && base + q < b);         // by value, then by index
+            rank += before ? 1 : 0;
         }
     }
     if (b < B) elite[b] = rank < n_elite ? 1 : 0;

@@ -798,10 +798,12 @@ def test_pipelined_descent_is_bit_identical_to_one_pass(api, name, T, N, graphs,
 # ------------------------------------------------------------------------------------------------
 # CEM baseline (irs_lqr/cem.py) — SURVEY.md section 8f row 2
 # ------------------------------------------------------------------------------------------------
-@pytest.mark.parametrize("name,T,B", [("pendulum", 60, 200), ("three_cart", 40, 128)])
+@pytest.mark.parametrize("name,T,B", [("pendulum", 60, 200), ("three_cart", 40, 128), ("bicycle", 40, 300),
+                                      ("quadrotor", 30, 1000)])
 def test_cem_matches_numpy_restatement(api, name, T, B):
     """Same seed -> same candidates (np.random.normal, as the reference); costs from the batched
     rollout kernel equal the float64 loop of cem.py:165-169, so the elite set and the refit agree."""
+    from irs_mpc_b200 import _device
     cfg = ec.CONFIGS[name](T=T)
     s = make_system(api, name)
     m = s.dim_u
@@ -819,6 +821,10 @@ def test_cem_matches_numpy_restatement(api, name, T, B):
     costs = np.array([cr.evaluate_cost(cr.rollout(orc, cfg["x0"], cand[k]), cand[k], cfg["xd_trj"], cfg["Q"],
                                        cfg["R"]) for k in range(B)])
     best = np.argpartition(costs, p.n_elite)[:p.n_elite]
+    # the device's elites are the first n_elite of the stable order (NaN last, ties by index)
+    want = np.zeros(B, np.int32)
+    want[np.argsort(costs, kind="stable")[:p.n_elite]] = 1
+    assert np.array_equal(_device.to_numpy(solver.last_elite), want)
     u_o = cand[best].mean(axis=0)
     np.testing.assert_allclose(u_new, u_o, rtol=1e-9, atol=1e-12)
     np.testing.assert_allclose(solver.std_trj, cand[best].std(axis=0), rtol=1e-9, atol=1e-12)
